@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mrays/s and frame ms of the eraytracer hot path on N B200s.
 
-  python bench.py --gpus N --steps K --warmup W [--workload c4] [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--workload c4] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one frame of the workload.  The scene is uploaded once before timing
 (BASELINE.json north_star: "uploads a flattened SoA scene once"); `value` is timed with the
@@ -13,6 +13,11 @@ one rank per GPU) the SAME frame is split into interleaved row bands, one part p
 --impl reference times the CPU oracle (a C restatement of raytracer.erl; the reference
 itself needs Erlang/OTP, which this image does not have) on all host cores over a bounded
 lattice of pixels of the same frame.
+
+--dump-outputs DIR writes the RGB8 frame the last step of the timed block rendered (this rank's rows; the values
+as float32) to DIR/frame.npy, DIR/frame_rank<R>.npy with N > 1, and the row index of each of its rows to
+DIR/frame_rows.npy (frame_rank<R>_rows.npy).  Frames over DUMP_BYTES in float32 keep a fixed, seeded sample of
+rows, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -39,6 +44,10 @@ WORKLOADS = {
     "c4d1": ("C4 synthetic 1M-sphere scene 3840x2160, 3 point lights, depth 1 (run-concurrent.sh depth)", "c4", 3840, 2160, 1),
     "c5": ("C5 demo scene 7680x4320 depth 1, camera pose k of 64 per step", "demo", 7680, 4320, 1),
 }
+
+
+DUMP_BYTES = 60 << 20       # float32 frame values written by --dump-outputs, over all ranks
+DUMP_SEED = 20260101
 
 
 def log(*a):
@@ -228,6 +237,22 @@ def reference_arm(args, rank):
 
 
 # --------------------------------------------------------------------------- GPU arm
+def dump_frame(out_dir, dev, w, h, band_rows, n_parts, rank, world):
+    """Writes the RGB8 rows of this rank's part that slot 0 rendered last (ert_download), see --dump-outputs."""
+    from eraytracer_b200 import _lib, multigpu
+    frame = np.zeros((h, w, 3), dtype=np.uint8)
+    _lib.check(_lib.load().ert_download(dev.handle, 0, frame.ctypes.data, frame.nbytes))
+    rows = multigpu.part_rows(h, band_rows, n_parts, rank)
+    max_rows = DUMP_BYTES // world // (w * 3 * 4)
+    if len(rows) > max_rows:
+        rows = np.sort(np.random.default_rng(DUMP_SEED).choice(rows, max_rows, replace=False))
+    name = "frame" if world == 1 else "frame_rank%d" % rank
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), frame[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+    log("[rank %d] wrote %d of %d rows of the last timed frame to %s" % (rank, len(rows), h, out_dir))
+
+
 def gpu_arm(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -340,6 +365,8 @@ def gpu_arm(args, rank, world, local_rank):
         rays += st["rays"]
         launches += st["gpu_launches"]
     barrier()
+    if args.dump_outputs:
+        dump_frame(args.dump_outputs, dev, w, h, band_rows, n_parts, rank, world)
     # split by kernel class: a separate pass with one event before and after EVERY launch (ERT_FLAG_TIME_KERNELS;
     # the events cost ~3 % on a 2 ms part, so the pass is kept out of `value`)
     split_steps = max(1, min(args.steps, 5))
@@ -618,7 +645,13 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=12.0, help="seconds of CPU-baseline sample at N=1")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-scan-roofline", action="store_true", help="skip the brute-force-scan roofline band")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the frame of the last timed step as DIR/*.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU frame; --impl reference has none")
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs at least one timed step")
     claim_stdout()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

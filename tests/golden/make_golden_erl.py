@@ -11,7 +11,11 @@ restatement is involved:
     the rows no reference test pins (planes, triangles, shading, shadows, reflection, un-normalised
     plane normals, exact distance ties, several lights, a seeded random-sphere scene);
   * rays: nearest_object_intersecting_ray/2 (erl:300-346) for ray batches -> (list position, Distance);
-  * ppm: write_pixels_to_ppm/5 (erl:668-685) run on a pixel list, i.e. the reference's own quantisation.
+  * ppm: write_pixels_to_ppm/5 (erl:668-685) run on a pixel list, i.e. the reference's own quantisation;
+  * erl_scene.json: the term scene/0 (erl:618-665) returns, atoms as strings.  Its first version was written
+    from eraytracer_b200.scene.demo_scene(), which test_scene_function_of_the_source_is_the_demo_scene_of_the_package
+    held equal to the evaluated scene/0 from commit 7ea1da3 on (the package's demo scene has not changed since);
+    running this script writes it from the source.
 
 The file travels to the GPU box (the reference does not); tests/test_erl_reference.py holds the
 oracle, the product's PPM writer and the CUDA path to it.
@@ -80,6 +84,9 @@ def main():
     out["ppm"]["demo_8x6_d2"] = {"pixels": erlref.to_py([list(p[1]) for p in demo]), "text": "".join(m.files["demo.ppm"])}
     with open(os.path.join(HERE, "erl_reference.json"), "w") as fh:
         json.dump(out, fh)
+    with open(os.path.join(HERE, "erl_scene.json"), "w") as fh:
+        json.dump({"source": "scene/0 of raytracer.erl (erl:618-665) evaluated by oracle/erlref.py",
+                   "scene": erlref.to_py(m.call("scene"))}, fh)
     print("wrote erl_reference.json in %.0fs (%d function calls evaluated)" % (time.time() - t0, m.calls))
 
 

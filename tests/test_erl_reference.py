@@ -1,16 +1,15 @@
-"""Parity pinned to the reference's SOURCE TEXT.
+"""Parity pinned to what the reference's SOURCE TEXT computes.
 
-oracle/erlref.py evaluates /root/reference/raytracer.erl itself (tokeniser, parser, Erlang semantics) and is
-checked by the reference's own test-suite run_tests/0 (erl:736-1133).  tests/golden/erl_reference.json holds
+oracle/erlref.py evaluates the reference's raytracer.erl itself (tokeniser, parser, Erlang semantics); the
+reference's own test-suite run_tests/0 (erl:736-1133) passed under it.  tests/golden/erl_reference.json holds
 what the reference's functions returned under it for the scenes of tests/erl_scenes.py: whole images through
 raytraced_pixel_list_simple/4, nearest hits through nearest_object_intersecting_ray/2, and the text
-write_pixels_to_ppm/5 wrote.  Here:
-
-  * where the reference is mounted (this container, not the GPU box): the suite is run again, images are
-    re-rendered live and must equal the oracle and the committed file bit for bit;
-  * everywhere: the C oracle, the Python restatement, the product's PPM writer and (gpu) the CUDA path are held
-    to the committed values — all doubles bit for bit on the CPU side; RGB8 equal and |d| <= 1e-9 relative
-    for the GPU (its shading is the forward form, DESIGN.md "Exactness"), (list position, Distance bits) for rays.
+write_pixels_to_ppm/5 wrote; tests/golden/erl_scene.json holds the term its scene/0 returns
+(tests/golden/make_golden_erl.py regenerates both from the reference's source).
+Here the C oracle, the Python restatement, the product's PPM writer, the Erlang host module and (gpu) the
+CUDA path are held to the committed values — all doubles bit for bit on the CPU side; RGB8 equal and
+|d| <= 1e-9 relative for the GPU (its shading is the forward form, DESIGN.md "Exactness"), (list position,
+Distance bits) for rays.
 """
 import json
 import os
@@ -24,18 +23,10 @@ from erl_scenes import SCENES, scene_records
 from helpers import assert_double_parity, assert_image_parity, quantise
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference/raytracer.erl"
-needs_reference = pytest.mark.skipif(not os.path.exists(REF), reason="the reference source is not mounted here")
 
 with open(os.path.join(HERE, "golden", "erl_reference.json")) as _fh:
     GOLD = json.load(_fh)
 IMAGES = sorted(GOLD["images"])
-
-
-def _module():
-    from oracle import erlref
-    sys.setrecursionlimit(200000)
-    return erlref, erlref.load(REF)
 
 
 def _oracle(name, w, h, depth):
@@ -51,42 +42,27 @@ def _gold_pixels(key):
     return g, np.array(g["pixels"], dtype=np.float64)
 
 
-# ------------------------------------------------------------------ the evaluator itself (reference mounted)
-@needs_reference
-def test_the_references_own_suite_passes_under_the_evaluator():
-    erlref, m = _module()
-    assert m.call("run_tests") == erlref.Atom("ok")
-    log = "".join(m.out)
-    assert log.count(" - OK") == 18 and "FAILED" not in log and "Success!" in log
-    assert GOLD["run_tests"] == "ok"
+# ------------------------------------------------------------------ both restatements == reference
+def test_both_oracles_render_the_references_demo_image():
+    """demo_8x6_d2 is what the reference's raytraced_pixel_list_simple/4 returned for its own scene/0; the C oracle
+    (on the package's demo scene) and the Python restatement (on its own scene/0) must both return it."""
+    gold = np.array(GOLD["ppm"]["demo_8x6_d2"]["pixels"], dtype=np.float64)
+    assert np.array_equal(_oracle("demo", 8, 6, 2), gold)
+    img = [p[1] for p in pyoracle.raytraced_pixel_list_simple(8, 6, pyoracle.scene(), 2)]
+    assert np.array_equal(np.array(img, dtype=np.float64), gold)
 
 
-@needs_reference
-def test_live_render_from_the_source_equals_the_oracles_and_the_committed_file():
-    erlref, m = _module()
-    from erl_scenes import scene_terms
-    for name, (w, h, depth) in (("demo", (8, 6, 2)), ("stress", (6, 5, 2))):
-        px = m.call("raytraced_pixel_list_simple", w, h, scene_terms(m, name), depth)
-        live = np.array([[float(c) for c in p[1]] for p in px])
-        assert np.array_equal(live, _oracle(name, w, h, depth)), name
-    # one committed image regenerated: the file is what this reference produces
-    g, gold = _gold_pixels("demo_16x12_d5")
-    px = m.call("raytraced_pixel_list_simple", 16, 12, m.call("scene"), 5)
-    assert np.array_equal(np.array([[float(c) for c in p[1]] for p in px]), gold)
-    # the second restatement agrees too
-    sc_py = pyoracle.scene()
-    img = [p[1] for p in pyoracle.raytraced_pixel_list_simple(8, 6, sc_py, 2)]
-    px = m.call("raytraced_pixel_list_simple", 8, 6, m.call("scene"), 2)
-    assert np.array_equal(np.array(img, dtype=np.float64), np.array([[float(c) for c in p[1]] for p in px]))
-
-
-@needs_reference
 def test_scene_function_of_the_source_is_the_demo_scene_of_the_package():
-    erlref, m = _module()
+    """tests/golden/erl_scene.json holds the term the reference's scene/0 returns (atoms as strings); every record,
+    material and value of the package's demo scene and of the Python restatement's scene/0 must equal it, hit by a
+    stored ray or not."""
     from eraytracer_b200 import scene as sc
     def plain(x):
         return [plain(y) for y in x] if isinstance(x, (tuple, list)) else x
-    assert erlref.to_py(m.call("scene")) == plain(sc.demo_scene())
+    with open(os.path.join(HERE, "golden", "erl_scene.json")) as fh:
+        want = json.load(fh)["scene"]
+    assert want == plain(sc.demo_scene())
+    assert want == plain(pyoracle.scene())
 
 
 # ------------------------------------------------------------------ oracle == reference (everywhere)
@@ -217,21 +193,23 @@ def _host_module():
         return erlref, erlref.Module(fh.read(), name="raytracer_gpu")
 
 
-@needs_reference
 def test_erlang_tracing_function_returns_the_references_pixel_list():
     """erl/raytracer_gpu.erl cannot be loaded by a BEAM here; its sequential functions are EVALUATED by oracle/erlref.py
     with the NIFs replaced by stand-ins that answer what the real ones answer (scene_upload -> {ok, Handle},
-    render_pixel_list -> the reference's own raytraced_pixel_list_simple/4 under the same evaluator).  The tracing
-    function must then return the reference's list — clause order, guards, ok_or_exit/1 and the case are the module's."""
+    render_pixel_list -> the pixel list the reference's raytraced_pixel_list_simple/4 returned for the demo scene at
+    8x6, depth 2: {1, Colour} per pixel, erl:86-99, colours from tests/golden/erl_reference.json).  The tracing
+    function must then return that list — clause order, guards, ok_or_exit/1 and the case are the module's."""
+    from erl_scenes import to_term
     erlref, host = _host_module()
-    _, ref = _module()
     A = erlref.Atom
-    scene = ref.call("scene")
+    scene = [to_term(None, e) for e in scene_records("demo")]
+    want = [(1, tuple(p)) for p in GOLD["ppm"]["demo_8x6_d2"]["pixels"]]
+    asked = []
     host.externals[("scene_upload", 2)] = lambda sc_, dev: (A("ok"), ("handle", sc_))
-    host.externals[("render_pixel_list", 5)] = lambda h, w, hh, d, opts: ref.call("raytraced_pixel_list_simple", w, hh, h[1], d)
+    host.externals[("render_pixel_list", 5)] = lambda h, w, hh, d, opts: asked.append((h, w, hh, d)) or want
     got = host.call("raytraced_pixel_list_gpu", 8, 6, scene, 2)
-    want = ref.call("raytraced_pixel_list_simple", 8, 6, scene, 2)
     assert len(got) == 48 and erlref.exact_eq(got, want)
+    assert len(asked) == 1 and erlref.exact_eq(asked[0], (("handle", scene), 8, 6, 2))
     assert host.call("raytraced_pixel_list_gpu", 0, 0, scene, 2) == A("done")          # erl:86-87
     assert host.call("raytraced_pixel_list_gpu_distributed", 0, 0, scene, 2) == A("done")
     with pytest.raises(erlref.ErlError, match="function_clause"):                    # the guards of erl:88-89

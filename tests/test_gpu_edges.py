@@ -278,6 +278,41 @@ def test_host_mirror_writes_the_reference_ppm(gpu, tmp_path):
     assert multi == single
 
 
+@pytest.mark.parametrize("workload", ["c1", "c5"])
+def test_bench_dumps_the_frame_of_its_last_timed_step(gpu, tmp_path, workload):
+    """bench.py --dump-outputs with two timed steps.  C1 (32x24) is written whole and is the RGB8 frame of the demo
+    scene.  C5 (7680x4320, camera pose k at step k) is written as a seeded sample of rows under 64 MB, and those rows
+    must show pose 1, the last timed step: not pose 0 (the untimed counting run and the first timed step) and not
+    pose 2 (the last warm-up frame on the same slot)."""
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", workload, "--steps", "2",
+                          "--warmup", "3", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=root)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout)["steps"] == 2
+    frame, rows = np.load(tmp_path / "frame.npy"), np.load(tmp_path / "frame_rows.npy")
+    assert frame.dtype == np.float32 and rows.dtype == np.float64
+    w, h, pose = (32, 24, None) if workload == "c1" else (7680, 4320, 1)
+    idx = rows.astype(np.int64)
+    assert np.array_equal(idx, rows) and np.all(np.diff(idx) > 0) and idx[0] >= 0 and idx[-1] < h
+    if workload == "c1":
+        assert idx.tolist() == list(range(h))
+    else:
+        assert len(idx) < h and frame.nbytes + rows.nbytes < 64_000_000
+    dev = sc.flatten(sc.demo_scene()).upload(0)
+    try:
+        def rows_of(k):
+            rgb8, _ = dev.render(w, h, 1, fmt="rgb8", camera=None if k is None else sc.pose_camera(k))
+            return rgb8[idx].astype(np.float32)
+        assert np.array_equal(frame, rows_of(pose))
+        if workload == "c5":
+            assert not np.array_equal(frame, rows_of(0)) and not np.array_equal(frame, rows_of(2))
+    finally:
+        dev.close()
+
+
 # ---- BASELINE.json's full sizes: size-independent properties -------------------------------
 def test_c3_full_4k_bvh_equals_linear_on_a_row_subset_and_oracle_on_a_lattice(gpu):
     flat = sc.synthetic_scene("c3")
