@@ -1,4 +1,4 @@
-// Binned-SAH builder for the sphere BVH.  See bvh_build.h.
+// Binned-SAH builder for the sphere and triangle BVHs.  See bvh_build.h.
 #include "bvh_build.h"
 
 #include <algorithm>
@@ -183,7 +183,7 @@ inline int32_t leaf_code(int32_t first, int32_t count) { return ~((first << 3) |
 
 }  // namespace
 
-void build_sphere_bvh(const double *centers, const double *radii, int64_t n, Bvh &out, int leaf_max, float trav_cost)
+void build_box_bvh(const float *boxes, const float *centroids, int64_t n, Bvh &out, int leaf_max, float trav_cost)
 {
     leaf_max = std::min(std::max(leaf_max, 1), 8);
     out.nodes.clear();
@@ -203,14 +203,12 @@ void build_sphere_bvh(const double *centers, const double *radii, int64_t n, Bvh
 
     Builder b;
     b.prim.resize((size_t)n);
-    b.cen.resize((size_t)n * 3);
+    b.cen.assign(centroids, centroids + (size_t)n * 3);
     b.idx.resize((size_t)n);
     for (int64_t i = 0; i < n; i++) {
         for (int a = 0; a < 3; a++) {
-            double c = centers[3 * i + a], r = std::fabs(radii[i]);
-            b.prim[(size_t)i].lo[a] = round_down(c - r);
-            b.prim[(size_t)i].hi[a] = round_up(c + r);
-            b.cen[3 * (size_t)i + a] = (float)c;
+            b.prim[(size_t)i].lo[a] = boxes[6 * i + a];
+            b.prim[(size_t)i].hi[a] = boxes[6 * i + 3 + a];
         }
         b.idx[(size_t)i] = (int32_t)i;
     }
@@ -264,6 +262,75 @@ void build_sphere_bvh(const double *centers, const double *radii, int64_t n, Bvh
         }
     }
     out.leaf_prim = std::move(b.idx);
+}
+
+void build_sphere_bvh(const double *centers, const double *radii, int64_t n, Bvh &out, int leaf_max, float trav_cost)
+{
+    std::vector<float> boxes((size_t)std::max<int64_t>(n, 0) * 6), cen((size_t)std::max<int64_t>(n, 0) * 3);
+    for (int64_t i = 0; i < n; i++) {
+        for (int a = 0; a < 3; a++) {
+            double c = centers[3 * i + a], r = std::fabs(radii[i]);
+            boxes[6 * (size_t)i + a] = round_down(c - r);
+            boxes[6 * (size_t)i + 3 + a] = round_up(c + r);
+            cen[3 * (size_t)i + a] = (float)c;
+        }
+    }
+    build_box_bvh(boxes.data(), cen.data(), n, out, leaf_max, trav_cost);
+}
+
+void build_triangle_bvh(const double *tris, int64_t n, TriBvh &out)
+{
+    out = TriBvh{};
+    // per triangle: largest edge (2-norm, as the literal test forms the edges) and largest |coordinate|
+    std::vector<double> edge((size_t)n), amax((size_t)n);
+    for (int64_t i = 0; i < n; i++) {
+        const double *v = tris + 9 * i;
+        double e = 0, m = 0;
+        for (int k = 0; k < 3; k++) {
+            const double *p = v + 3 * k, *q = v + 3 * ((k + 1) % 3);
+            double dx = q[0] - p[0], dy = q[1] - p[1], dz = q[2] - p[2];
+            e = std::max(e, std::sqrt(dx * dx + dy * dy + dz * dz));
+            for (int a = 0; a < 3; a++) m = std::max(m, std::fabs(p[a]));
+        }
+        edge[(size_t)i] = e;
+        amax[(size_t)i] = m;
+    }
+    // A tree triangle's prune margin grows with the largest edge and coordinate of the tree (tri_walk.h), so a
+    // triangle far larger than the typical one, or one whose box float cannot hold, is tested by every ray instead.
+    double median = 0;
+    if (n > 0) {
+        std::vector<double> s = edge;
+        std::nth_element(s.begin(), s.begin() + n / 2, s.end());
+        median = s[(size_t)n / 2];
+    }
+    const double edge_cap = kTriAlwaysEdge * median;
+    std::vector<int32_t> tree;
+    tree.reserve((size_t)n);
+    for (int64_t i = 0; i < n; i++) {
+        if (!(edge[(size_t)i] <= edge_cap) || !(amax[(size_t)i] <= kTriAlwaysAbs)) out.always.push_back((int32_t)i);
+        else tree.push_back((int32_t)i);
+    }
+    const size_t m = tree.size();
+    std::vector<float> boxes(m * 6), cen(m * 3);
+    for (size_t j = 0; j < m; j++) {
+        const double *v = tris + 9 * (size_t)tree[j];
+        for (int a = 0; a < 3; a++) {
+            double lo = std::min(v[a], std::min(v[3 + a], v[6 + a]));
+            double hi = std::max(v[a], std::max(v[3 + a], v[6 + a]));
+            boxes[6 * j + a] = round_down(lo);
+            boxes[6 * j + 3 + a] = round_up(hi);
+            cen[3 * j + a] = (float)(0.5 * lo + 0.5 * hi);
+        }
+        out.edge_max = std::max(out.edge_max, edge[(size_t)tree[j]]);
+        out.abs_max = std::max(out.abs_max, amax[(size_t)tree[j]]);
+    }
+    // the sqrt and the sums above are correctly rounded: one part in 2^40 covers them
+    out.edge_max *= 1.0 + 1.0 / 1099511627776.0;
+    build_box_bvh(boxes.data(), cen.data(), (int64_t)m, out.bvh, kBvhLeafMax, 0.f);
+    for (int32_t &p : out.bvh.leaf_prim) p = tree[(size_t)p];
+    out.leaf_tris.resize(m * 9);
+    for (size_t j = 0; j < m; j++)
+        std::copy(tris + 9 * (size_t)out.bvh.leaf_prim[j], tris + 9 * (size_t)out.bvh.leaf_prim[j] + 9, &out.leaf_tris[9 * j]);
 }
 
 }  // namespace ert

@@ -27,6 +27,9 @@
 // tile, no queue traffic); larger ones run the wavefront with the brute-force scan kernels.
 constexpr int kWfScanFrom = 192;
 
+// ERT_ACCEL_AUTO for a scene with a triangle BVH and few spheres (DESIGN.md "Triangle BVH": measured on m4)
+constexpr int kTriAutoAccel = ERT_ACCEL_BVH_MEGAKERNEL;
+
 #ifndef ERT_WF_REFILL_FROM
 #define ERT_WF_REFILL_FROM 2        /* first bounce whose path rays use the refilling kernel */
 #endif
@@ -71,6 +74,8 @@ struct HostScene {
     std::vector<float> sph_pairs;      // pair-interleaved, padded to whole scan tiles (ert_scan.cuh)
     std::vector<float> leaf_filter;    // [n][4]
     Bvh bvh;
+    TriBvh tbvh;                       // triangle BVH (n_tris >= kTriBvhMin); leaf-ordered vertices, always-list
+    bool has_tri_bvh = false;
     std::vector<LightGrid> lgrids;     // direction grids of the first lights (shadow queries)
     CellGrid cgrid;                    // uniform cell grid over the spheres (path rays)
     float r_max = 0, pad_c_max = 0, eta_c_max = 0, abs_max = 0;
@@ -285,6 +290,8 @@ int flatten(const ert_scene_desc *d, HostScene &h)
             build_sphere_bvh(centers.data(), radii.data(), h.n_spheres, h.bvh, kBvhLeafMax, kBvhTravCost);
         });
     }
+    h.has_tri_bvh = h.n_tris >= kTriBvhMin;
+    if (h.has_tri_bvh) builders.spawn([&h] { build_triangle_bvh(h.tris.data(), h.n_tris, h.tbvh); });
     if (h.n_spheres > 0) {
         double lo[3] = {DBL_MAX, DBL_MAX, DBL_MAX}, hi[3] = {-DBL_MAX, -DBL_MAX, -DBL_MAX};
         for (int64_t k = 0; k < h.n_spheres; k++)
@@ -337,6 +344,8 @@ int flatten(const ert_scene_desc *d, HostScene &h)
     // trees far below that, and a tree that is not must not be walked with a stack that silently drops subtrees
     if (h.bvh.depth >= kBvhStack)
         return fail(ERT_ERR_BADARG, "sphere BVH is deeper than the traversal stack");
+    if (h.has_tri_bvh && h.tbvh.bvh.depth >= kBvhStack)
+        return fail(ERT_ERR_BADARG, "triangle BVH is deeper than the traversal stack");
     h.leaf_filter.resize((size_t)h.n_spheres * 4);
     for (int64_t k = 0; k < h.n_spheres; k++)
         memcpy(&h.leaf_filter[(size_t)k * 4], &h.sph_filter[(size_t)h.bvh.leaf_prim[(size_t)k] * 4], 16);
@@ -385,6 +394,16 @@ int upload_scene(ert_scene *s)
     UP(h.leaf_filter, leaf_filter, float);
     UP(h.bvh.leaf_prim, leaf_sph, int);
     UP(h.bvh.nodes, nodes, BvhNode);
+    if (h.has_tri_bvh) {
+        UP(h.tbvh.bvh.nodes, tri_nodes, BvhNode);
+        UP(h.tbvh.leaf_tris, tri_leaf, double);
+        UP(h.tbvh.bvh.leaf_prim, tri_leaf_id, int);
+        UP(h.tbvh.always, tri_always, int);
+        d.n_tri_tree = (int)h.tbvh.bvh.leaf_prim.size();
+        d.n_tri_always = (int)h.tbvh.always.size();
+        d.tri_edge_max = h.tbvh.edge_max;
+        d.tri_abs_max = h.tbvh.abs_max;
+    }
 #undef UP
     {
         std::vector<LightGridDev> lg(h.lgrids.size());
@@ -460,6 +479,10 @@ int upload_scene(ert_scene *s)
     CU(cudaFuncSetAttribute(render_tiled_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                             2 * kTileSpheres * 16));
     CU(cudaFuncSetAttribute(render_tiled_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            2 * kTileSpheres * 16));
+    CU(cudaFuncSetAttribute(render_tiled_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            2 * kTileSpheres * 16));
+    CU(cudaFuncSetAttribute(render_tiled_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                             2 * kTileSpheres * 16));
     {
         cudaDeviceProp prop;
@@ -579,6 +602,8 @@ int pick_accel(const ert_scene *s, int requested)
 {
     if (requested == ERT_ACCEL_GRID) return s->host.cgrid.enabled ? ERT_ACCEL_GRID : ERT_ACCEL_BVH;
     if (requested != ERT_ACCEL_AUTO) return requested;
+    // a scene with a triangle BVH never goes to the linear triangle scan of ERT_ACCEL_EXACT (DESIGN.md "Triangle BVH")
+    if (s->host.has_tri_bvh && s->host.n_spheres <= 192) return kTriAutoAccel;
     if (s->host.n_spheres <= 16) return ERT_ACCEL_EXACT;
     if (s->host.n_spheres <= 192) return ERT_ACCEL_LINEAR;
     return s->host.cgrid.enabled ? ERT_ACCEL_GRID : ERT_ACCEL_BVH;
@@ -622,13 +647,27 @@ int copy_part_to_host(ert_scene *s, Slot &sl, const ert_render_params &p, void *
     return ERT_OK;
 }
 
-template <bool COUNT>
+template <bool COUNT, bool TRI>
 void launch_render(int accel, dim3 grid, cudaStream_t st, const DevScene &d, const FrameParams &fp)
 {
     switch (accel) {
-    case ERT_ACCEL_EXACT: render_free_kernel<1, COUNT><<<grid, 256, 0, st>>>(d, fp); break;
-    case ERT_ACCEL_LINEAR: render_tiled_kernel<COUNT><<<grid, 256, 2 * kTileSpheres * 16, st>>>(d, fp); break;
-    default: render_free_kernel<3, COUNT><<<grid, 256, 0, st>>>(d, fp); break;   // BVH megakernel (also depth 0)
+    case ERT_ACCEL_EXACT: render_free_kernel<1, COUNT><<<grid, 256, 0, st>>>(d, fp); break;    // the linear FP64 scan
+    case ERT_ACCEL_LINEAR: render_tiled_kernel<COUNT, TRI><<<grid, 256, 2 * kTileSpheres * 16, st>>>(d, fp); break;
+    default: render_free_kernel<3, COUNT, TRI><<<grid, 256, 0, st>>>(d, fp); break;   // BVH megakernel (also depth 0)
+    }
+}
+
+template <bool TRI>
+void launch_trace_rays(int accel, unsigned blocks, cudaStream_t st, const DevScene &d, long long n_rays, const double *rays,
+                       int *ord, double *t)
+{
+    switch (accel) {
+    case ERT_ACCEL_WARP: trace_rays_warp_kernel<TRI><<<(unsigned)((n_rays * 32 + 255) / 256), 256, 0, st>>>(d, n_rays, rays, ord, t); break;
+    case ERT_ACCEL_EXACT: trace_rays_kernel<1><<<blocks, 256, 0, st>>>(d, n_rays, rays, ord, t); break;    // the linear FP64 scan
+    case ERT_ACCEL_LINEAR: trace_rays_kernel<2, TRI><<<blocks, 256, 0, st>>>(d, n_rays, rays, ord, t); break;
+    case ERT_ACCEL_BVH_MEGAKERNEL: trace_rays_kernel<3, TRI><<<blocks, 256, 0, st>>>(d, n_rays, rays, ord, t); break;
+    case ERT_ACCEL_GRID: trace_rays_kernel<5, TRI><<<blocks, 256, 0, st>>>(d, n_rays, rays, ord, t); break;
+    default: trace_rays_kernel<4, TRI><<<blocks, 256, 0, st>>>(d, n_rays, rays, ord, t); break;
     }
 }
 
@@ -704,7 +743,7 @@ int wf_prepare(ert_scene *s, Slot &sl, const FrameParams &fp, WfBuf &wf, bool sc
     return ERT_OK;
 }
 
-template <bool COUNT>
+template <bool COUNT, bool TRI>
 int launch_wavefront(ert_scene *s, Slot &sl, const FrameParams &fp_in, bool unsorted, bool no_grid, bool timed,
                      bool scan, bool cells, uint64_t *launches)
 {
@@ -801,8 +840,8 @@ int launch_wavefront(ert_scene *s, Slot &sl, const FrameParams &fp_in, bool unso
         const bool emitted = !scan && (b == 0 || !sort);
         if (scan) {
             // planes/triangles seed every ray's result (counted with the other kernels), then every ray meets every sphere
-            if (b == 0) wf_scan_init<false, true, COUNT><<<s->wf_grid[3], 256, 0, st>>>(d, fp, wf, b);
-            else wf_scan_init<false, false, COUNT><<<s->wf_grid[3], 256, 0, st>>>(d, fp, wf, b);
+            if (b == 0) wf_scan_init<false, true, COUNT, TRI><<<s->wf_grid[3], 256, 0, st>>>(d, fp, wf, b);
+            else wf_scan_init<false, false, COUNT, TRI><<<s->wf_grid[3], 256, 0, st>>>(d, fp, wf, b);
             n++;
             TICK(2);
             if (b == 0) wf_scan<false, true, COUNT><<<s->wf_grid_scan, kScanThreads, kScanSmem, st>>>(d, fp, wf, b);
@@ -810,17 +849,17 @@ int launch_wavefront(ert_scene *s, Slot &sl, const FrameParams &fp_in, bool unso
         }
         else if (cells && b >= cells_from) {
             // path rays step through the cell grid (ERT_ACCEL_GRID)
-            if (b == 0) wf_trace_path<true, COUNT, true, true><<<s->wf_grid[4], kWfThreads, 0, st>>>(d, fp, wf, b);
-            else if (!refill && !emitted) wf_trace_path<false, COUNT, false, true><<<s->wf_grid[5], kWfThreads, 0, st>>>(d, fp, wf, b);
-            else if (!refill) wf_trace_path<false, COUNT, true, true><<<s->wf_grid[5], kWfThreads, 0, st>>>(d, fp, wf, b);
-            else if (!emitted) wf_trace_path_refill<COUNT, true, false><<<s->wf_grid[5], kWfThreads, 0, st>>>(d, fp, wf, b);
-            else wf_trace_path_refill<COUNT, true, true><<<s->wf_grid[5], kWfThreads, 0, st>>>(d, fp, wf, b);
+            if (b == 0) wf_trace_path<true, COUNT, true, true, TRI><<<s->wf_grid[4], kWfThreads, 0, st>>>(d, fp, wf, b);
+            else if (!refill && !emitted) wf_trace_path<false, COUNT, false, true, TRI><<<s->wf_grid[5], kWfThreads, 0, st>>>(d, fp, wf, b);
+            else if (!refill) wf_trace_path<false, COUNT, true, true, TRI><<<s->wf_grid[5], kWfThreads, 0, st>>>(d, fp, wf, b);
+            else if (!emitted) wf_trace_path_refill<COUNT, true, false, TRI><<<s->wf_grid[5], kWfThreads, 0, st>>>(d, fp, wf, b);
+            else wf_trace_path_refill<COUNT, true, true, TRI><<<s->wf_grid[5], kWfThreads, 0, st>>>(d, fp, wf, b);
         }
-        else if (b == 0) wf_trace_path<true, COUNT, true, false><<<s->wf_grid[0], kWfThreads, 0, st>>>(d, fp, wf, b);
-        else if (!refill && !emitted) wf_trace_path<false, COUNT, false, false><<<s->wf_grid[1], kWfThreads, 0, st>>>(d, fp, wf, b);
-        else if (!refill) wf_trace_path<false, COUNT, true, false><<<s->wf_grid[1], kWfThreads, 0, st>>>(d, fp, wf, b);
-        else if (!emitted) wf_trace_path_refill<COUNT, false, false><<<s->wf_grid[1], kWfThreads, 0, st>>>(d, fp, wf, b);
-        else wf_trace_path_refill<COUNT, false, true><<<s->wf_grid[1], kWfThreads, 0, st>>>(d, fp, wf, b);
+        else if (b == 0) wf_trace_path<true, COUNT, true, false, TRI><<<s->wf_grid[0], kWfThreads, 0, st>>>(d, fp, wf, b);
+        else if (!refill && !emitted) wf_trace_path<false, COUNT, false, false, TRI><<<s->wf_grid[1], kWfThreads, 0, st>>>(d, fp, wf, b);
+        else if (!refill) wf_trace_path<false, COUNT, true, false, TRI><<<s->wf_grid[1], kWfThreads, 0, st>>>(d, fp, wf, b);
+        else if (!emitted) wf_trace_path_refill<COUNT, false, false, TRI><<<s->wf_grid[1], kWfThreads, 0, st>>>(d, fp, wf, b);
+        else wf_trace_path_refill<COUNT, false, true, TRI><<<s->wf_grid[1], kWfThreads, 0, st>>>(d, fp, wf, b);
         n++;
         TICK(0);
         WF_CHECK("wf_trace_path");
@@ -854,14 +893,14 @@ int launch_wavefront(ert_scene *s, Slot &sl, const FrameParams &fp_in, bool unso
             CU(cudaStreamWaitEvent(st2, sl.ev_path[(size_t)b], 0));
         }
         if (scan) {
-            wf_scan_init<true, false, COUNT><<<s->wf_grid[3], 256, 0, st2>>>(d, fps, wf, b);
+            wf_scan_init<true, false, COUNT, TRI><<<s->wf_grid[3], 256, 0, st2>>>(d, fps, wf, b);
             n++;
             TICK(2);
             wf_scan<true, false, COUNT><<<s->wf_grid_scan, kScanThreads, kScanSmem, st2>>>(d, fps, wf, b);
         }
-        else if (fused_shade) wf_shadow_shade<COUNT><<<s->wf_grid[6], kWfThreads, 0, st2>>>(d, fps, wf, b);
-        else if (no_grid) wf_trace_shadow<COUNT, false><<<s->wf_grid[2], kWfThreads, 0, st2>>>(d, fps, wf, b);
-        else wf_trace_shadow<COUNT, true><<<s->wf_grid[2], kWfThreads, 0, st2>>>(d, fps, wf, b);
+        else if (fused_shade) wf_shadow_shade<COUNT, TRI><<<s->wf_grid[6], kWfThreads, 0, st2>>>(d, fps, wf, b);
+        else if (no_grid) wf_trace_shadow<COUNT, false, TRI><<<s->wf_grid[2], kWfThreads, 0, st2>>>(d, fps, wf, b);
+        else wf_trace_shadow<COUNT, true, TRI><<<s->wf_grid[2], kWfThreads, 0, st2>>>(d, fps, wf, b);
         TICK(1);
         WF_CHECK("wf_trace_shadow");
         if (scan) {
@@ -1108,14 +1147,25 @@ int ert_render_async(ert_scene *scene, const ert_render_params *params, int slot
         const bool unsorted = (p.flags & ERT_FLAG_WF_UNSORTED) != 0;
         const bool no_grid = (p.flags & ERT_FLAG_NO_LIGHT_GRID) != 0;
         const bool timed = (p.flags & ERT_FLAG_TIME_KERNELS) != 0;
-        rc = (p.flags & ERT_FLAG_COUNT_TESTS) ? launch_wavefront<true>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, &n)
-                                              : launch_wavefront<false>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, &n);
+        const bool count = (p.flags & ERT_FLAG_COUNT_TESTS) != 0;
+        if (scene->host.has_tri_bvh)
+            rc = count ? launch_wavefront<true, true>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, &n)
+                       : launch_wavefront<false, true>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, &n);
+        else
+            rc = count ? launch_wavefront<true, false>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, &n)
+                       : launch_wavefront<false, false>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, &n);
         if (rc != ERT_OK) return rc;
         sl.stats.gpu_launches = n;
     } else if (fp.local_rows > 0) {
         dim3 grid((unsigned)((p.width + 31) / 32), (unsigned)((fp.local_rows + 7) / 8));
-        if (p.flags & ERT_FLAG_COUNT_TESTS) launch_render<true>(accel, grid, sl.stream, scene->dev, fp);
-        else launch_render<false>(accel, grid, sl.stream, scene->dev, fp);
+        const bool count = (p.flags & ERT_FLAG_COUNT_TESTS) != 0;
+        if (scene->host.has_tri_bvh) {
+            if (count) launch_render<true, true>(accel, grid, sl.stream, scene->dev, fp);
+            else launch_render<false, true>(accel, grid, sl.stream, scene->dev, fp);
+        } else {
+            if (count) launch_render<true, false>(accel, grid, sl.stream, scene->dev, fp);
+            else launch_render<false, false>(accel, grid, sl.stream, scene->dev, fp);
+        }
         CU(cudaGetLastError());
         sl.stats.gpu_launches = 1;
     }
@@ -1218,17 +1268,12 @@ int ert_trace_rays(ert_scene *scene, int64_t n_rays, const double *rays6, int ac
         Slot &sl0 = scene->slots[0];
         timed = !sl0.busy;
         if (timed) TRY(cudaEventRecord(sl0.ev0, st));
-        switch (accel) {
-        case ERT_ACCEL_WARP:
-            if (n_rays > (1ll << 26)) { rc = fail(ERT_ERR_BADARG, "ERT_ACCEL_WARP takes at most 2^26 rays per call"); goto done; }
-            trace_rays_warp_kernel<<<(unsigned)((n_rays * 32 + 255) / 256), 256, 0, st>>>(scene->dev, n_rays, d_rays, d_ord, d_t);
-            break;
-        case ERT_ACCEL_EXACT: trace_rays_kernel<1><<<blocks, 256, 0, st>>>(scene->dev, n_rays, d_rays, d_ord, d_t); break;
-        case ERT_ACCEL_LINEAR: trace_rays_kernel<2><<<blocks, 256, 0, st>>>(scene->dev, n_rays, d_rays, d_ord, d_t); break;
-        case ERT_ACCEL_BVH_MEGAKERNEL: trace_rays_kernel<3><<<blocks, 256, 0, st>>>(scene->dev, n_rays, d_rays, d_ord, d_t); break;
-        case ERT_ACCEL_GRID: trace_rays_kernel<5><<<blocks, 256, 0, st>>>(scene->dev, n_rays, d_rays, d_ord, d_t); break;
-        default: trace_rays_kernel<4><<<blocks, 256, 0, st>>>(scene->dev, n_rays, d_rays, d_ord, d_t); break;
+        if (accel == ERT_ACCEL_WARP && n_rays > (1ll << 26)) {
+            rc = fail(ERT_ERR_BADARG, "ERT_ACCEL_WARP takes at most 2^26 rays per call");
+            goto done;
         }
+        if (scene->host.has_tri_bvh) launch_trace_rays<true>(accel, blocks, st, scene->dev, n_rays, d_rays, d_ord, d_t);
+        else launch_trace_rays<false>(accel, blocks, st, scene->dev, n_rays, d_rays, d_ord, d_t);
     }
     TRY(cudaGetLastError());
     if (timed) TRY(cudaEventRecord(scene->slots[0].ev1, st));

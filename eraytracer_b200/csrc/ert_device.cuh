@@ -16,6 +16,7 @@
 #include <stdint.h>
 
 #include "bvh_build.h"
+#include "tri_walk.h"
 
 namespace ert {
 
@@ -74,6 +75,13 @@ struct DevScene {
         float lo[3], hi[3];
         float cs, eps;
     } cg;
+    // BVH over triangles (scenes with >= kTriBvhMin triangles): walked by the kernels instantiated with TRI
+    const BvhNode *tri_nodes;
+    const double *tri_leaf;      // [slot][9] v1 v2 v3 in leaf order
+    const int *tri_leaf_id;      // leaf slot -> triangle index
+    const int *tri_always;       // triangles outside the tree: every ray tests them
+    int n_tri_tree, n_tri_always;
+    double tri_edge_max, tri_abs_max;   // the tree's constants of tri_walk.h
 };
 
 // One entry of a light's direction grid: 32 bytes, one 256-bit load.
@@ -248,19 +256,95 @@ struct Tally<false> {};
 #define PROBE(k, n) do { } while (0)
 #endif
 
-// planes and triangles (erl:353-356): always FP64, list order kept through `order`
+// one triangle through the literal test, folded into `best`
 template <bool COUNT>
+__device__ __forceinline__ void try_triangle(const DevScene &sc, d3 O, d3 D, const double *tr, int i, int skip_obj,
+                                             Hit &best, Tally<COUNT> &tl)
+{
+    int code = obj_code(OBJ_TRIANGLE, i);
+    if (code == skip_obj) return;
+    double t;
+    TALLY(exact_other);
+    if (triangle_exact(O, D, tr, t)) {
+        int ord = sc.tri_order[i];
+        if (better(t, ord, best)) { best.t = t; best.order = ord; best.obj = code; }
+    }
+}
+
+// The triangles of a scene with a triangle BVH (tri_walk.h): the always-list, then a front-to-back walk of the
+// whole line from -inf that leaves a node when its entry parameter is beyond the incumbent's cull.  With ANY the
+// walk stops at the first improvement of the incumbent (shadow queries, which start from their target).
+template <bool COUNT>
+__device__ __noinline__ void scan_tris_bvh(const DevScene &sc, d3 O, d3 D, Hit &best, int skip_obj, bool any,
+                                           Tally<COUNT> &tl)
+{
+    for (int k = 0; k < sc.n_tri_always; k++) {
+        const int i = __ldg(sc.tri_always + k);
+        try_triangle<COUNT>(sc, O, D, sc.tris + 9 * (size_t)i, i, skip_obj, best, tl);
+        if (any && best.obj != skip_obj) return;
+    }
+    const double Oa[3] = {O.x, O.y, O.z}, Da[3] = {D.x, D.y, D.z};
+    TriRay tr;
+    if (!tri_ray_setup(Oa, Da, sc.tri_edge_max, sc.tri_abs_max, true, tr)) {
+        // the bounds do not hold for this ray: every tree triangle
+        for (int k = 0; k < sc.n_tri_tree; k++) {
+            try_triangle<COUNT>(sc, O, D, sc.tri_leaf + 9 * (size_t)k, __ldg(sc.tri_leaf_id + k), skip_obj, best, tl);
+            if (any && best.obj != skip_obj) return;
+        }
+        return;
+    }
+    int stack[kBvhStack];
+    int sp = 0;
+    int node = 0;
+    double cull = tri_cull(tr, best.obj >= 0, best.t);
+    while (true) {
+        if (node >= 0) {
+            const float4 *np = reinterpret_cast<const float4 *>(sc.tri_nodes + node);
+            float4 a0 = __ldg(np), a1 = __ldg(np + 1), a2 = __ldg(np + 2);
+            int4 ch = __ldg(reinterpret_cast<const int4 *>(np + 3));
+            double tn0, tn1;
+            if constexpr (COUNT) tl.box += 2;
+            bool h0 = tri_slab(tr, a0.x, a0.y, a0.z, a0.w, a2.x, a2.y, cull, tn0);
+            bool h1 = tri_slab(tr, a1.x, a1.y, a1.z, a1.w, a2.z, a2.w, cull, tn1);
+            if (h0 && h1) {
+                bool swap = tn1 < tn0;
+                int nearc = swap ? ch.y : ch.x, farc = swap ? ch.x : ch.y;
+                if (sp < kBvhStack) stack[sp++] = farc;      // always true: ert_scene_create rejects trees of depth >= kBvhStack
+                node = nearc;
+                continue;
+            } else if (h0) { node = ch.x; continue; }
+            else if (h1) { node = ch.y; continue; }
+        } else {
+            int code = ~node;
+            int first = code >> 3, cnt = (code & 7) + 1;
+            for (int k = first; k < first + cnt; k++)
+                try_triangle<COUNT>(sc, O, D, sc.tri_leaf + 9 * (size_t)k, __ldg(sc.tri_leaf_id + k), skip_obj, best, tl);
+            if (any && best.obj != skip_obj) return;
+            cull = tri_cull(tr, best.obj >= 0, best.t);
+        }
+        if (sp == 0) return;
+        node = stack[--sp];
+    }
+}
+
+// planes and triangles (erl:353-356): always FP64, list order kept through `order`.  TRI: the scene has a
+// triangle BVH and its triangles are reached through scan_tris_bvh.
+template <bool COUNT, bool TRI = false>
 __device__ __forceinline__ void scan_others(const DevScene &sc, d3 O, d3 D, Hit &best, int skip_obj,
                                             Tally<COUNT> &tl)
 {
-    for (int i = 0; i < sc.n_tris; i++) {
-        int code = obj_code(OBJ_TRIANGLE, i);
-        if (code == skip_obj) continue;
-        double t;
-        TALLY(exact_other);
-        if (triangle_exact(O, D, sc.tris + 9 * i, t)) {
-            int ord = sc.tri_order[i];
-            if (better(t, ord, best)) { best.t = t; best.order = ord; best.obj = code; }
+    if constexpr (TRI) {
+        scan_tris_bvh<COUNT>(sc, O, D, best, skip_obj, false, tl);
+    } else {
+        for (int i = 0; i < sc.n_tris; i++) {
+            int code = obj_code(OBJ_TRIANGLE, i);
+            if (code == skip_obj) continue;
+            double t;
+            TALLY(exact_other);
+            if (triangle_exact(O, D, sc.tris + 9 * i, t)) {
+                int ord = sc.tri_order[i];
+                if (better(t, ord, best)) { best.t = t; best.order = ord; best.obj = code; }
+            }
         }
     }
     for (int i = 0; i < sc.n_planes; i++) {
@@ -279,18 +363,22 @@ __device__ __forceinline__ void scan_others(const DevScene &sc, d3 O, d3 D, Hit 
 // something beats its (Distance, list position).  A plane certainly farther than the target is dismissed before the
 // division of erl:468: with Vd < 0, Distance = V0 / Vd >= X  <=>  V0 <= X * Vd, and X = Distance(target) * (1 + 1e-9)
 // leaves seven decimal orders for the roundings of the products.  Everything nearer goes through the literal test.
-template <bool COUNT>
+template <bool COUNT, bool TRI = false>
 __device__ __forceinline__ void scan_others_shadow(const DevScene &sc, d3 O, d3 D, Hit &best, int skip_obj,
                                                    Tally<COUNT> &tl)
 {
-    for (int i = 0; i < sc.n_tris; i++) {
-        int code = obj_code(OBJ_TRIANGLE, i);
-        if (code == skip_obj) continue;
-        double t;
-        TALLY(exact_other);
-        if (triangle_exact(O, D, sc.tris + 9 * i, t)) {
-            int ord = sc.tri_order[i];
-            if (better(t, ord, best)) { best.t = t; best.order = ord; best.obj = code; }
+    if constexpr (TRI) {
+        scan_tris_bvh<COUNT>(sc, O, D, best, skip_obj, true, tl);
+    } else {
+        for (int i = 0; i < sc.n_tris; i++) {
+            int code = obj_code(OBJ_TRIANGLE, i);
+            if (code == skip_obj) continue;
+            double t;
+            TALLY(exact_other);
+            if (triangle_exact(O, D, sc.tris + 9 * i, t)) {
+                int ord = sc.tri_order[i];
+                if (better(t, ord, best)) { best.t = t; best.order = ord; best.obj = code; }
+            }
         }
     }
     for (int i = 0; i < sc.n_planes; i++) {
@@ -783,13 +871,13 @@ __device__ __forceinline__ void flush_counters(const FrameParams &fp, int rays, 
 }
 
 // resolve one query without block cooperation (EXACT and BVH strategies)
-template <int ACCEL, bool COUNT>
+template <int ACCEL, bool COUNT, bool TRI>
 __device__ __forceinline__ void resolve_free(const DevScene &sc, Query &q, Tally<COUNT> &tl)
 {
     if (!q.need) return;
     // a shadow query that starts from its target skips re-testing the target
     int skip = q.seed_obj;
-    scan_others<COUNT>(sc, q.O, q.D, q.best, skip, tl);
+    scan_others<COUNT, TRI>(sc, q.O, q.D, q.best, skip, tl);
     if (q.any && q.best.obj != q.seed_obj) return;
     if constexpr (ACCEL == 1) {
         double a = q.D.x * q.D.x + q.D.y * q.D.y + q.D.z * q.D.z;
@@ -802,7 +890,7 @@ __device__ __forceinline__ void resolve_free(const DevScene &sc, Query &q, Tally
 }
 
 // ------------------------------------------------------------------ kernels
-template <int ACCEL, bool COUNT>
+template <int ACCEL, bool COUNT, bool TRI = false>
 __global__ void __launch_bounds__(256)
 render_free_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ FrameParams fp)
 {
@@ -815,7 +903,7 @@ render_free_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ 
     while (__any_sync(0xffffffffu, p.alive)) {
         Query q;
         pix_prepare(p, sc, q);
-        resolve_free<ACCEL, COUNT>(sc, q, tl);
+        resolve_free<ACCEL, COUNT, TRI>(sc, q, tl);
         pix_consume(p, sc, fp, q);
     }
     if (inside) pix_store(p, fp, X, ly);
@@ -855,7 +943,7 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity)
         "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
 }
 
-template <bool COUNT>
+template <bool COUNT, bool TRI = false>
 __global__ void __launch_bounds__(256)
 render_tiled_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ FrameParams fp)
 {
@@ -889,7 +977,7 @@ render_tiled_kernel(const __grid_constant__ DevScene sc, const __grid_constant__
         FRay f;
         float cull = 0.f;
         if (active) {
-            scan_others<COUNT>(sc, q.O, q.D, q.best, skip, tl);
+            scan_others<COUNT, TRI>(sc, q.O, q.D, q.best, skip, tl);
             if (q.any && q.best.obj != q.seed_obj) active = false;
         }
         if (active) {
@@ -960,7 +1048,7 @@ __device__ void trace_ray_wavefront(const DevScene &sc, d3 O, d3 D, Hit &best); 
 __device__ void trace_ray_grid(const DevScene &sc, d3 O, d3 D, Hit &best);        // ert_wavefront.cuh
 
 // ---- ray batch: nearest_object_intersecting_ray/2 for arbitrary rays (tests, BVH == scan) ----
-template <int ACCEL>
+template <int ACCEL, bool TRI = false>
 __global__ void __launch_bounds__(256)
 trace_rays_kernel(const __grid_constant__ DevScene sc, long long n_rays, const double *__restrict__ rays6,
                   int *__restrict__ order_out, double *__restrict__ t_out)
@@ -975,7 +1063,7 @@ trace_rays_kernel(const __grid_constant__ DevScene sc, long long n_rays, const d
     Tally<false> tl;
     if constexpr (ACCEL == 2) {
         // same filter as the tiled kernel, spheres read straight from global memory
-        scan_others<false>(sc, q.O, q.D, q.best, -1, tl);
+        scan_others<false, TRI>(sc, q.O, q.D, q.best, -1, tl);
         FRay f;
         make_fray(sc, q.O, q.D, f, false);
         float cull = cull_from(f, q.best);
@@ -983,14 +1071,14 @@ trace_rays_kernel(const __grid_constant__ DevScene sc, long long n_rays, const d
             try_sphere<false>(sc, f, q.O, q.D, __ldg(sc.sph_filter + s), s, -1, q.best, cull, tl);
     } else if constexpr (ACCEL == 4) {
         // the traversal of the wavefront kernels (ert_wavefront.cuh)
-        scan_others<false>(sc, q.O, q.D, q.best, -1, tl);
+        scan_others<false, TRI>(sc, q.O, q.D, q.best, -1, tl);
         if (sc.n_spheres > 0) trace_ray_wavefront(sc, q.O, q.D, q.best);
     } else if constexpr (ACCEL == 5) {
         // the cell-grid walk of the wavefront's path kernels (ert_wavefront.cuh)
-        scan_others<false>(sc, q.O, q.D, q.best, -1, tl);
+        scan_others<false, TRI>(sc, q.O, q.D, q.best, -1, tl);
         if (sc.n_spheres > 0) trace_ray_grid(sc, q.O, q.D, q.best);
     } else {
-        resolve_free<ACCEL, false>(sc, q, tl);
+        resolve_free<ACCEL, false, TRI>(sc, q, tl);
     }
     order_out[i] = q.best.obj < 0 ? -1 : q.best.order;
     t_out[i] = q.best.obj < 0 ? 0.0 : q.best.t;
@@ -1006,6 +1094,7 @@ __device__ __forceinline__ unsigned long long sortable_bits(double t)
     const unsigned long long b = (unsigned long long)__double_as_longlong(t);
     return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
 }
+template <bool TRI = false>
 __global__ void __launch_bounds__(256)
 trace_rays_warp_kernel(const __grid_constant__ DevScene sc, long long n_rays, const double *__restrict__ rays6,
                        int *__restrict__ order_out, double *__restrict__ t_out)
@@ -1018,7 +1107,7 @@ trace_rays_warp_kernel(const __grid_constant__ DevScene sc, long long n_rays, co
     Tally<false> tl;
     Hit best;
     best.obj = -1; best.t = 0.0; best.order = 0x7fffffff;
-    if (lane == 0) scan_others<false>(sc, O, D, best, -1, tl);
+    if (lane == 0) scan_others<false, TRI>(sc, O, D, best, -1, tl);
     // every lane starts from lane 0's plane / triangle incumbent: it culls, and it is a candidate of the minimum
     best.t = __shfl_sync(0xffffffffu, best.t, 0);
     best.order = __shfl_sync(0xffffffffu, best.order, 0);

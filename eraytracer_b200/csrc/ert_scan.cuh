@@ -115,7 +115,7 @@ __device__ __forceinline__ void scan_ray_of_index(const DevScene &sc, const Fram
 // Before the scan, once per ray: planes and triangles (FP64, erl:353-356) seed the path ray's result; a shadow
 // ray's target is tested ("nearest == Object", erl:263, needs the target hit), its Distance kept for the
 // candidates to beat, and planes/triangles in front of it settle the ray at once.
-template <bool SHADOW, bool FIRST, bool COUNT>
+template <bool SHADOW, bool FIRST, bool COUNT, bool TRI = false>
 __global__ void __launch_bounds__(256)
 wf_scan_init(const __grid_constant__ DevScene sc, const __grid_constant__ FrameParams fp, const __grid_constant__ WfBuf wf,
              int bounce)
@@ -140,13 +140,13 @@ wf_scan_init(const __grid_constant__ DevScene sc, const __grid_constant__ FrameP
             bool occluded = true;
             if (object_exact(sc, target, O, D, a, t)) {
                 best.t = t; best.order = target_order; best.obj = target;
-                scan_others_shadow<COUNT>(sc, O, D, best, target, tl);
+                scan_others_shadow<COUNT, TRI>(sc, O, D, best, target, tl);
                 occluded = best.obj != target;
             }
             wf.sp_occ[i] = occluded ? 1 : 0;
             wf.sp_t[i] = t;
         } else {
-            if (valid) scan_others<COUNT>(sc, O, D, best, -1, tl);
+            if (valid) scan_others<COUNT, TRI>(sc, O, D, best, -1, tl);
             ScanBest b;
             b.t = best.t; b.order = best.order; b.obj = valid ? best.obj : -2;       // -2: no ray here (padding pixel)
             wf.sp_best[i] = b;

@@ -1054,7 +1054,7 @@ __device__ __forceinline__ void prefetch_path_chunk(const WfBuf &wf, unsigned lo
 // its hits into hit records (what wf_emit_hits does from the result arrays) — the warp is back
 // together after every batch, so the FP64 of the hit location and normal runs on full warps and
 // the results never travel through HBM.
-template <bool FIRST, bool COUNT, bool EMIT, bool GRID>
+template <bool FIRST, bool COUNT, bool EMIT, bool GRID, bool TRI = false>
 __global__ void __launch_bounds__(kWfThreads, GRID ? ERT_GRID_MINBLOCKS : ERT_WF_MINBLOCKS)
 wf_trace_path(const __grid_constant__ DevScene sc, const __grid_constant__ FrameParams fp,
               const __grid_constant__ WfBuf wf, int bounce)
@@ -1096,7 +1096,7 @@ wf_trace_path(const __grid_constant__ DevScene sc, const __grid_constant__ Frame
                 path_ray_of_index(fp, wf, FIRST, i, O, D, pid, valid);
                 if (valid) {
                     rays++;
-                    scan_others<COUNT>(sc, O, D, best, -1, tl);
+                    scan_others<COUNT, TRI>(sc, O, D, best, -1, tl);
                     double a, inv;
                     make_sray(sc, O, D, f, a, inv);
                     ray.put(O, D, a, inv);
@@ -1187,7 +1187,7 @@ struct alignas(16) FinishedHit {
     int obj;
 };
 constexpr int kFinQueue = 64;   // up to 31 waiting + 32 lanes finishing in one step
-template <bool COUNT, bool GRID, bool EMIT>
+template <bool COUNT, bool GRID, bool EMIT, bool TRI = false>
 __global__ void __launch_bounds__(kWfThreads, GRID ? ERT_GRID_MINBLOCKS : ERT_WF_REFILL_MINBLOCKS)
 wf_trace_path_refill(const __grid_constant__ DevScene sc, const __grid_constant__ FrameParams fp,
                      const __grid_constant__ WfBuf wf, int bounce)
@@ -1266,7 +1266,7 @@ wf_trace_path_refill(const __grid_constant__ DevScene sc, const __grid_constant_
                     idx = i;
                     rays++;
                     best.obj = -1; best.t = 0.0; best.order = 0x7fffffff;
-                    scan_others<COUNT>(sc, O, D, best, -1, tl);
+                    scan_others<COUNT, TRI>(sc, O, D, best, -1, tl);
                     if (sc.n_spheres > 0) {
                         double a, inv;
                         make_sray(sc, O, D, f, a, inv);
@@ -1411,7 +1411,7 @@ wf_emit_hits(const __grid_constant__ DevScene sc, const __grid_constant__ FrameP
 // against the sphere that shadowed this lane's previous ray: any object that beats the target's
 // (t, order) settles the question (erl:263), so a neighbour's occluder usually ends the query
 // without a walk.
-template <bool COUNT, bool USE_GRID>
+template <bool COUNT, bool USE_GRID, bool TRI = false>
 __global__ void __launch_bounds__(kWfThreads, ERT_SHADOW_MINBLOCKS)
 wf_trace_shadow(const __grid_constant__ DevScene sc, const __grid_constant__ FrameParams fp,
                 const __grid_constant__ WfBuf wf, int bounce)
@@ -1473,7 +1473,7 @@ wf_trace_shadow(const __grid_constant__ DevScene sc, const __grid_constant__ Fra
                 if (object_exact(sc, target, O, D, a, t)) {
                     Hit best;
                     best.t = t; best.order = order; best.obj = target;
-                    scan_others_shadow<COUNT>(sc, O, D, best, target, tl);
+                    scan_others_shadow<COUNT, TRI>(sc, O, D, best, target, tl);
                     lit = best.obj == target;
                     if (lit && hint >= 0 && obj_code(OBJ_SPHERE, hint) != target) {
                         double th;
@@ -1719,7 +1719,7 @@ __device__ __forceinline__ bool shadow_blocked(const DevScene &sc, const LightGr
 #endif
 constexpr int kSsMaxLights = 8;                  // three bits of a pair's entry; ert_api.cu uses the kernel for <= 8 lights
 static_assert(kWfChunk <= 128, "a chunk's hits are numbered with seven bits");
-template <bool COUNT>
+template <bool COUNT, bool TRI = false>
 __global__ void __launch_bounds__(kWfThreads, ERT_SS_MINBLOCKS)
 wf_shadow_shade(const __grid_constant__ DevScene sc, const __grid_constant__ FrameParams fp,
                 const __grid_constant__ WfBuf wf, int bounce)
@@ -1798,7 +1798,7 @@ wf_shadow_shade(const __grid_constant__ DevScene sc, const __grid_constant__ Fra
                 if (object_exact(sc, tgt, O, D, a, t)) {
                     Hit best;
                     best.t = t; best.order = order; best.obj = tgt;
-                    scan_others_shadow<COUNT>(sc, O, D, best, tgt, tl);
+                    scan_others_shadow<COUNT, TRI>(sc, O, D, best, tgt, tl);
                     bool lit = best.obj == tgt;
                     if (lit && sc.n_spheres > 0) {
                         SRay f;

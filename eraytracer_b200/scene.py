@@ -225,3 +225,111 @@ def pose_camera(k, n_poses=64):
     cam.fov = 90.0
     cam.screen_width, cam.screen_height = 4.0, 3.0
     return cam
+
+
+# ---------------------------------------------------------------------------
+# Triangle meshes.  A mesh of a million faces goes straight from index arrays to the
+# triangle table, without one Erlang-shaped tuple per face.
+# ---------------------------------------------------------------------------
+def mesh_triangles(vertices, faces, material, first_order):
+    """vertices (V, 3) numbers, faces (F, 3) vertex indices, material ((r, g, b), specular_power, shininess,
+    reflectivity) -> a TRIANGLE_DT table whose rows are the faces in order, list positions first_order,
+    first_order + 1, ...  Equal to flatten() of the same faces written as #triangle{} records."""
+    v = np.asarray(vertices, dtype=np.float64)
+    f = np.asarray(faces)
+    if v.ndim != 2 or v.shape[1] != 3 or f.ndim != 2 or f.shape[1] != 3:
+        raise _lib.BadArg(_lib.ERT_ERR_BADARG, "vertices and faces must be (n, 3) arrays")
+    if not np.issubdtype(f.dtype, np.integer):
+        raise _lib.BadArg(_lib.ERT_ERR_BADARG, "faces must hold vertex indices")
+    if len(f) and (f.min() < 0 or f.max() >= len(v)):
+        raise _lib.BadArg(_lib.ERT_ERR_BADARG, "a face refers to a vertex that does not exist")
+    colour, sp, sh, refl = material
+    t = np.zeros(len(f), dtype=_lib.TRIANGLE_DT)
+    t['v1'], t['v2'], t['v3'] = v[f[:, 0]], v[f[:, 1]], v[f[:, 2]]
+    t['material']['colour'] = [_num(c) for c in colour]
+    t['material']['specular_power'] = _num(sp)
+    t['material']['shininess'] = _num(sh)
+    t['material']['reflectivity'] = _num(refl)
+    t['order'] = np.arange(first_order, first_order + len(f), dtype=np.int32)
+    return t
+
+
+def _icosphere(level):
+    """Unit icosphere: (vertices, faces), faces wound so that (v2 - v1) x (v3 - v1) points outwards."""
+    p = (1.0 + math.sqrt(5.0)) / 2.0
+    verts = [(-1, p, 0), (1, p, 0), (-1, -p, 0), (1, -p, 0), (0, -1, p), (0, 1, p), (0, -1, -p), (0, 1, -p),
+             (p, 0, -1), (p, 0, 1), (-p, 0, -1), (-p, 0, 1)]
+    verts = [tuple(c / math.sqrt(1 + p * p) for c in v) for v in verts]
+    faces = [(0, 11, 5), (0, 5, 1), (0, 1, 7), (0, 7, 10), (0, 10, 11), (1, 5, 9), (5, 11, 4), (11, 10, 2),
+             (10, 7, 6), (7, 1, 8), (3, 9, 4), (3, 4, 2), (3, 2, 6), (3, 6, 8), (3, 8, 9), (4, 9, 5), (2, 4, 11),
+             (6, 2, 10), (8, 6, 7), (9, 8, 1)]
+    for _ in range(level):
+        mid = {}
+
+        def m(a, b):
+            key = (min(a, b), max(a, b))
+            if key not in mid:
+                x = [(verts[a][k] + verts[b][k]) / 2 for k in range(3)]
+                n = math.sqrt(sum(c * c for c in x))
+                verts.append(tuple(c / n for c in x))
+                mid[key] = len(verts) - 1
+            return mid[key]
+        nf = []
+        for a, b, c in faces:
+            ab, bc, ca = m(a, b), m(b, c), m(c, a)
+            nf += [(a, ab, ca), (b, bc, ab), (c, ca, bc), (ab, bc, ca)]
+        faces = nf
+    v = np.array(verts)
+    f = np.array(faces, dtype=np.int64)
+    n = np.cross(v[f[:, 1]] - v[f[:, 0]], v[f[:, 2]] - v[f[:, 0]])
+    inward = np.einsum('ij,ij->i', n, v[f].mean(axis=1)) < 0
+    f[inward] = f[inward][:, [0, 2, 1]]
+    return v, f
+
+
+def _f1(x):
+    return float(np.float32(x))
+
+
+MESH_CONFIGS = {
+    # name: (C3 spheres, heightfield cells per side, icospheres, icosphere level, seed)
+    "m3": (3000, 64, 10, 3, 0xE7A9C0DE00000103),
+    "m4": (10_000, 512, 24, 5, 0xE7A9C0DE00000104),
+}
+
+
+def mesh_scene(name="m3", n_triangles=None):
+    """Triangle-mesh workload: the camera, lights and plane of synthetic_scene, the spheres of the C3 recipe,
+    a heightfield sheet over the floor and closed icosphere meshes among the spheres (their back faces put
+    entry faces behind reflection and shadow rays).  Both meshes face the camera and the outside.  Every value
+    is float32-rounded and drawn from splitmix64_uniform.  List order: lights, spheres, triangles, plane.
+    n_triangles keeps the first that many triangles (scenes either side of the triangle-BVH threshold)."""
+    n_sph, cells, n_ico, level, seed = MESH_CONFIGS[name]
+    base = synthetic_scene("c3", n_spheres=n_sph)
+    u = splitmix64_uniform(seed, 4 + 8 * n_ico)
+    # heightfield sheet 0.5 above the floor (y = 5): y grows downwards, so faces wound with (e1 x e2).y < 0
+    xs = np.linspace(-40.0, 40.0, cells + 1)
+    zs = np.linspace(5.0, 85.0, cells + 1)
+    X, Z = np.meshgrid(xs, zs, indexing='ij')
+    Y = 4.5 - 0.4 * (np.sin(X * (0.3 + u[0] * 0.2)) * np.cos(Z * (0.3 + u[1] * 0.2)) + 1.0)
+    sheet_v = _f32(np.stack([X, Y, Z], axis=-1).reshape(-1, 3))
+    idx = np.arange((cells + 1) * (cells + 1)).reshape(cells + 1, cells + 1)
+    p00, p10, p01, p11 = idx[:-1, :-1].ravel(), idx[1:, :-1].ravel(), idx[:-1, 1:].ravel(), idx[1:, 1:].ravel()
+    sheet_f = np.stack([np.stack([p00, p10, p01], 1), np.stack([p10, p11, p01], 1)], 1).reshape(-1, 3)
+    first = 3 + n_sph
+    tabs = [mesh_triangles(sheet_v, sheet_f, ((_f1(0.6), _f1(0.55), _f1(0.5)), 4.0, _f1(0.2), _f1(0.1)), first)]
+    first += len(sheet_f)
+    ico_v, ico_f = _icosphere(level)
+    for k in range(n_ico):
+        r = u[4 + 8 * k: 12 + 8 * k]
+        c = (-35.0 + 70.0 * r[0], -25.0 + 26.0 * r[1], 10.0 + 70.0 * r[2])
+        rad = 2.0 + 3.0 * r[3]
+        mat = ((_f1(r[4]), _f1(r[5]), _f1(r[6])), 20.0, _f1(0.5), _f1(0.2 + 0.5 * r[7]))
+        tabs.append(mesh_triangles(_f32(ico_v * rad + np.array(c)), ico_f, mat, first))
+        first += len(ico_f)
+    tris = np.concatenate(tabs)
+    if n_triangles is not None:
+        tris = tris[:int(n_triangles)].copy()
+    planes = base.planes.copy()
+    planes['order'] = 3 + n_sph + len(tris)
+    return FlatScene(base.camera, base.lights, base.spheres, tris, planes)
