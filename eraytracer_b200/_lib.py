@@ -20,6 +20,12 @@ FLAG_WF_UNSORTED = 2
 FLAG_NO_LIGHT_GRID = 4
 FLAG_TIME_KERNELS = 8
 MAX_SLOTS = 4
+UPDATE_REBUILD_GRIDS = 1
+UPDATE_REBUILD = 2
+# ert_update_info.changed / .done bits (include/ert_b200.h)
+UPDATE_CHANGED = ["camera", "lights", "light_pos", "spheres", "sphere_mat", "triangles", "triangle_mat", "planes"]
+UPDATE_DONE = ["refit_spheres", "refit_triangles", "drop_cell_grid", "drop_light_grids", "rebuild_cell_grid",
+               "rebuild_light_grids", "rebuild_tri_bvh", "rebuild"]
 
 FORMATS = {"rgb8": FMT_RGB8, "f32": FMT_F32, "f64": FMT_F64}
 FORMAT_DTYPES = {FMT_RGB8: np.uint8, FMT_F32: np.float32, FMT_F64: np.float64}
@@ -83,6 +89,19 @@ class Stats(ctypes.Structure):
         return d
 
 
+class UpdateInfo(ctypes.Structure):
+    _fields_ = [("changed", ctypes.c_uint32), ("done", ctypes.c_uint32), ("has_cell_grid", ctypes.c_int32),
+                ("light_grids", ctypes.c_int32), ("light_grids_rebuilt", ctypes.c_int32), ("reserved", ctypes.c_int32),
+                ("h2d_bytes", ctypes.c_uint64), ("host_ms", ctypes.c_double), ("device_ms", ctypes.c_double),
+                ("sphere_area_ratio", ctypes.c_double), ("triangle_area_ratio", ctypes.c_double)]
+
+    def as_dict(self):
+        d = {n: getattr(self, n) for n, _ in self._fields_ if n != "reserved"}
+        d["changed"] = [n for k, n in enumerate(UPDATE_CHANGED) if self.changed >> k & 1]
+        d["done"] = [n for k, n in enumerate(UPDATE_DONE) if self.done >> k & 1]
+        return d
+
+
 # numpy views of the element records (same layout as the C structs)
 MATERIAL_DT = np.dtype([("colour", "<f8", 3), ("specular_power", "<f8"), ("shininess", "<f8"),
                         ("reflectivity", "<f8")])
@@ -102,6 +121,7 @@ EXPORTS = [
     "ert_scene_destroy", "ert_render", "ert_render_async", "ert_wait", "ert_download",
     "ert_get_stats", "ert_trace_rays", "ert_host_alloc", "ert_host_free", "ert_host_register",
     "ert_host_unregister", "ert_fp32_peak", "ert_fp32_peak_rrr", "ert_fp64_peak", "ert_d2h_peak", "ert_l2_flush",
+    "ert_scene_update",
 ]
 
 _lib = None
@@ -124,6 +144,7 @@ def load():
     L.ert_scene_create.argtypes = [ctypes.POINTER(SceneDesc), ctypes.c_int, ctypes.POINTER(vp)]
     L.ert_scene_clone.argtypes = [vp, ctypes.c_int, ctypes.POINTER(vp)]
     L.ert_scene_destroy.argtypes = [vp]
+    L.ert_scene_update.argtypes = [vp, ctypes.POINTER(SceneDesc), ctypes.c_uint32, ctypes.POINTER(UpdateInfo)]
     L.ert_render.argtypes = [vp, ctypes.POINTER(RenderParams), vp, ctypes.c_size_t]
     L.ert_render_async.argtypes = [vp, ctypes.POINTER(RenderParams), ctypes.c_int, vp,
                                    ctypes.c_size_t]
@@ -189,9 +210,9 @@ class Scene:
         self.device = device
         self._tables = tables        # keeps the numpy tables alive during create
 
-    @classmethod
-    def create(cls, camera, lights, spheres, triangles, planes, device=0):
-        L = load()
+    @staticmethod
+    def _desc(camera, lights, spheres, triangles, planes):
+        """(SceneDesc, the contiguous tables it points into: keep them alive for the call)."""
         desc = SceneDesc()
         desc.camera = camera
         tabs = []
@@ -201,9 +222,24 @@ class Scene:
             tabs.append(arr)
             setattr(desc, "n_" + name, len(arr))
             setattr(desc, name, arr.ctypes.data if len(arr) else None)
+        return desc, tabs
+
+    @classmethod
+    def create(cls, camera, lights, spheres, triangles, planes, device=0):
+        desc, tabs = cls._desc(camera, lights, spheres, triangles, planes)
         h = ctypes.c_void_p()
-        check(L.ert_scene_create(ctypes.byref(desc), int(device), ctypes.byref(h)))
+        check(load().ert_scene_create(ctypes.byref(desc), int(device), ctypes.byref(h)))
         return cls(h, device)
+
+    def update(self, camera, lights, spheres, triangles, planes, rebuild_grids=False, rebuild=False):
+        """ert_scene_update: new values for the scene's elements (same counts, same `order` values per kind, tables in
+        any order).  Returns the ert_update_info as a dict; raises BadArg (scene untouched) on a shape mismatch, a
+        non-finite value or a duplicate `order`."""
+        desc, tabs = self._desc(camera, lights, spheres, triangles, planes)
+        flags = (UPDATE_REBUILD_GRIDS if rebuild_grids else 0) | (UPDATE_REBUILD if rebuild else 0)
+        info = UpdateInfo()
+        check(load().ert_scene_update(self.handle, ctypes.byref(desc), flags, ctypes.byref(info)))
+        return info.as_dict()
 
     def clone(self, device):
         h = ctypes.c_void_p()

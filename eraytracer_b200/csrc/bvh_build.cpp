@@ -8,21 +8,10 @@
 #include <future>
 #include <thread>
 
+#include "scene_math.h"
+
 namespace ert {
 namespace {
-
-inline float round_down(double x)
-{
-    float f = (float)x;
-    if ((double)f > x) f = std::nextafterf(f, -INFINITY);
-    return f;
-}
-inline float round_up(double x)
-{
-    float f = (float)x;
-    if ((double)f < x) f = std::nextafterf(f, INFINITY);
-    return f;
-}
 
 struct Box {
     float lo[3], hi[3];
@@ -270,8 +259,8 @@ void build_sphere_bvh(const double *centers, const double *radii, int64_t n, Bvh
     for (int64_t i = 0; i < n; i++) {
         for (int a = 0; a < 3; a++) {
             double c = centers[3 * i + a], r = std::fabs(radii[i]);
-            boxes[6 * (size_t)i + a] = round_down(c - r);
-            boxes[6 * (size_t)i + 3 + a] = round_up(c + r);
+            boxes[6 * (size_t)i + a] = f_round_down(c - r);
+            boxes[6 * (size_t)i + 3 + a] = f_round_up(c + r);
             cen[3 * (size_t)i + a] = (float)c;
         }
     }
@@ -283,18 +272,7 @@ void build_triangle_bvh(const double *tris, int64_t n, TriBvh &out)
     out = TriBvh{};
     // per triangle: largest edge (2-norm, as the literal test forms the edges) and largest |coordinate|
     std::vector<double> edge((size_t)n), amax((size_t)n);
-    for (int64_t i = 0; i < n; i++) {
-        const double *v = tris + 9 * i;
-        double e = 0, m = 0;
-        for (int k = 0; k < 3; k++) {
-            const double *p = v + 3 * k, *q = v + 3 * ((k + 1) % 3);
-            double dx = q[0] - p[0], dy = q[1] - p[1], dz = q[2] - p[2];
-            e = std::max(e, std::sqrt(dx * dx + dy * dy + dz * dz));
-            for (int a = 0; a < 3; a++) m = std::max(m, std::fabs(p[a]));
-        }
-        edge[(size_t)i] = e;
-        amax[(size_t)i] = m;
-    }
+    for (int64_t i = 0; i < n; i++) triangle_extent(tris + 9 * i, edge[(size_t)i], amax[(size_t)i]);
     // A tree triangle's prune margin grows with the largest edge and coordinate of the tree (tri_walk.h), so a
     // triangle far larger than the typical one, or one whose box float cannot hold, is tested by every ray instead.
     double median = 0;
@@ -314,11 +292,10 @@ void build_triangle_bvh(const double *tris, int64_t n, TriBvh &out)
     std::vector<float> boxes(m * 6), cen(m * 3);
     for (size_t j = 0; j < m; j++) {
         const double *v = tris + 9 * (size_t)tree[j];
+        triangle_box(v, &boxes[6 * j], &boxes[6 * j + 3]);
         for (int a = 0; a < 3; a++) {
             double lo = std::min(v[a], std::min(v[3 + a], v[6 + a]));
             double hi = std::max(v[a], std::max(v[3 + a], v[6 + a]));
-            boxes[6 * j + a] = round_down(lo);
-            boxes[6 * j + 3 + a] = round_up(hi);
             cen[3 * j + a] = (float)(0.5 * lo + 0.5 * hi);
         }
         out.edge_max = std::max(out.edge_max, edge[(size_t)tree[j]]);

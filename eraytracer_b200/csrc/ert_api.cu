@@ -5,6 +5,7 @@
 
 #include <algorithm>
 #include <cfloat>
+#include <chrono>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -22,6 +23,8 @@
 #include "ert_device.cuh"
 #include "ert_wavefront.cuh"
 #include "ert_scan.cuh"
+#include "ert_update.cuh"
+#include "scene_math.h"
 
 // ERT_ACCEL_LINEAR: scenes up to this many spheres stay in the single-launch tiled kernel (one resident
 // tile, no queue traffic); larger ones run the wavefront with the brute-force scan kernels.
@@ -62,6 +65,7 @@ int cuda_fail(cudaError_t e, const char *what)
 struct HostScene {
     ert_camera camera;
     std::vector<double> lights;        // [n][9]
+    std::vector<int> light_order;      // their list positions (ascending)
     std::vector<double> planes, plane_mat;
     std::vector<int> plane_order;
     std::vector<double> tris, tri_mat;
@@ -81,6 +85,18 @@ struct HostScene {
     float r_max = 0, pad_c_max = 0, eta_c_max = 0, abs_max = 0;
     float grid_lo[3] = {0, 0, 0}, grid_scale[3] = {0, 0, 0};
     int n_lights = 0, n_planes = 0, n_tris = 0, n_spheres = 0;
+    // ert_scene_update
+    bool derived_stale = false;        // filters, pairs, leaf filters, tree nodes, leaf vertices: the device holds the
+                                       // current ones (a clone downloads them)
+    bool cgrid_dropped = false;        // an update dropped the cell grid / direction grids (ERT_UPDATE_REBUILD_GRIDS
+    bool lgrids_dropped = false;       // builds them again)
+    double sph_build_area = 0, tri_build_area = 0;   // total child-box half area at the trees' last build (0: not yet taken)
+};
+
+// Node indices of a tree by depth, on the device (scene_math.h refit_levels), made on the first update.
+struct RefitPlan {
+    int *order = nullptr;
+    std::vector<int32_t> off;
 };
 
 struct Slot {
@@ -123,8 +139,17 @@ struct ert_scene {
     HostScene host;
     DevScene dev{};
     std::vector<void *> allocs;
+    std::vector<void *> cg_allocs, lg_allocs;   // the grids' arrays (an update may build them again)
+    uint64_t uploaded = 0;                      // bytes upload() has copied to the device
     Slot slots[ERT_MAX_SLOTS];
     std::mutex mu;
+    // ert_scene_update
+    bool broken = false;                        // a CUDA call failed during an update: renders refuse until one succeeds
+    unsigned char *staging = nullptr;           // pinned: the new element tables, then their uploads
+    size_t staging_cap = 0;
+    UpdateScalars *upd_dev = nullptr, *upd_host = nullptr;
+    cudaEvent_t upd_ev[2] = {nullptr, nullptr};
+    RefitPlan plan_sph, plan_tri;
 };
 
 namespace {
@@ -139,30 +164,37 @@ void push_mat(std::vector<double> &v, const ert_material &m)
 {
     v.insert(v.end(), {m.colour[0], m.colour[1], m.colour[2], m.specular_power, m.shininess, m.reflectivity});
 }
-float f_up(double x)
+float f_up(double x) { return f_round_up(x); }
+
+// the uniform grid that orders the wavefront queues, from the bounds of every [c - |r|, c + |r|]
+void set_sort_grid(HostScene &h, const double lo[3], const double hi[3])
 {
-    float f = (float)x;
-    if ((double)f < x) f = std::nextafterf(f, INFINITY);
-    return f;
+    for (int a = 0; a < 3; a++) {
+        double ext = hi[a] - lo[a];
+        h.grid_lo[a] = (float)lo[a];
+        h.grid_scale[a] = ext > 0 ? (float)((double)(1 << kSortBits) / ext) : 0.f;
+        if (!std::isfinite(h.grid_scale[a]) || !std::isfinite(h.grid_lo[a])) { h.grid_lo[a] = 0; h.grid_scale[a] = 0; }
+    }
 }
 
-// FP32 filter sphere {fl(c), R}: R >= r^2 with the slack the stage-1 bound needs
-// (DESIGN.md "Filter bounds"): r^2 (1 + 2^-18) + 16 r eta_c + 4 eta_c^2 / u.
-void make_filter_sphere(const double *c, double r, float out[4], float &pad_c, float &eta_c)
+// direction-grid resolution (ERT_LIGHT_GRID_RES, 0 turns them off) and the number of lights that get one
+int light_grid_res()
 {
-    const double u = 5.9604644775390625e-8;
-    double eta = 0;
-    for (int a = 0; a < 3; a++) {
-        out[a] = (float)c[a];
-        eta = std::max(eta, std::fabs(c[a] - (double)out[a]));
-    }
-    eta *= 2.0;
-    r = std::fabs(r);
-    double pad = 16.0 * r * eta + 4.0 * eta * eta / u;
-    double R = r * r * (1.0 + 3.814697265625e-6) + pad;
-    out[3] = std::nextafterf(f_up(R), INFINITY);
-    pad_c = f_up(pad);
-    eta_c = f_up(eta);
+    int res = kLightGridRes;
+    if (const char *e = getenv("ERT_LIGHT_GRID_RES")) res = atoi(e);
+    return std::min(std::max(res, 0), 1024);
+}
+int light_grid_target(const HostScene &h, int res)
+{
+    return (res > 0 && h.n_spheres >= kLightGridMinSpheres) ? std::min(h.n_lights, kMaxLightGrids) : 0;
+}
+// ERT_CELL_GRID=0 turns the cell grid off, ERT_CELL_GRID_DENSITY = cells per sphere
+bool cell_grid_wanted(double &density)
+{
+    density = kCellGridDensity;
+    if (const char *e = getenv("ERT_CELL_GRID_DENSITY")) density = atof(e);
+    const char *off = getenv("ERT_CELL_GRID");
+    return !(off && atoi(off) == 0);
 }
 
 int flatten(const ert_scene_desc *d, HostScene &h)
@@ -206,6 +238,7 @@ int flatten(const ert_scene_desc *d, HostScene &h)
         const ert_point_light &l = d->lights[k];
         if (!finite3(l.diffuse_colour) || !finite3(l.location) || !finite3(l.specular_colour))
             return fail(ERT_ERR_BADARG, "point_light has a non-finite field");
+        h.light_order.push_back(l.order);
         h.lights.insert(h.lights.end(), {l.diffuse_colour[0], l.diffuse_colour[1], l.diffuse_colour[2], l.location[0],
                                          l.location[1], l.location[2], l.specular_colour[0], l.specular_colour[1],
                                          l.specular_colour[2]});
@@ -299,19 +332,12 @@ int flatten(const ert_scene_desc *d, HostScene &h)
                 lo[a] = std::min(lo[a], centers[(size_t)k * 3 + a] - std::fabs(radii[(size_t)k]));
                 hi[a] = std::max(hi[a], centers[(size_t)k * 3 + a] + std::fabs(radii[(size_t)k]));
             }
-        for (int a = 0; a < 3; a++) {
-            double ext = hi[a] - lo[a];
-            h.grid_lo[a] = (float)lo[a];
-            h.grid_scale[a] = ext > 0 ? (float)((double)(1 << kSortBits) / ext) : 0.f;
-            if (!std::isfinite(h.grid_scale[a]) || !std::isfinite(h.grid_lo[a])) { h.grid_lo[a] = 0; h.grid_scale[a] = 0; }
-        }
+        set_sort_grid(h, lo, hi);
     }
     {
-        // cell grid for the path rays; ERT_CELL_GRID=0 turns it off, ERT_CELL_GRID_DENSITY = cells per sphere
-        double density = kCellGridDensity;
-        if (const char *e = getenv("ERT_CELL_GRID_DENSITY")) density = atof(e);
-        const char *off = getenv("ERT_CELL_GRID");
-        if (!(off && atoi(off) == 0))
+        // cell grid for the path rays
+        double density;
+        if (cell_grid_wanted(density))
             builders.spawn([&h, &centers, &radii, density] {
                 build_cell_grid(centers.data(), radii.data(), h.sph_filter.data(), h.n_spheres, h.abs_max, density, h.cgrid);
             });
@@ -319,11 +345,9 @@ int flatten(const ert_scene_desc *d, HostScene &h)
     std::vector<char> lg_built;
     {
         // direction grids for shadow rays: worth their memory once a walk through the BVH costs more
-        // than a handful of candidate tests; ERT_LIGHT_GRID_RES=0 turns them off
-        int res = kLightGridRes;
-        if (const char *e = getenv("ERT_LIGHT_GRID_RES")) res = atoi(e);
-        res = std::min(std::max(res, 0), 1024);
-        int n_grids = (res > 0 && h.n_spheres >= kLightGridMinSpheres) ? std::min(h.n_lights, kMaxLightGrids) : 0;
+        // than a handful of candidate tests
+        const int res = light_grid_res();
+        const int n_grids = light_grid_target(h, res);
         h.lgrids.resize((size_t)n_grids);
         lg_built.assign((size_t)n_grids, 0);
         for (int g = 0; g < n_grids; g++)
@@ -352,20 +376,112 @@ int flatten(const ert_scene_desc *d, HostScene &h)
     return ERT_OK;
 }
 
+// owner: the list the allocation is freed from (the scene's tables by default)
 template <typename T>
-int upload(ert_scene *s, const std::vector<T> &v, const T **out)
+int upload(ert_scene *s, const std::vector<T> &v, const T **out, std::vector<void *> *owner = nullptr)
 {
     *out = nullptr;
     size_t bytes = std::max<size_t>(v.size() * sizeof(T), 16);
     void *p = nullptr;
     CU(cudaMalloc(&p, bytes));
-    s->allocs.push_back(p);
+    (owner ? owner : &s->allocs)->push_back(p);
     if (!v.empty()) CU(cudaMemcpy(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
+    s->uploaded += v.size() * sizeof(T);
     *out = (const T *)p;
     return ERT_OK;
 }
 
-int upload_scene(ert_scene *s)
+void free_all(std::vector<void *> &allocs)
+{
+    for (void *p : allocs) cudaFree(p);
+    allocs.clear();
+}
+
+// the direction grids of h.lgrids (replacing any the device had)
+int upload_light_grids(ert_scene *s)
+{
+    HostScene &h = s->host;
+    DevScene &d = s->dev;
+    int rc;
+    free_all(s->lg_allocs);
+    std::vector<void *> *own = &s->lg_allocs;
+    {
+        std::vector<LightGridDev> lg(h.lgrids.size());
+        for (size_t g = 0; g < h.lgrids.size(); g++) {
+            const LightGrid &G = h.lgrids[g];
+            std::vector<LightGridCand> cand(G.entries.size());
+            for (size_t e = 0; e < cand.size(); e++) {
+                LightGridCand &c = cand[e];
+                c.cx = G.fs[4 * e]; c.cy = G.fs[4 * e + 1]; c.cz = G.fs[4 * e + 2]; c.R = G.fs[4 * e + 3];
+                c.sphere = G.entries[e].sphere; c.dmin = G.entries[e].dmin; c.pad[0] = c.pad[1] = 0;
+            }
+            // per-cell heads: the nearest candidate inline, the rest by range
+            const size_t n_cells = G.cell_off.empty() ? 0 : G.cell_off.size() - 1;
+            std::vector<LightGridCand> head(n_cells);
+            for (size_t c = 0; c < n_cells; c++) {
+                const uint32_t e0 = G.cell_off[c], e1 = G.cell_off[c + 1];
+                LightGridCand &hd = head[c];
+                if (e0 < e1) {
+                    hd = cand[e0];
+                    hd.pad[0] = (int)(e0 + 1); hd.pad[1] = (int)e1;
+                } else {
+                    hd.cx = hd.cy = hd.cz = 0.f; hd.R = -3.0e38f; hd.sphere = -1; hd.dmin = INFINITY;
+                    hd.pad[0] = hd.pad[1] = 0;
+                }
+            }
+            const unsigned int *off; const LightGridCand *cd; const LightGridCand *hd; const int *al;
+            if ((rc = upload<unsigned int>(s, G.cell_off, &off, own)) != ERT_OK) return rc;
+            if ((rc = upload<LightGridCand>(s, cand, &cd, own)) != ERT_OK) return rc;
+            if ((rc = upload<LightGridCand>(s, head, &hd, own)) != ERT_OK) return rc;
+            if ((rc = upload<int>(s, G.always, &al, own)) != ERT_OK) return rc;
+            lg[g].cell_off = off; lg[g].cand = cd; lg[g].head = hd; lg[g].always = al;
+            lg[g].n_always = (int)G.always.size(); lg[g].res = G.res;
+        }
+        const LightGridDev *lgd;
+        if ((rc = upload<LightGridDev>(s, lg, &lgd, own)) != ERT_OK) return rc;
+        d.lgrids = lgd;
+        d.lg_count = (int)lg.size();
+    }
+    return ERT_OK;
+}
+
+// the cell grid of h.cgrid (replacing any the device had)
+int upload_cell_grid(ert_scene *s)
+{
+    HostScene &h = s->host;
+    DevScene &d = s->dev;
+    int rc;
+    free_all(s->cg_allocs);
+    std::vector<void *> *own = &s->cg_allocs;
+    {
+        const CellGrid &G = h.cgrid;
+        const CellBlock *blocks; const float *rf; const int *rs; const int *big;
+        if ((rc = upload<CellBlock>(s, G.blocks, &blocks, own)) != ERT_OK) return rc;
+        if ((rc = upload<float>(s, G.over_filter, &rf, own)) != ERT_OK) return rc;
+        if ((rc = upload<int>(s, G.over_sph, &rs, own)) != ERT_OK) return rc;
+        if ((rc = upload<int>(s, G.big, &big, own)) != ERT_OK) return rc;
+        d.cg.blocks = reinterpret_cast<const uint4 *>(blocks); d.cg.over_filter = reinterpret_cast<const float4 *>(rf);
+        d.cg.over_sph = rs; d.cg.big = big;
+        d.cg.n_big = (int)G.big.size(); d.cg.enabled = G.enabled ? 1 : 0;
+        d.cg.rx = G.res[0]; d.cg.ry = G.res[1]; d.cg.rz = G.res[2];
+        for (int a = 0; a < 3; a++) { d.cg.lo[a] = G.lo[a]; d.cg.hi[a] = G.hi[a]; }
+        d.cg.cs = G.cs; d.cg.eps = G.eps;
+    }
+    return ERT_OK;
+}
+
+// the scene constants of h in the kernels' parameter block
+void set_constants(ert_scene *s)
+{
+    HostScene &h = s->host;
+    DevScene &d = s->dev;
+    for (int a = 0; a < 3; a++) { d.grid_lo[a] = h.grid_lo[a]; d.grid_scale[a] = h.grid_scale[a]; }
+    d.r_max = h.r_max; d.pad_c_max = h.pad_c_max; d.eta_c_max = h.eta_c_max; d.abs_max = h.abs_max;
+    if (h.has_tri_bvh) { d.tri_edge_max = h.tbvh.edge_max; d.tri_abs_max = h.tbvh.abs_max; }
+}
+
+// every table, tree and grid of s->host to the device (the scene's streams are untouched)
+int upload_tables(ert_scene *s)
 {
     HostScene &h = s->host;
     DevScene &d = s->dev;
@@ -401,64 +517,19 @@ int upload_scene(ert_scene *s)
         UP(h.tbvh.always, tri_always, int);
         d.n_tri_tree = (int)h.tbvh.bvh.leaf_prim.size();
         d.n_tri_always = (int)h.tbvh.always.size();
-        d.tri_edge_max = h.tbvh.edge_max;
-        d.tri_abs_max = h.tbvh.abs_max;
     }
 #undef UP
-    {
-        std::vector<LightGridDev> lg(h.lgrids.size());
-        for (size_t g = 0; g < h.lgrids.size(); g++) {
-            const LightGrid &G = h.lgrids[g];
-            std::vector<LightGridCand> cand(G.entries.size());
-            for (size_t e = 0; e < cand.size(); e++) {
-                LightGridCand &c = cand[e];
-                c.cx = G.fs[4 * e]; c.cy = G.fs[4 * e + 1]; c.cz = G.fs[4 * e + 2]; c.R = G.fs[4 * e + 3];
-                c.sphere = G.entries[e].sphere; c.dmin = G.entries[e].dmin; c.pad[0] = c.pad[1] = 0;
-            }
-            // per-cell heads: the nearest candidate inline, the rest by range
-            const size_t n_cells = G.cell_off.empty() ? 0 : G.cell_off.size() - 1;
-            std::vector<LightGridCand> head(n_cells);
-            for (size_t c = 0; c < n_cells; c++) {
-                const uint32_t e0 = G.cell_off[c], e1 = G.cell_off[c + 1];
-                LightGridCand &hd = head[c];
-                if (e0 < e1) {
-                    hd = cand[e0];
-                    hd.pad[0] = (int)(e0 + 1); hd.pad[1] = (int)e1;
-                } else {
-                    hd.cx = hd.cy = hd.cz = 0.f; hd.R = -3.0e38f; hd.sphere = -1; hd.dmin = INFINITY;
-                    hd.pad[0] = hd.pad[1] = 0;
-                }
-            }
-            const unsigned int *off; const LightGridCand *cd; const LightGridCand *hd; const int *al;
-            if ((rc = upload<unsigned int>(s, G.cell_off, &off)) != ERT_OK) return rc;
-            if ((rc = upload<LightGridCand>(s, cand, &cd)) != ERT_OK) return rc;
-            if ((rc = upload<LightGridCand>(s, head, &hd)) != ERT_OK) return rc;
-            if ((rc = upload<int>(s, G.always, &al)) != ERT_OK) return rc;
-            lg[g].cell_off = off; lg[g].cand = cd; lg[g].head = hd; lg[g].always = al;
-            lg[g].n_always = (int)G.always.size(); lg[g].res = G.res;
-        }
-        const LightGridDev *lgd;
-        if ((rc = upload<LightGridDev>(s, lg, &lgd)) != ERT_OK) return rc;
-        d.lgrids = lgd;
-        d.lg_count = (int)lg.size();
-    }
-    {
-        const CellGrid &G = h.cgrid;
-        const CellBlock *blocks; const float *rf; const int *rs; const int *big;
-        if ((rc = upload<CellBlock>(s, G.blocks, &blocks)) != ERT_OK) return rc;
-        if ((rc = upload<float>(s, G.over_filter, &rf)) != ERT_OK) return rc;
-        if ((rc = upload<int>(s, G.over_sph, &rs)) != ERT_OK) return rc;
-        if ((rc = upload<int>(s, G.big, &big)) != ERT_OK) return rc;
-        d.cg.blocks = reinterpret_cast<const uint4 *>(blocks); d.cg.over_filter = reinterpret_cast<const float4 *>(rf);
-        d.cg.over_sph = rs; d.cg.big = big;
-        d.cg.n_big = (int)G.big.size(); d.cg.enabled = G.enabled ? 1 : 0;
-        d.cg.rx = G.res[0]; d.cg.ry = G.res[1]; d.cg.rz = G.res[2];
-        for (int a = 0; a < 3; a++) { d.cg.lo[a] = G.lo[a]; d.cg.hi[a] = G.hi[a]; }
-        d.cg.cs = G.cs; d.cg.eps = G.eps;
-    }
+    if ((rc = upload_light_grids(s)) != ERT_OK) return rc;
+    if ((rc = upload_cell_grid(s)) != ERT_OK) return rc;
     d.n_nodes = (int)h.bvh.nodes.size();
-    for (int a = 0; a < 3; a++) { d.grid_lo[a] = h.grid_lo[a]; d.grid_scale[a] = h.grid_scale[a]; }
-    d.r_max = h.r_max; d.pad_c_max = h.pad_c_max; d.eta_c_max = h.eta_c_max; d.abs_max = h.abs_max;
+    set_constants(s);
+    return ERT_OK;
+}
+
+int upload_scene(ert_scene *s)
+{
+    int rc;
+    if ((rc = upload_tables(s)) != ERT_OK) return rc;
     for (int i = 0; i < ERT_MAX_SLOTS; i++) {
         Slot &sl = s->slots[i];
         {
@@ -570,6 +641,15 @@ void destroy(ert_scene *s)
         if (sl.stream) cudaStreamDestroy(sl.stream);
     }
     for (void *p : s->allocs) cudaFree(p);
+    free_all(s->cg_allocs);
+    free_all(s->lg_allocs);
+    if (s->plan_sph.order) cudaFree(s->plan_sph.order);
+    if (s->plan_tri.order) cudaFree(s->plan_tri.order);
+    if (s->upd_dev) cudaFree(s->upd_dev);
+    if (s->upd_host) cudaFreeHost(s->upd_host);
+    if (s->staging) cudaFreeHost(s->staging);
+    for (cudaEvent_t e : s->upd_ev)
+        if (e) cudaEventDestroy(e);
     delete s;
 }
 
@@ -988,6 +1068,451 @@ int finish_slot(ert_scene *s, Slot &sl)
     return ERT_OK;
 }
 
+// ---- in-place update (ert_scene_update) ---------------------------------------------------------------------------
+
+// Scene element i (list position want[i]) is element map[i] of the new table; an empty map is the identity (the
+// caller lists the elements as the scene does, the animation case: one linear pass).
+template <typename E>
+int map_by_order(const E *tab, int64_t n, const std::vector<int> &want, const char *kind, std::vector<int64_t> &map)
+{
+    map.clear();
+    bool same = true;
+    for (int64_t i = 0; i < n && same; i++) same = tab[i].order == want[(size_t)i];
+    if (same) return ERT_OK;
+    std::vector<std::pair<int32_t, int64_t>> got((size_t)n), had((size_t)n);
+    for (int64_t i = 0; i < n; i++) {
+        got[(size_t)i] = {tab[i].order, i};
+        had[(size_t)i] = {want[(size_t)i], i};
+    }
+    std::sort(got.begin(), got.end());
+    std::sort(had.begin(), had.end());
+    for (size_t i = 1; i < got.size(); i++)
+        if (got[i].first == got[i - 1].first)
+            return fail(ERT_ERR_BADARG, std::string("duplicate list position in `order` among the ") + kind);
+    map.assign((size_t)n, 0);
+    for (size_t i = 0; i < got.size(); i++) {
+        if (got[i].first != had[i].first)
+            return fail(ERT_ERR_BADARG, std::string("the ") + kind + " do not have the list positions of the scene's create");
+        map[(size_t)had[i].second] = got[i].second;
+    }
+    return ERT_OK;
+}
+inline int64_t src_of(const std::vector<int64_t> &map, int64_t i) { return map.empty() ? i : map[(size_t)i]; }
+
+// The element tables an update may upload, in the order they sit in the staging buffer.
+enum { T_LIGHTS, T_PLANES, T_PLANE_MAT, T_TRIS, T_TRI_MAT, T_SPH_EXACT, T_SPH_MAT, T_SPH_REFL, T_COUNT };
+
+struct UpdateTables {
+    double *p[T_COUNT];
+    size_t n[T_COUNT];                 // doubles
+    bool changed[T_COUNT];
+    std::vector<double> *host[T_COUNT];
+    const void *dev[T_COUNT];
+};
+
+// Checks desc against the scene's list shape and every value, and writes the new tables into the staging buffer in
+// the scene's element order.  Nothing of the scene is written.
+int update_stage(ert_scene *s, const ert_scene_desc *d, UpdateTables &t)
+{
+    HostScene &h = s->host;
+    if (!d) return fail(ERT_ERR_BADARG, "scene descriptor is NULL");
+    if (d->n_lights != h.n_lights || d->n_spheres != h.n_spheres || d->n_triangles != h.n_tris ||
+        d->n_planes != h.n_planes)
+        return fail(ERT_ERR_BADARG, "element counts differ from the scene's (a new list shape needs ert_scene_create)");
+    if ((d->n_lights && !d->lights) || (d->n_spheres && !d->spheres) || (d->n_triangles && !d->triangles) ||
+        (d->n_planes && !d->planes))
+        return fail(ERT_ERR_BADARG, "element table pointer is NULL");
+    const ert_camera &c = d->camera;
+    if (!finite3(c.location) || !std::isfinite(c.fov) || !std::isfinite(c.screen_width) ||
+        !std::isfinite(c.screen_height))
+        return fail(ERT_ERR_BADARG, "camera has a non-finite field");
+    std::vector<int64_t> ml, ms, mt, mp;
+    int rc;
+    if ((rc = map_by_order(d->lights, d->n_lights, h.light_order, "lights", ml)) != ERT_OK) return rc;
+    if ((rc = map_by_order(d->spheres, d->n_spheres, h.sph_order, "spheres", ms)) != ERT_OK) return rc;
+    if ((rc = map_by_order(d->triangles, d->n_triangles, h.tri_order, "triangles", mt)) != ERT_OK) return rc;
+    if ((rc = map_by_order(d->planes, d->n_planes, h.plane_order, "planes", mp)) != ERT_OK) return rc;
+
+    const DevScene &dv = s->dev;
+    const size_t ns = (size_t)h.n_spheres, nt = (size_t)h.n_tris, np = (size_t)h.n_planes;
+    const size_t counts[T_COUNT] = {9 * (size_t)h.n_lights, 4 * np, 6 * np, 9 * nt, 6 * nt, 4 * ns, 6 * ns, ns};
+    std::vector<double> *host[T_COUNT] = {&h.lights, &h.planes, &h.plane_mat, &h.tris, &h.tri_mat,
+                                          &h.sph_exact, &h.sph_mat, &h.sph_refl};
+    const void *dev[T_COUNT] = {dv.lights, dv.planes, dv.plane_mat, dv.tris, dv.tri_mat, dv.sph_exact, dv.sph_mat,
+                                dv.sph_refl};
+    size_t total = 0;
+    for (int k = 0; k < T_COUNT; k++) total += counts[k];
+    if (s->staging_cap < total * sizeof(double)) {
+        if (s->staging) CU(cudaFreeHost(s->staging));
+        s->staging = nullptr;
+        s->staging_cap = 0;
+        if (cudaMallocHost(&s->staging, std::max<size_t>(total, 1) * sizeof(double)) != cudaSuccess) {
+            cudaGetLastError();
+            s->staging = nullptr;
+            return fail(ERT_ERR_NOMEM, "out of pinned host memory for the update's staging buffer");
+        }
+        s->staging_cap = total * sizeof(double);
+    }
+    double *p = (double *)s->staging;
+    for (int k = 0; k < T_COUNT; k++) {
+        t.p[k] = p;
+        t.n[k] = counts[k];
+        t.host[k] = host[k];
+        t.dev[k] = dev[k];
+        p += counts[k];
+    }
+    for (int64_t i = 0; i < d->n_lights; i++) {
+        const ert_point_light &l = d->lights[src_of(ml, i)];
+        if (!finite3(l.diffuse_colour) || !finite3(l.location) || !finite3(l.specular_colour))
+            return fail(ERT_ERR_BADARG, "point_light has a non-finite field");
+        double *o = t.p[T_LIGHTS] + 9 * i;
+        for (int a = 0; a < 3; a++) { o[a] = l.diffuse_colour[a]; o[3 + a] = l.location[a]; o[6 + a] = l.specular_colour[a]; }
+    }
+    auto mat = [](double *o, const ert_material &m) {
+        o[0] = m.colour[0]; o[1] = m.colour[1]; o[2] = m.colour[2];
+        o[3] = m.specular_power; o[4] = m.shininess; o[5] = m.reflectivity;
+    };
+    for (int64_t i = 0; i < d->n_planes; i++) {
+        const ert_plane &q = d->planes[src_of(mp, i)];
+        if (!finite3(q.normal) || !std::isfinite(q.distance) || !finite_mat(q.material))
+            return fail(ERT_ERR_BADARG, "plane has a non-finite field");
+        double *o = t.p[T_PLANES] + 4 * i;
+        o[0] = q.normal[0]; o[1] = q.normal[1]; o[2] = q.normal[2]; o[3] = q.distance;
+        mat(t.p[T_PLANE_MAT] + 6 * i, q.material);
+    }
+    for (int64_t i = 0; i < d->n_triangles; i++) {
+        const ert_triangle &q = d->triangles[src_of(mt, i)];
+        if (!finite3(q.v1) || !finite3(q.v2) || !finite3(q.v3) || !finite_mat(q.material))
+            return fail(ERT_ERR_BADARG, "triangle has a non-finite field");
+        double *o = t.p[T_TRIS] + 9 * i;
+        for (int a = 0; a < 3; a++) { o[a] = q.v1[a]; o[3 + a] = q.v2[a]; o[6 + a] = q.v3[a]; }
+        mat(t.p[T_TRI_MAT] + 6 * i, q.material);
+    }
+    for (int64_t i = 0; i < d->n_spheres; i++) {
+        const ert_sphere &q = d->spheres[src_of(ms, i)];
+        if (!finite3(q.center) || !std::isfinite(q.radius) || !finite_mat(q.material))
+            return fail(ERT_ERR_BADARG, "sphere has a non-finite field");
+        double *o = t.p[T_SPH_EXACT] + 4 * i;
+        o[0] = q.center[0]; o[1] = q.center[1]; o[2] = q.center[2]; o[3] = q.radius;
+        mat(t.p[T_SPH_MAT] + 6 * i, q.material);
+        t.p[T_SPH_REFL][i] = q.material.reflectivity;
+    }
+    for (int k = 0; k < T_COUNT; k++)
+        t.changed[k] = s->broken || (t.n[k] && memcmp(t.p[k], host[k]->data(), t.n[k] * sizeof(double)) != 0);
+    return ERT_OK;
+}
+
+int free_alloc(ert_scene *s, const void *p)
+{
+    auto it = std::find(s->allocs.begin(), s->allocs.end(), p);
+    if (it == s->allocs.end()) return ERT_OK;
+    s->allocs.erase(it);
+    CU(cudaFree(const_cast<void *>(p)));
+    return ERT_OK;
+}
+
+void drop_plan(RefitPlan &plan)
+{
+    if (plan.order) cudaFree(plan.order);
+    plan.order = nullptr;
+    plan.off.clear();
+}
+
+double tree_area(const std::vector<BvhNode> &nodes)
+{
+    double a = 0;
+    for (const BvhNode &n : nodes) a += child_half_area(n, 0) + child_half_area(n, 1);
+    return a;
+}
+
+// The refit schedule of a tree, made on its first refit, and its area at build (the host mirror still holds the
+// built nodes then).
+int ensure_plan(RefitPlan &plan, const std::vector<BvhNode> &nodes, double &build_area)
+{
+    if (plan.order) return ERT_OK;
+    std::vector<int32_t> order;
+    refit_levels(nodes, order, plan.off);
+    CU(cudaMalloc(&plan.order, std::max<size_t>(order.size(), 1) * sizeof(int32_t)));
+    CU(cudaMemcpy(plan.order, order.data(), order.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+    if (build_area == 0) build_area = tree_area(nodes);
+    return ERT_OK;
+}
+
+template <typename LeafBox>
+void launch_refit(const RefitPlan &plan, BvhNode *nodes, const LeafBox &leaf_box, double *area, cudaStream_t st)
+{
+    for (int lvl = (int)plan.off.size() - 2; lvl >= 0; lvl--) {
+        const int cnt = plan.off[(size_t)lvl + 1] - plan.off[(size_t)lvl];
+        if (cnt > 0)
+            upd_refit_level<<<(cnt + kUpdThreads - 1) / kUpdThreads, kUpdThreads, 0, st>>>(
+                nodes, plan.order + plan.off[(size_t)lvl], cnt, leaf_box, area);
+    }
+}
+
+// The arrays derived on the device by updates (filters, pairs, leaf filters, tree nodes, leaf vertices) from
+// src's device into h.
+int download_derived(const ert_scene *src, HostScene &h)
+{
+    const DevScene &d = src->dev;
+    CU(cudaSetDevice(src->device));
+    auto get = [](void *dst, const void *p, size_t bytes) -> int {
+        if (bytes) CU(cudaMemcpy(dst, p, bytes, cudaMemcpyDeviceToHost));
+        return ERT_OK;
+    };
+    int rc;
+    if ((rc = get(h.sph_filter.data(), d.sph_filter, h.sph_filter.size() * sizeof(float))) != ERT_OK) return rc;
+    if ((rc = get(h.sph_pairs.data(), d.sph_pairs, h.sph_pairs.size() * sizeof(float))) != ERT_OK) return rc;
+    if ((rc = get(h.leaf_filter.data(), d.leaf_filter, h.leaf_filter.size() * sizeof(float))) != ERT_OK) return rc;
+    if ((rc = get(h.bvh.nodes.data(), d.nodes, h.bvh.nodes.size() * sizeof(BvhNode))) != ERT_OK) return rc;
+    if (h.has_tri_bvh) {
+        if ((rc = get(h.tbvh.bvh.nodes.data(), d.tri_nodes, h.tbvh.bvh.nodes.size() * sizeof(BvhNode))) != ERT_OK) return rc;
+        if ((rc = get(h.tbvh.leaf_tris.data(), d.tri_leaf, h.tbvh.leaf_tris.size() * sizeof(double))) != ERT_OK) return rc;
+    }
+    h.derived_stale = false;
+    return ERT_OK;
+}
+
+// A tree triangle left the float range of the boxes (kTriAlwaysAbs): the triangle BVH is built again on the host.
+int rebuild_tri_bvh(ert_scene *s)
+{
+    HostScene &h = s->host;
+    DevScene &d = s->dev;
+    TriBvh t;
+    build_triangle_bvh(h.tris.data(), h.n_tris, t);
+    if (t.bvh.depth >= kBvhStack) return fail(ERT_ERR_BADARG, "triangle BVH is deeper than the traversal stack");
+    int rc;
+    const void *old[4] = {d.tri_nodes, d.tri_leaf, d.tri_leaf_id, d.tri_always};
+    for (const void *p : old)
+        if ((rc = free_alloc(s, p)) != ERT_OK) return rc;
+    h.tbvh = std::move(t);
+    const BvhNode *nodes; const double *leaf; const int *id; const int *always;
+    if ((rc = upload(s, h.tbvh.bvh.nodes, &nodes)) != ERT_OK) return rc;
+    if ((rc = upload(s, h.tbvh.leaf_tris, &leaf)) != ERT_OK) return rc;
+    if ((rc = upload(s, h.tbvh.bvh.leaf_prim, &id)) != ERT_OK) return rc;
+    if ((rc = upload(s, h.tbvh.always, &always)) != ERT_OK) return rc;
+    d.tri_nodes = nodes; d.tri_leaf = leaf; d.tri_leaf_id = id; d.tri_always = always;
+    d.n_tri_tree = (int)h.tbvh.bvh.leaf_prim.size();
+    d.n_tri_always = (int)h.tbvh.always.size();
+    drop_plan(s->plan_tri);
+    h.tri_build_area = tree_area(h.tbvh.bvh.nodes);
+    return ERT_OK;
+}
+
+// ERT_UPDATE_REBUILD_GRIDS: the cell grid (cell) and the direction grids of `stale` lights, and any an earlier
+// update dropped, built again by the host builders from the current spheres.
+int rebuild_grids(ert_scene *s, bool cell, const std::vector<char> &stale, ert_update_info &inf)
+{
+    HostScene &h = s->host;
+    int rc;
+    if (h.derived_stale && (rc = download_derived(s, h)) != ERT_OK) return rc;
+    const size_t n = (size_t)h.n_spheres;
+    std::vector<double> centers(n * 3), radii(n);
+    for (size_t k = 0; k < n; k++) {
+        for (int a = 0; a < 3; a++) centers[k * 3 + a] = h.sph_exact[k * 4 + a];
+        radii[k] = h.sph_exact[k * 4 + 3];
+    }
+    const int res = light_grid_res();
+    const int n_target = light_grid_target(h, res);
+    const size_t have = h.lgrids.size();
+    std::vector<LightGrid> lg((size_t)n_target);
+    std::vector<char> built((size_t)n_target, 0);
+    int n_need = 0;
+    WorkerGroup builders;
+    for (int g = 0; g < n_target; g++) {
+        if ((size_t)g < have && !((size_t)g < stale.size() && stale[(size_t)g])) {
+            lg[(size_t)g] = std::move(h.lgrids[(size_t)g]);
+            built[(size_t)g] = 1;
+            continue;
+        }
+        n_need++;
+        builders.spawn([&h, &centers, &radii, &lg, &built, g, res] {
+            built[(size_t)g] = build_light_grid(centers.data(), radii.data(), h.sph_filter.data(), h.n_spheres,
+                                                &h.lights[(size_t)g * 9 + 3], res, lg[(size_t)g]) ? 1 : 0;
+        });
+    }
+    CellGrid cg;
+    double density;
+    const bool want_cell = cell && cell_grid_wanted(density);
+    if (want_cell)
+        builders.spawn([&h, &centers, &radii, &cg, density] {
+            build_cell_grid(centers.data(), radii.data(), h.sph_filter.data(), h.n_spheres, h.abs_max, density, cg);
+        });
+    builders.join();
+    if (cell) {
+        h.cgrid = std::move(cg);
+        h.cgrid_dropped = false;
+        if ((rc = upload_cell_grid(s)) != ERT_OK) return rc;
+        inf.done |= ERT_DID_REBUILD_CELL_GRID;
+    }
+    if (n_need > 0 || have < (size_t)n_target) {
+        size_t keep = 0;
+        while (keep < built.size() && built[keep]) keep++;
+        lg.resize(keep);
+        h.lgrids = std::move(lg);
+        h.lgrids_dropped = false;
+        if ((rc = upload_light_grids(s)) != ERT_OK) return rc;
+        inf.done |= ERT_DID_REBUILD_LIGHT_GRIDS;
+        inf.light_grids_rebuilt = n_need;
+    }
+    return ERT_OK;
+}
+
+// Everything after the checks: the host mirror takes the staged tables, the changed ones go to the device, the
+// kernels of ert_update.cuh recompute what create derived from them, and stale grids are dropped or rebuilt.
+void update_changes(const HostScene &h, const UpdateTables &t, const ert_camera &camera, ert_update_info &inf)
+{
+    for (int64_t i = 0; i < h.n_lights; i++)
+        if (memcmp(&t.p[T_LIGHTS][i * 9 + 3], &h.lights[(size_t)i * 9 + 3], 3 * sizeof(double)) != 0)
+            inf.changed |= ERT_CHANGED_LIGHT_POS;
+    if (memcmp(&camera, &h.camera, sizeof camera) != 0) inf.changed |= ERT_CHANGED_CAMERA;
+    const uint32_t bit[T_COUNT] = {ERT_CHANGED_LIGHTS, ERT_CHANGED_PLANES, ERT_CHANGED_PLANES, ERT_CHANGED_TRIANGLES,
+                                   ERT_CHANGED_TRIANGLE_MAT, ERT_CHANGED_SPHERES, ERT_CHANGED_SPHERE_MAT,
+                                   ERT_CHANGED_SPHERE_MAT};
+    for (int k = 0; k < T_COUNT; k++)
+        if (t.changed[k] && t.n[k]) inf.changed |= bit[k];
+}
+
+int update_apply(ert_scene *s, UpdateTables &t, const ert_camera &camera, uint32_t flags, ert_update_info &inf)
+{
+    HostScene &h = s->host;
+    DevScene &d = s->dev;
+    cudaStream_t st = s->slots[0].stream;
+    int rc;
+    const bool was_broken = s->broken;
+    const bool sph_geo = t.changed[T_SPH_EXACT] && h.n_spheres > 0;
+    const bool tri_geo = t.changed[T_TRIS] && h.has_tri_bvh && !h.tbvh.bvh.leaf_prim.empty();
+    // lights whose direction grid went stale
+    std::vector<char> lg_stale(h.lgrids.size(), 0);
+    for (size_t g = 0; g < h.lgrids.size(); g++)
+        lg_stale[g] = sph_geo || was_broken || memcmp(&t.p[T_LIGHTS][g * 9 + 3], &h.lights[g * 9 + 3], 3 * sizeof(double)) != 0;
+    s->broken = true;                 // until every step below has succeeded
+    h.camera = camera;
+    if (!s->upd_dev) CU(cudaMalloc(&s->upd_dev, sizeof(UpdateScalars)));
+    if (!s->upd_host) CU(cudaMallocHost(&s->upd_host, sizeof(UpdateScalars)));
+    if (sph_geo && (rc = ensure_plan(s->plan_sph, h.bvh.nodes, h.sph_build_area)) != ERT_OK) return rc;
+    if (tri_geo && (rc = ensure_plan(s->plan_tri, h.tbvh.bvh.nodes, h.tri_build_area)) != ERT_OK) return rc;
+
+    CU(cudaEventRecord(s->upd_ev[0], st));
+    for (int k = 0; k < T_COUNT; k++) {
+        if (!t.changed[k] || !t.n[k]) continue;
+        const size_t bytes = t.n[k] * sizeof(double);
+        memcpy(t.host[k]->data(), t.p[k], bytes);
+        CU(cudaMemcpyAsync(const_cast<void *>(t.dev[k]), t.p[k], bytes, cudaMemcpyHostToDevice, st));
+        inf.h2d_bytes += bytes;
+    }
+    UpdateScalars &u = *s->upd_host;
+    memset(&u, 0, sizeof u);
+    for (int a = 0; a < 3; a++) u.lo[a] = ~0ull;
+    CU(cudaMemcpyAsync(s->upd_dev, &u, sizeof u, cudaMemcpyHostToDevice, st));
+    if (sph_geo) {
+        const int n = h.n_spheres;
+        upd_spheres<<<(n + kUpdThreads - 1) / kUpdThreads, kUpdThreads, 0, st>>>(
+            d.sph_exact, d.leaf_sph, n, const_cast<float4 *>(d.sph_filter), const_cast<float *>((const float *)d.sph_pairs),
+            const_cast<float4 *>(d.leaf_filter), s->upd_dev);
+        launch_refit(s->plan_sph, const_cast<BvhNode *>(d.nodes), SphereLeafBox{d.sph_exact, d.leaf_sph},
+                     &s->upd_dev->area_sph, st);
+    }
+    if (tri_geo) {
+        const int n = d.n_tri_tree;
+        upd_triangles<<<(n + kUpdThreads - 1) / kUpdThreads, kUpdThreads, 0, st>>>(d.tris, d.tri_leaf_id, n,
+                                                                                   const_cast<double *>(d.tri_leaf), s->upd_dev);
+        launch_refit(s->plan_tri, const_cast<BvhNode *>(d.tri_nodes), TriangleLeafBox{d.tri_leaf}, &s->upd_dev->area_tri, st);
+    }
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(s->upd_ev[1], st));
+    CU(cudaMemcpyAsync(&u, s->upd_dev, sizeof u, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, s->upd_ev[0], s->upd_ev[1]));
+    inf.device_ms = ms;
+
+    if (sph_geo) {
+        // the constants flatten() folds over the spheres, from the same per-sphere values (max and min do not
+        // depend on the order)
+        memcpy(&h.r_max, &u.r_max, 4); memcpy(&h.pad_c_max, &u.pad_c_max, 4);
+        memcpy(&h.eta_c_max, &u.eta_c_max, 4); memcpy(&h.abs_max, &u.abs_max, 4);
+        double lo[3], hi[3];
+        for (int a = 0; a < 3; a++) { lo[a] = dkey_value(u.lo[a]); hi[a] = dkey_value(u.hi[a]); }
+        set_sort_grid(h, lo, hi);
+        h.derived_stale = true;
+        inf.done |= ERT_DID_REFIT_SPHERES;
+        if (h.sph_build_area > 0) inf.sphere_area_ratio = u.area_sph / h.sph_build_area;
+    }
+    if (tri_geo) {
+        double e, m;
+        memcpy(&e, &u.tri_edge, 8);
+        memcpy(&m, &u.tri_abs, 8);
+        if (!(m <= kTriAlwaysAbs)) {
+            // the builder's admission rule: a box of float cannot hold this triangle
+            if ((rc = rebuild_tri_bvh(s)) != ERT_OK) return rc;
+            inf.done |= ERT_DID_REBUILD_TRI_BVH;
+        } else {
+            h.tbvh.edge_max = e * (1.0 + 1.0 / 1099511627776.0);   // as build_triangle_bvh rounds it up
+            h.tbvh.abs_max = m;
+            h.derived_stale = true;
+            inf.done |= ERT_DID_REFIT_TRIANGLES;
+            if (h.tri_build_area > 0) inf.triangle_area_ratio = u.area_tri / h.tri_build_area;
+        }
+    }
+    set_constants(s);
+
+    // grids: the cell grid and the direction grids hold copies of filter spheres, a direction grid its light
+    const bool cell_stale = sph_geo && h.cgrid.enabled;
+    bool lg_any = false;
+    for (char c : lg_stale) lg_any = lg_any || c;
+    if (flags & ERT_UPDATE_REBUILD_GRIDS) {
+        const bool cell = cell_stale || h.cgrid_dropped;
+        const uint64_t before = s->uploaded;
+        if ((cell || lg_any || h.lgrids_dropped) && (rc = rebuild_grids(s, cell, lg_stale, inf)) != ERT_OK) return rc;
+        inf.h2d_bytes += s->uploaded - before;
+    } else {
+        if (cell_stale) {
+            h.cgrid.enabled = false;
+            d.cg.enabled = 0;
+            h.cgrid_dropped = true;
+            inf.done |= ERT_DID_DROP_CELL_GRID;
+        }
+        if (lg_any) {
+            size_t keep = 0;
+            while (keep < lg_stale.size() && !lg_stale[keep]) keep++;
+            h.lgrids.resize(keep);
+            d.lg_count = (int)keep;
+            h.lgrids_dropped = true;
+            inf.done |= ERT_DID_DROP_LIGHT_GRIDS;
+        }
+    }
+    s->broken = false;
+    return ERT_OK;
+}
+
+// ERT_UPDATE_REBUILD: the create path into the scene's handle
+int update_rebuild(ert_scene *s, const ert_scene_desc *desc, ert_update_info &inf)
+{
+    HostScene h;
+    int rc = flatten(desc, h);
+    if (rc != ERT_OK) return rc;
+    s->broken = true;
+    CU(cudaEventRecord(s->upd_ev[0], 0));
+    for (void *p : s->allocs) cudaFree(p);
+    s->allocs.clear();
+    drop_plan(s->plan_sph);
+    drop_plan(s->plan_tri);
+    s->host = std::move(h);
+    s->host.sph_build_area = tree_area(s->host.bvh.nodes);
+    if (s->host.has_tri_bvh) s->host.tri_build_area = tree_area(s->host.tbvh.bvh.nodes);
+    const uint64_t before = s->uploaded;
+    if ((rc = upload_tables(s)) != ERT_OK) return rc;
+    CU(cudaEventRecord(s->upd_ev[1], 0));
+    CU(cudaEventSynchronize(s->upd_ev[1]));
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, s->upd_ev[0], s->upd_ev[1]));
+    inf.device_ms = ms;
+    inf.h2d_bytes = s->uploaded - before;
+    inf.done |= ERT_DID_REBUILD;
+    s->broken = false;
+    return ERT_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1061,11 +1586,21 @@ int ert_scene_clone(const ert_scene *src, int device, ert_scene **out)
     ert_scene *s = new (std::nothrow) ert_scene();
     if (!s) return fail(ERT_ERR_NOMEM, "out of host memory");
     s->device = device;
-    try {
-        s->host = src->host;
-    } catch (const std::exception &) {
-        delete s;
-        return fail(ERT_ERR_NOMEM, "out of host memory");
+    {
+        // an updated source's filters and trees are current on its device only
+        std::lock_guard<std::mutex> lock(const_cast<ert_scene *>(src)->mu);
+        if (src->broken) {
+            delete s;
+            return fail(ERT_ERR_CUDA, "the source scene's last update failed");
+        }
+        try {
+            s->host = src->host;
+            rc = s->host.derived_stale ? download_derived(src, s->host) : ERT_OK;
+        } catch (const std::exception &) {
+            delete s;
+            return fail(ERT_ERR_NOMEM, "out of host memory");
+        }
+        if (rc != ERT_OK) { delete s; return rc; }
     }
     try {
         rc = upload_scene(s);
@@ -1090,6 +1625,43 @@ int ert_scene_destroy(ert_scene *scene)
     return ERT_OK;
 }
 
+int ert_scene_update(ert_scene *scene, const ert_scene_desc *desc, uint32_t flags, ert_update_info *info)
+{
+    const auto t0 = std::chrono::steady_clock::now();
+    if (!scene) return fail(ERT_ERR_BADARG, "scene is NULL");
+    if (flags & ~(ERT_UPDATE_REBUILD_GRIDS | ERT_UPDATE_REBUILD)) return fail(ERT_ERR_BADARG, "unknown update flags");
+    std::lock_guard<std::mutex> lock(scene->mu);
+    CU(cudaSetDevice(scene->device));
+    ert_update_info inf{};
+    inf.sphere_area_ratio = inf.triangle_area_ratio = 1.0;
+    UpdateTables t{};
+    int rc;
+    try {
+        rc = update_stage(scene, desc, t);
+    } catch (const std::exception &) {
+        return fail(ERT_ERR_NOMEM, "out of host memory while checking the update");
+    }
+    if (rc != ERT_OK) return rc;
+    // frames already queued render the scene they were queued with
+    for (Slot &sl : scene->slots)
+        if ((rc = finish_slot(scene, sl)) != ERT_OK) return rc;
+    update_changes(scene->host, t, desc->camera, inf);
+    if (!scene->upd_ev[0]) CU(cudaEventCreate(&scene->upd_ev[0]));
+    if (!scene->upd_ev[1]) CU(cudaEventCreate(&scene->upd_ev[1]));
+    try {
+        rc = (flags & ERT_UPDATE_REBUILD) ? update_rebuild(scene, desc, inf) : update_apply(scene, t, desc->camera, flags, inf);
+    } catch (const std::exception &e) {
+        scene->broken = true;
+        rc = fail(ERT_ERR_NOMEM, std::string("scene update failed: ") + e.what());
+    }
+    if (rc != ERT_OK) return rc;
+    inf.has_cell_grid = scene->host.cgrid.enabled ? 1 : 0;
+    inf.light_grids = (int32_t)scene->host.lgrids.size();
+    inf.host_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (info) *info = inf;
+    return ERT_OK;
+}
+
 int ert_render_async(ert_scene *scene, const ert_render_params *params, int slot, void *host_frame,
                      size_t host_frame_bytes)
 {
@@ -1098,6 +1670,7 @@ int ert_render_async(ert_scene *scene, const ert_render_params *params, int slot
     if ((rc = check_params(params)) != ERT_OK) return rc;
     if (slot < 0 || slot >= ERT_MAX_SLOTS) return fail(ERT_ERR_BADARG, "slot out of range");
     std::lock_guard<std::mutex> lock(scene->mu);
+    if (scene->broken) return fail(ERT_ERR_CUDA, "the scene's last update failed: update it again or destroy it");
     CU(cudaSetDevice(scene->device));
     Slot &sl = scene->slots[slot];
     if ((rc = finish_slot(scene, sl)) != ERT_OK) return rc;
@@ -1242,6 +1815,7 @@ int ert_trace_rays(ert_scene *scene, int64_t n_rays, const double *rays6, int ac
     if (accel < ERT_ACCEL_AUTO || accel > ERT_ACCEL_WARP) return fail(ERT_ERR_BADARG, "unknown accel");
     if (n_rays == 0) return ERT_OK;
     std::lock_guard<std::mutex> lock(scene->mu);
+    if (scene->broken) return fail(ERT_ERR_CUDA, "the scene's last update failed: update it again or destroy it");
     CU(cudaSetDevice(scene->device));
     accel = pick_accel(scene, accel);
     double *d_rays = nullptr, *d_t = nullptr;

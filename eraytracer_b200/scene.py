@@ -6,6 +6,7 @@ Records are the tagged tuples of raytracer.erl:72-81 as `scene_test` pins them
 A scene is a list with the camera first (raytracer.erl:617-619).  Every numeric
 field may be an int or a float (Erlang scene literals mix both, erl:619-664).
 """
+import functools
 import math
 
 import numpy as np
@@ -82,6 +83,11 @@ class FlatScene:
     def upload(self, device=0):
         return _lib.Scene.create(self.camera, self.lights, self.spheres, self.triangles,
                                  self.planes, device=device)
+
+    def update(self, dev, rebuild_grids=False, rebuild=False):
+        """Puts these tables into the device scene `dev` (an upload of a scene with the same list shape)."""
+        return dev.update(self.camera, self.lights, self.spheres, self.triangles, self.planes,
+                          rebuild_grids=rebuild_grids, rebuild=rebuild)
 
     @property
     def n_elements(self):
@@ -254,6 +260,7 @@ def mesh_triangles(vertices, faces, material, first_order):
     return t
 
 
+@functools.lru_cache(maxsize=None)
 def _icosphere(level):
     """Unit icosphere: (vertices, faces), faces wound so that (v2 - v1) x (v3 - v1) points outwards."""
     p = (1.0 + math.sqrt(5.0)) / 2.0
@@ -298,12 +305,14 @@ MESH_CONFIGS = {
 }
 
 
-def mesh_scene(name="m3", n_triangles=None):
+def mesh_scene(name="m3", n_triangles=None, frame=0):
     """Triangle-mesh workload: the camera, lights and plane of synthetic_scene, the spheres of the C3 recipe,
     a heightfield sheet over the floor and closed icosphere meshes among the spheres (their back faces put
     entry faces behind reflection and shadow rays).  Both meshes face the camera and the outside.  Every value
     is float32-rounded and drawn from splitmix64_uniform.  List order: lights, spheres, triangles, plane.
-    n_triangles keeps the first that many triangles (scenes either side of the triangle-BVH threshold)."""
+    n_triangles keeps the first that many triangles (scenes either side of the triangle-BVH threshold).  frame k
+    (animated_scene) moves the spheres, shifts the sheet's waves by the phase 2 pi k / 64 and moves every icosphere
+    rigidly; frame 0 is the still scene."""
     n_sph, cells, n_ico, level, seed = MESH_CONFIGS[name]
     base = synthetic_scene("c3", n_spheres=n_sph)
     u = splitmix64_uniform(seed, 4 + 8 * n_ico)
@@ -311,7 +320,8 @@ def mesh_scene(name="m3", n_triangles=None):
     xs = np.linspace(-40.0, 40.0, cells + 1)
     zs = np.linspace(5.0, 85.0, cells + 1)
     X, Z = np.meshgrid(xs, zs, indexing='ij')
-    Y = 4.5 - 0.4 * (np.sin(X * (0.3 + u[0] * 0.2)) * np.cos(Z * (0.3 + u[1] * 0.2)) + 1.0)
+    phase, swing = _frame_motion(frame)
+    Y = 4.5 - 0.4 * (np.sin(X * (0.3 + u[0] * 0.2) + phase) * np.cos(Z * (0.3 + u[1] * 0.2)) + 1.0)
     sheet_v = _f32(np.stack([X, Y, Z], axis=-1).reshape(-1, 3))
     idx = np.arange((cells + 1) * (cells + 1)).reshape(cells + 1, cells + 1)
     p00, p10, p01, p11 = idx[:-1, :-1].ravel(), idx[1:, :-1].ravel(), idx[:-1, 1:].ravel(), idx[1:, 1:].ravel()
@@ -320,16 +330,61 @@ def mesh_scene(name="m3", n_triangles=None):
     tabs = [mesh_triangles(sheet_v, sheet_f, ((_f1(0.6), _f1(0.55), _f1(0.5)), 4.0, _f1(0.2), _f1(0.1)), first)]
     first += len(sheet_f)
     ico_v, ico_f = _icosphere(level)
+    ico_dir = _directions(seed ^ ANIM_SEED, n_ico)
     for k in range(n_ico):
         r = u[4 + 8 * k: 12 + 8 * k]
-        c = (-35.0 + 70.0 * r[0], -25.0 + 26.0 * r[1], 10.0 + 70.0 * r[2])
+        c = np.array((-35.0 + 70.0 * r[0], -25.0 + 26.0 * r[1], 10.0 + 70.0 * r[2])) + swing * ANIM_AMPLITUDE * ico_dir[k]
         rad = 2.0 + 3.0 * r[3]
         mat = ((_f1(r[4]), _f1(r[5]), _f1(r[6])), 20.0, _f1(0.5), _f1(0.2 + 0.5 * r[7]))
-        tabs.append(mesh_triangles(_f32(ico_v * rad + np.array(c)), ico_f, mat, first))
+        tabs.append(mesh_triangles(_f32(ico_v * rad + c), ico_f, mat, first))
         first += len(ico_f)
     tris = np.concatenate(tabs)
     if n_triangles is not None:
         tris = tris[:int(n_triangles)].copy()
     planes = base.planes.copy()
     planes['order'] = 3 + n_sph + len(tris)
-    return FlatScene(base.camera, base.lights, base.spheres, tris, planes)
+    return FlatScene(base.camera, base.lights, _moved_spheres(base.spheres, seed0_of("c3"), frame), tris, planes)
+
+
+# ---------------------------------------------------------------------------
+# Animation: frame k of a scene whose values move and whose list shape stays (ert_scene_update).
+# ---------------------------------------------------------------------------
+ANIM_SEED = 0xA11E0000A11E0000      # xor-ed into a scene's seed for the motion directions
+ANIM_AMPLITUDE = 1.0                # scene units
+ANIM_PERIOD = 64                    # frames
+
+
+def seed0_of(name):
+    return SYNTH_CONFIGS[name][5]
+
+
+def _frame_motion(k):
+    """(sheet phase, sphere / icosphere displacement factor) of frame k: both periodic in ANIM_PERIOD frames."""
+    a = 2.0 * math.pi * k / ANIM_PERIOD
+    return a, math.sin(a)
+
+
+def _directions(seed, n):
+    """n unit vectors from splitmix64_uniform (uniform in the cube, normalised)."""
+    d = splitmix64_uniform(seed, 3 * n).reshape(n, 3) * 2.0 - 1.0
+    return d / np.maximum(np.linalg.norm(d, axis=1), 1e-12)[:, None]
+
+
+def _moved_spheres(spheres, seed, k):
+    """Every sphere displaced by ANIM_AMPLITUDE sin(2 pi k / 64) along its own direction, float32-rounded."""
+    out = spheres.copy()
+    _, swing = _frame_motion(k)
+    if swing:
+        d = _directions(seed ^ ANIM_SEED, len(spheres))
+        out['center'] = _f32(spheres['center'] + swing * ANIM_AMPLITUDE * d)
+    return out
+
+
+def animated_scene(name, k):
+    """Frame k of the animation of c3 / c4 (synthetic_scene) or m3 / m4 (mesh_scene): the same list as frame 0 (the
+    still scene) with moved spheres, a travelling wave on the heightfield sheet and rigidly moved icospheres."""
+    if name in MESH_CONFIGS:
+        return mesh_scene(name, frame=k)
+    base = synthetic_scene(name)
+    return FlatScene(base.camera, base.lights, _moved_spheres(base.spheres, seed0_of(name), k), base.triangles,
+                     base.planes)

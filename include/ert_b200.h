@@ -204,6 +204,57 @@ ERT_API int ert_scene_clone(const ert_scene *src, int device, ert_scene **out);
 
 ERT_API int ert_scene_destroy(ert_scene *scene);
 
+/* ---- in-place update ------------------------------------------------------ */
+#define ERT_UPDATE_REBUILD_GRIDS 1u  /* rebuild stale cell / direction grids with the host builders */
+#define ERT_UPDATE_REBUILD       2u  /* full rebuild of every structure in place (the create path), handle kept */
+
+/* ert_update_info.changed: the tables that differ from the scene's (element for element, by `order`) */
+#define ERT_CHANGED_CAMERA         1u
+#define ERT_CHANGED_LIGHTS         2u   /* any light field */
+#define ERT_CHANGED_LIGHT_POS      4u   /* a light location */
+#define ERT_CHANGED_SPHERES        8u   /* sphere centres or radii */
+#define ERT_CHANGED_SPHERE_MAT    16u
+#define ERT_CHANGED_TRIANGLES     32u   /* triangle vertices */
+#define ERT_CHANGED_TRIANGLE_MAT  64u
+#define ERT_CHANGED_PLANES       128u   /* plane normals, distances or materials */
+
+/* ert_update_info.done */
+#define ERT_DID_REFIT_SPHERES        1u  /* sphere BVH refitted on the device (filters and constants recomputed) */
+#define ERT_DID_REFIT_TRIANGLES      2u  /* triangle BVH refitted on the device */
+#define ERT_DID_DROP_CELL_GRID       4u  /* the cell grid went stale and was dropped */
+#define ERT_DID_DROP_LIGHT_GRIDS     8u  /* direction grids went stale and were dropped */
+#define ERT_DID_REBUILD_CELL_GRID   16u  /* ERT_UPDATE_REBUILD_GRIDS: the cell grid was built again on the host */
+#define ERT_DID_REBUILD_LIGHT_GRIDS 32u  /* ERT_UPDATE_REBUILD_GRIDS: direction grids were built again on the host */
+#define ERT_DID_REBUILD_TRI_BVH     64u  /* a tree triangle broke the builder's admission rule: triangle BVH rebuilt on the host */
+#define ERT_DID_REBUILD            128u  /* ERT_UPDATE_REBUILD: every structure built again on the host */
+
+typedef struct ert_update_info {
+    uint32_t changed;               /* ERT_CHANGED_* */
+    uint32_t done;                  /* ERT_DID_* */
+    int32_t has_cell_grid;          /* after the update */
+    int32_t light_grids;            /* lights with a direction grid after the update */
+    int32_t light_grids_rebuilt;
+    int32_t reserved;
+    uint64_t h2d_bytes;             /* element tables uploaded (and grids / trees rebuilt on the host) */
+    double host_ms;                 /* wall time of the call */
+    double device_ms;               /* CUDA events around the uploads and the update kernels */
+    /* per tree: total child-box surface area now over the area at its last build (1 when unchanged or absent);
+     * a refitted tree degrades as this grows, ERT_UPDATE_REBUILD resets it */
+    double sphere_area_ratio;
+    double triangle_area_ratio;
+} ert_update_info;
+
+/* Replaces the scene's values with those of `desc`, keeping the handle.  `desc` must have the list shape of the
+ * scene's create: the same element counts per kind and the same set of `order` values per kind, in any table order.
+ * Any value may change.  A shape mismatch, a non-finite value or a duplicate `order` returns ERT_ERR_BADARG and
+ * leaves the scene untouched (everything is validated before any device write).  The call first finishes every
+ * slot, so a frame already queued renders the old scene.  Without ERT_UPDATE_REBUILD the BVHs are refitted on the
+ * device, and a cell or direction grid that the change made stale is dropped (ERT_ACCEL_GRID falls back to the BVH
+ * wavefront, shadow rays walk the BVH) unless ERT_UPDATE_REBUILD_GRIDS rebuilds it.  Every frame stays the linear
+ * scan's.  A CUDA failure during the update leaves the scene unusable (renders return ERT_ERR_CUDA) until a
+ * successful update.  `info` may be NULL. */
+ERT_API int ert_scene_update(ert_scene *scene, const ert_scene_desc *desc, uint32_t flags, ert_update_info *info);
+
 /* Renders the rows of params->part and copies them into `host_frame`, a buffer
  * for the FULL width*height frame (each part lands at its own rows, so parts
  * rendered on different GPUs assemble one frame without a gather step).
