@@ -233,8 +233,9 @@ class Scene:
 
     def update(self, camera, lights, spheres, triangles, planes, rebuild_grids=False, rebuild=False):
         """ert_scene_update: new values for the scene's elements (same counts, same `order` values per kind, tables in
-        any order).  Returns the ert_update_info as a dict; raises BadArg (scene untouched) on a shape mismatch, a
-        non-finite value or a duplicate `order`."""
+        any order).  rebuild_grids builds stale cell / direction grids again on the device (the grids of a fresh
+        create of the same tables); rebuild runs the whole create path in place.  Returns the ert_update_info as a
+        dict; raises BadArg (scene untouched) on a shape mismatch, a non-finite value or a duplicate `order`."""
         desc, tabs = self._desc(camera, lights, spheres, triangles, planes)
         flags = (UPDATE_REBUILD_GRIDS if rebuild_grids else 0) | (UPDATE_REBUILD if rebuild else 0)
         info = UpdateInfo()

@@ -6,43 +6,24 @@
 #include <cmath>
 #include <cstring>
 
+#include "grid_math.h"
+
 namespace ert {
-namespace {
-
-float f_down(double x)
-{
-    float f = (float)x;
-    if ((double)f > x) f = std::nextafterf(f, -INFINITY);
-    return f;
-}
-float f_up(double x)
-{
-    float f = (float)x;
-    if ((double)f < x) f = std::nextafterf(f, INFINITY);
-    return f;
-}
-
-}  // namespace
 
 void cell_grid_range(const CellGrid &g, int axis, double a, double b, int &i0, int &i1)
 {
-    const double lo = (double)g.lo[axis], cs = (double)g.cs;
-    double f0 = std::floor((a - (double)g.eps - lo) / cs), f1 = std::floor((b + (double)g.eps - lo) / cs);
-    const double top = (double)(g.res[axis] - 1);
-    i0 = (int)std::min(std::max(f0, 0.0), top);
-    i1 = (int)std::min(std::max(f1, 0.0), top);
+    cell_range(g.lo, g.cs, g.eps, g.res, axis, a, b, i0, i1);
 }
 
-void build_cell_grid(const double *centers, const double *radii, const float *filter, int64_t n, float abs_max,
-                     double density, CellGrid &out)
+void cell_grid_set_geometry(CellGrid &g, const CellGridGeom &geo)
 {
-    out = CellGrid();
-    if (n < kCellGridMinSpheres || !(density > 0) || !std::isfinite(abs_max) || abs_max > 1e6f) return;
-    const double u = 5.9604644775390625e-8;
-    // The walk follows the FP32 ray within m/2 of the true one (m: the per-ray margin of make_sray,
-    // >= 32u(|o|+abs_max)); boxes are inflated by eps and a ray may use the grid iff 4m <= eps.
-    const double eps = 1024.0 * u * std::max((double)abs_max, 1.0);
-    double lo[3] = {DBL_MAX, DBL_MAX, DBL_MAX}, hi[3] = {-DBL_MAX, -DBL_MAX, -DBL_MAX};
+    for (int a = 0; a < 3; a++) { g.res[a] = geo.res[a]; g.lo[a] = geo.lo[a]; g.hi[a] = geo.hi[a]; }
+    g.cs = geo.cs; g.inv_cs = geo.inv_cs; g.eps = geo.eps;
+}
+
+void sphere_bounds(const double *centers, const double *radii, int64_t n, double lo[3], double hi[3])
+{
+    for (int a = 0; a < 3; a++) { lo[a] = DBL_MAX; hi[a] = -DBL_MAX; }
     for (int64_t k = 0; k < n; k++) {
         const double r = std::fabs(radii[k]);
         for (int a = 0; a < 3; a++) {
@@ -50,30 +31,21 @@ void build_cell_grid(const double *centers, const double *radii, const float *fi
             hi[a] = std::max(hi[a], centers[k * 3 + a] + r);
         }
     }
-    double ext[3], vol = 1.0;
-    for (int a = 0; a < 3; a++) {
-        out.lo[a] = f_down(lo[a] - 2.0 * eps);
-        out.hi[a] = f_up(hi[a] + 2.0 * eps);
-        ext[a] = (double)out.hi[a] - (double)out.lo[a];
-        if (!(ext[a] > 0) || !std::isfinite(ext[a])) return;
-        vol *= ext[a];
-    }
-    // cubic cells: edge from the wanted cell count, then never so small that an axis needs more
-    // than kCellGridMaxRes cells
-    double cs = std::cbrt(vol / (density * (double)n));
-    for (int a = 0; a < 3; a++) cs = std::max(cs, ext[a] / (double)(kCellGridMaxRes - 1));
-    if (!(cs > 64.0 * eps) || !std::isfinite(cs)) return;
-    out.cs = f_up(cs);
-    out.inv_cs = (float)(1.0 / (double)out.cs);
-    out.eps = (float)eps;
-    size_t n_cells = 1;
-    for (int a = 0; a < 3; a++) {
-        int r = (int)std::ceil(ext[a] / (double)out.cs) + 1;
-        out.res[a] = std::min(std::max(r, 1), kCellGridMaxRes);
-        if ((double)out.res[a] * (double)out.cs < ext[a]) return;
-        n_cells *= (size_t)out.res[a];
-    }
-    if (n_cells > ((size_t)1 << 23)) return;           // 256 bytes per cell on the device
+}
+
+void build_cell_grid(const double *centers, const double *radii, const float *filter, int64_t n, float abs_max,
+                     double density, CellGrid &out)
+{
+    out = CellGrid();
+    if (n < kCellGridMinSpheres || !(density > 0) || !std::isfinite(abs_max) || abs_max > 1e6f) return;
+    double lo[3], hi[3];
+    sphere_bounds(centers, radii, n, lo, hi);
+    CellGridGeom geo;
+    const bool ok = cell_grid_geometry(lo, hi, n, abs_max, density, kCellGridMinSpheres, kCellGridMaxRes, geo);
+    cell_grid_set_geometry(out, geo);
+    if (!ok) return;
+    const size_t n_cells = (size_t)geo.n_cells;
+    const double eps = geo.eps_d;
 
     // pass 1: counts
     std::vector<uint32_t> count(n_cells, 0);
@@ -84,19 +56,8 @@ void build_cell_grid(const double *centers, const double *radii, const float *fi
         for (int a = 0; a < 3; a++) cell_grid_range(out, a, centers[k * 3 + a] - r, centers[k * 3 + a] + r, i0[a], i1[a]);
     };
     const size_t sx = 1, sy = (size_t)out.res[0], sz = (size_t)out.res[0] * (size_t)out.res[1];
-    // A cell inside the box of a sphere may still be out of the ball's reach (the corners of the box):
-    // the ball inflated by eps must come within the cell, also inflated by eps for the float planes.
     auto reaches = [&](int64_t k, int x, int y, int z) {
-        const double r = std::fabs(radii[k]) + 2.0 * eps;
-        const int c[3] = {x, y, z};
-        double d2 = 0;
-        for (int a = 0; a < 3; a++) {
-            const double lo_a = (double)out.lo[a] + (double)c[a] * (double)out.cs, hi_a = lo_a + (double)out.cs;
-            const double p = centers[k * 3 + a];
-            const double d = p < lo_a ? lo_a - p : (p > hi_a ? p - hi_a : 0.0);
-            d2 += d * d;
-        }
-        return d2 <= r * r * (1.0 + 1e-9);
+        return cell_reaches(out.lo, out.cs, eps, &centers[k * 3], radii[k], x, y, z);
     };
     for (int64_t k = 0; k < n; k++) {
         int i0[3], i1[3];

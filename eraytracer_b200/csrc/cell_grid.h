@@ -66,4 +66,12 @@ void build_cell_grid(const double *centers, const double *radii, const float *fi
 // Cell range [i0, i1] of the interval [a, b] along one axis (shared with the tests).
 void cell_grid_range(const CellGrid &g, int axis, double a, double b, int &i0, int &i1);
 
+// The double bounds [min (c - |r|), max (c + |r|)] of the sphere boxes, the input of the grid's geometry
+// (cell_grid_geometry in grid_math.h).
+void sphere_bounds(const double *centers, const double *radii, int64_t n, double lo[3], double hi[3]);
+
+// Copies res, lo, hi, cs, inv_cs and eps of geo into g.
+struct CellGridGeom;
+void cell_grid_set_geometry(CellGrid &g, const CellGridGeom &geo);
+
 }  // namespace ert

@@ -24,6 +24,7 @@
 #include "ert_wavefront.cuh"
 #include "ert_scan.cuh"
 #include "ert_update.cuh"
+#include "grid_build.cuh"
 #include "scene_math.h"
 
 // ERT_ACCEL_LINEAR: scenes up to this many spheres stay in the single-launch tiled kernel (one resident
@@ -90,6 +91,9 @@ struct HostScene {
                                        // current ones (a clone downloads them)
     bool cgrid_dropped = false;        // an update dropped the cell grid / direction grids (ERT_UPDATE_REBUILD_GRIDS
     bool lgrids_dropped = false;       // builds them again)
+    bool cgrid_dev = false;            // the cell grid / direction grid g was built on the device: the host mirror keeps
+    bool lgrid_dev[kMaxLightGrids] = {};   // its geometry only (a clone builds it again on its own device)
+    double sph_lo[3] = {0, 0, 0}, sph_hi[3] = {0, 0, 0};   // min (c - |r|), max (c + |r|): the cell grid's bounds
     double sph_build_area = 0, tri_build_area = 0;   // total child-box half area at the trees' last build (0: not yet taken)
 };
 
@@ -139,7 +143,12 @@ struct ert_scene {
     HostScene host;
     DevScene dev{};
     std::vector<void *> allocs;
-    std::vector<void *> cg_allocs, lg_allocs;   // the grids' arrays (an update may build them again)
+    // the grids' arrays, whether uploaded from the host builders or built on the device (grid_build.cuh); each
+    // direction grid owns its own, so an update rebuilds only the stale ones
+    CellGridDevOut cg_buf;
+    std::vector<LightGridDevOut> lg_buf;
+    DevBuf lg_desc;                             // the LightGridDev array
+    GridScratch grid_tmp;
     uint64_t uploaded = 0;                      // bytes upload() has copied to the device
     Slot slots[ERT_MAX_SLOTS];
     std::mutex mu;
@@ -333,6 +342,7 @@ int flatten(const ert_scene_desc *d, HostScene &h)
                 hi[a] = std::max(hi[a], centers[(size_t)k * 3 + a] + std::fabs(radii[(size_t)k]));
             }
         set_sort_grid(h, lo, hi);
+        for (int a = 0; a < 3; a++) { h.sph_lo[a] = lo[a]; h.sph_hi[a] = hi[a]; }
     }
     {
         // cell grid for the path rays
@@ -391,82 +401,94 @@ int upload(ert_scene *s, const std::vector<T> &v, const T **out, std::vector<voi
     return ERT_OK;
 }
 
-void free_all(std::vector<void *> &allocs)
+// v into the device array b (grown if needed)
+template <typename T>
+int upload_buf(ert_scene *s, DevBuf &b, const std::vector<T> &v)
 {
-    for (void *p : allocs) cudaFree(p);
-    allocs.clear();
+    CU(b.reserve(v.size() * sizeof(T)));
+    if (!v.empty()) CU(cudaMemcpy(b.p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
+    s->uploaded += v.size() * sizeof(T);
+    return ERT_OK;
+}
+
+// The LightGridDev array of the first `count` direction grids (s->lg_buf) to the device, on stream st; adds its
+// bytes to *h2d.
+int write_light_desc(ert_scene *s, int count, cudaStream_t st, uint64_t *h2d)
+{
+    std::vector<LightGridDev> lg((size_t)count);
+    for (int g = 0; g < count; g++) {
+        const LightGridDevOut &o = s->lg_buf[(size_t)g];
+        lg[(size_t)g].cell_off = o.cell_off.as<const unsigned int>();
+        lg[(size_t)g].cand = o.cand.as<const LightGridCand>();
+        lg[(size_t)g].head = o.head.as<const LightGridCand>();
+        lg[(size_t)g].always = o.always.as<const int>();
+        lg[(size_t)g].n_always = o.n_always;
+        lg[(size_t)g].res = o.res;
+    }
+    const size_t bytes = lg.size() * sizeof(LightGridDev);
+    CU(s->lg_desc.reserve(bytes));
+    if (bytes) CU(cudaMemcpyAsync(s->lg_desc.p, lg.data(), bytes, cudaMemcpyHostToDevice, st));
+    CU(cudaStreamSynchronize(st));                  // lg is pageable and goes out of scope
+    s->uploaded += bytes;
+    if (h2d) *h2d += bytes;
+    s->dev.lgrids = s->lg_desc.as<const LightGridDev>();
+    s->dev.lg_count = count;
+    return ERT_OK;
 }
 
 // the direction grids of h.lgrids (replacing any the device had)
 int upload_light_grids(ert_scene *s)
 {
     HostScene &h = s->host;
-    DevScene &d = s->dev;
     int rc;
-    free_all(s->lg_allocs);
-    std::vector<void *> *own = &s->lg_allocs;
-    {
-        std::vector<LightGridDev> lg(h.lgrids.size());
-        for (size_t g = 0; g < h.lgrids.size(); g++) {
-            const LightGrid &G = h.lgrids[g];
-            std::vector<LightGridCand> cand(G.entries.size());
-            for (size_t e = 0; e < cand.size(); e++) {
-                LightGridCand &c = cand[e];
-                c.cx = G.fs[4 * e]; c.cy = G.fs[4 * e + 1]; c.cz = G.fs[4 * e + 2]; c.R = G.fs[4 * e + 3];
-                c.sphere = G.entries[e].sphere; c.dmin = G.entries[e].dmin; c.pad[0] = c.pad[1] = 0;
-            }
-            // per-cell heads: the nearest candidate inline, the rest by range
-            const size_t n_cells = G.cell_off.empty() ? 0 : G.cell_off.size() - 1;
-            std::vector<LightGridCand> head(n_cells);
-            for (size_t c = 0; c < n_cells; c++) {
-                const uint32_t e0 = G.cell_off[c], e1 = G.cell_off[c + 1];
-                LightGridCand &hd = head[c];
-                if (e0 < e1) {
-                    hd = cand[e0];
-                    hd.pad[0] = (int)(e0 + 1); hd.pad[1] = (int)e1;
-                } else {
-                    hd.cx = hd.cy = hd.cz = 0.f; hd.R = -3.0e38f; hd.sphere = -1; hd.dmin = INFINITY;
-                    hd.pad[0] = hd.pad[1] = 0;
-                }
-            }
-            const unsigned int *off; const LightGridCand *cd; const LightGridCand *hd; const int *al;
-            if ((rc = upload<unsigned int>(s, G.cell_off, &off, own)) != ERT_OK) return rc;
-            if ((rc = upload<LightGridCand>(s, cand, &cd, own)) != ERT_OK) return rc;
-            if ((rc = upload<LightGridCand>(s, head, &hd, own)) != ERT_OK) return rc;
-            if ((rc = upload<int>(s, G.always, &al, own)) != ERT_OK) return rc;
-            lg[g].cell_off = off; lg[g].cand = cd; lg[g].head = hd; lg[g].always = al;
-            lg[g].n_always = (int)G.always.size(); lg[g].res = G.res;
-        }
-        const LightGridDev *lgd;
-        if ((rc = upload<LightGridDev>(s, lg, &lgd, own)) != ERT_OK) return rc;
-        d.lgrids = lgd;
-        d.lg_count = (int)lg.size();
+    if (s->lg_buf.size() < h.lgrids.size()) s->lg_buf.resize(h.lgrids.size());
+    std::vector<LightGridCand> cand, head;
+    for (size_t g = 0; g < h.lgrids.size(); g++) {
+        const LightGrid &G = h.lgrids[g];
+        LightGridDevOut &o = s->lg_buf[g];
+        pack_light_grid(G, cand, head);
+        if ((rc = upload_buf(s, o.cell_off, G.cell_off)) != ERT_OK) return rc;
+        if ((rc = upload_buf(s, o.cand, cand)) != ERT_OK) return rc;
+        if ((rc = upload_buf(s, o.head, head)) != ERT_OK) return rc;
+        if ((rc = upload_buf(s, o.always, G.always)) != ERT_OK) return rc;
+        o.ok = true;
+        o.res = G.res;
+        o.n_always = (int)G.always.size();
+        o.n_entries = G.entries.size();
     }
-    return ERT_OK;
+    return write_light_desc(s, (int)h.lgrids.size(), 0, nullptr);
+}
+
+// the kernels' view of s->cg_buf
+void set_cell_desc(ert_scene *s)
+{
+    DevScene &d = s->dev;
+    const CellGridDevOut &G = s->cg_buf;
+    d.cg.blocks = G.blocks.as<const uint4>(); d.cg.over_filter = G.over_filter.as<const float4>();
+    d.cg.over_sph = G.over_sph.as<const int>(); d.cg.big = G.big.as<const int>();
+    d.cg.n_big = G.n_big; d.cg.enabled = G.enabled ? 1 : 0;
+    d.cg.rx = G.geo.res[0]; d.cg.ry = G.geo.res[1]; d.cg.rz = G.geo.res[2];
+    for (int a = 0; a < 3; a++) { d.cg.lo[a] = G.geo.lo[a]; d.cg.hi[a] = G.geo.hi[a]; }
+    d.cg.cs = G.geo.cs; d.cg.eps = G.geo.eps;
 }
 
 // the cell grid of h.cgrid (replacing any the device had)
 int upload_cell_grid(ert_scene *s)
 {
-    HostScene &h = s->host;
-    DevScene &d = s->dev;
+    const CellGrid &G = s->host.cgrid;
+    CellGridDevOut &o = s->cg_buf;
     int rc;
-    free_all(s->cg_allocs);
-    std::vector<void *> *own = &s->cg_allocs;
-    {
-        const CellGrid &G = h.cgrid;
-        const CellBlock *blocks; const float *rf; const int *rs; const int *big;
-        if ((rc = upload<CellBlock>(s, G.blocks, &blocks, own)) != ERT_OK) return rc;
-        if ((rc = upload<float>(s, G.over_filter, &rf, own)) != ERT_OK) return rc;
-        if ((rc = upload<int>(s, G.over_sph, &rs, own)) != ERT_OK) return rc;
-        if ((rc = upload<int>(s, G.big, &big, own)) != ERT_OK) return rc;
-        d.cg.blocks = reinterpret_cast<const uint4 *>(blocks); d.cg.over_filter = reinterpret_cast<const float4 *>(rf);
-        d.cg.over_sph = rs; d.cg.big = big;
-        d.cg.n_big = (int)G.big.size(); d.cg.enabled = G.enabled ? 1 : 0;
-        d.cg.rx = G.res[0]; d.cg.ry = G.res[1]; d.cg.rz = G.res[2];
-        for (int a = 0; a < 3; a++) { d.cg.lo[a] = G.lo[a]; d.cg.hi[a] = G.hi[a]; }
-        d.cg.cs = G.cs; d.cg.eps = G.eps;
-    }
+    if ((rc = upload_buf(s, o.blocks, G.blocks)) != ERT_OK) return rc;
+    if ((rc = upload_buf(s, o.over_filter, G.over_filter)) != ERT_OK) return rc;
+    if ((rc = upload_buf(s, o.over_sph, G.over_sph)) != ERT_OK) return rc;
+    if ((rc = upload_buf(s, o.big, G.big)) != ERT_OK) return rc;
+    o.enabled = G.enabled;
+    o.n_big = (int)G.big.size();
+    o.n_over = G.over_sph.size();
+    o.geo = CellGridGeom();
+    for (int a = 0; a < 3; a++) { o.geo.res[a] = G.res[a]; o.geo.lo[a] = G.lo[a]; o.geo.hi[a] = G.hi[a]; }
+    o.geo.cs = G.cs; o.geo.inv_cs = G.inv_cs; o.geo.eps = G.eps;
+    set_cell_desc(s);
     return ERT_OK;
 }
 
@@ -641,8 +663,10 @@ void destroy(ert_scene *s)
         if (sl.stream) cudaStreamDestroy(sl.stream);
     }
     for (void *p : s->allocs) cudaFree(p);
-    free_all(s->cg_allocs);
-    free_all(s->lg_allocs);
+    s->cg_buf.release();
+    for (LightGridDevOut &o : s->lg_buf) o.release();
+    s->lg_desc.release();
+    s->grid_tmp.release();
     if (s->plan_sph.order) cudaFree(s->plan_sph.order);
     if (s->plan_tri.order) cudaFree(s->plan_tri.order);
     if (s->upd_dev) cudaFree(s->upd_dev);
@@ -1298,59 +1322,81 @@ int rebuild_tri_bvh(ert_scene *s)
     return ERT_OK;
 }
 
+// Builds on the device (grid_build.cuh), from the device's current spheres and filter spheres, the cell grid (cell)
+// and the direction grids of the lights flagged in `need`; a light whose grid goes over its entry budget ends the
+// run of grids.  Adds the H2D bytes (the LightGridDev array) to *h2d.
+int build_grids_on_device(ert_scene *s, bool cell, const std::vector<char> &need, cudaStream_t st, uint64_t *h2d)
+{
+    HostScene &h = s->host;
+    const DevScene &d = s->dev;
+    if (cell) {
+        double density;
+        if (cell_grid_wanted(density))
+            CU(build_cell_grid_device(d.sph_exact, d.sph_filter, h.n_spheres, h.sph_lo, h.sph_hi, h.abs_max, density,
+                                      s->grid_tmp, s->cg_buf, st));
+        else
+            s->cg_buf.enabled = false;
+        h.cgrid = CellGrid();
+        h.cgrid.enabled = s->cg_buf.enabled;
+        if (h.cgrid.enabled) cell_grid_set_geometry(h.cgrid, s->cg_buf.geo);
+        h.cgrid_dev = h.cgrid.enabled;
+        set_cell_desc(s);
+    }
+    if (!need.empty()) {
+        const int res = light_grid_res();
+        if (s->lg_buf.size() < need.size()) s->lg_buf.resize(need.size());
+        size_t keep = 0;
+        for (; keep < need.size(); keep++) {
+            if (!need[keep]) continue;
+            LightGridDevOut &o = s->lg_buf[keep];
+            CU(build_light_grid_device(d.sph_exact, d.sph_filter, h.n_spheres, &h.lights[keep * 9 + 3], res,
+                                       kLightGridMaxEntries, s->grid_tmp, o, st));
+            if (!o.ok) break;
+        }
+        h.lgrids.resize(keep);
+        for (size_t g = 0; g < keep; g++)
+            if (need[g]) {
+                h.lgrids[g] = LightGrid();
+                h.lgrids[g].res = res;
+                h.lgrid_dev[g] = true;
+            }
+        int rc;
+        if ((rc = write_light_desc(s, (int)keep, st, h2d)) != ERT_OK) return rc;
+    }
+    CU(cudaStreamSynchronize(st));
+    return ERT_OK;
+}
+
 // ERT_UPDATE_REBUILD_GRIDS: the cell grid (cell) and the direction grids of `stale` lights, and any an earlier
-// update dropped, built again by the host builders from the current spheres.
-int rebuild_grids(ert_scene *s, bool cell, const std::vector<char> &stale, ert_update_info &inf)
+// update dropped, built again on the device.
+int rebuild_grids(ert_scene *s, bool cell, const std::vector<char> &stale, cudaStream_t st, ert_update_info &inf)
 {
     HostScene &h = s->host;
     int rc;
-    if (h.derived_stale && (rc = download_derived(s, h)) != ERT_OK) return rc;
-    const size_t n = (size_t)h.n_spheres;
-    std::vector<double> centers(n * 3), radii(n);
-    for (size_t k = 0; k < n; k++) {
-        for (int a = 0; a < 3; a++) centers[k * 3 + a] = h.sph_exact[k * 4 + a];
-        radii[k] = h.sph_exact[k * 4 + 3];
-    }
-    const int res = light_grid_res();
-    const int n_target = light_grid_target(h, res);
+    const int n_target = light_grid_target(h, light_grid_res());
     const size_t have = h.lgrids.size();
-    std::vector<LightGrid> lg((size_t)n_target);
-    std::vector<char> built((size_t)n_target, 0);
+    std::vector<char> need((size_t)n_target, 0);
     int n_need = 0;
-    WorkerGroup builders;
-    for (int g = 0; g < n_target; g++) {
-        if ((size_t)g < have && !((size_t)g < stale.size() && stale[(size_t)g])) {
-            lg[(size_t)g] = std::move(h.lgrids[(size_t)g]);
-            built[(size_t)g] = 1;
-            continue;
+    for (int g = 0; g < n_target; g++)
+        if ((size_t)g >= have || ((size_t)g < stale.size() && stale[(size_t)g])) {
+            need[(size_t)g] = 1;
+            n_need++;
         }
-        n_need++;
-        builders.spawn([&h, &centers, &radii, &lg, &built, g, res] {
-            built[(size_t)g] = build_light_grid(centers.data(), radii.data(), h.sph_filter.data(), h.n_spheres,
-                                                &h.lights[(size_t)g * 9 + 3], res, lg[(size_t)g]) ? 1 : 0;
-        });
-    }
-    CellGrid cg;
-    double density;
-    const bool want_cell = cell && cell_grid_wanted(density);
-    if (want_cell)
-        builders.spawn([&h, &centers, &radii, &cg, density] {
-            build_cell_grid(centers.data(), radii.data(), h.sph_filter.data(), h.n_spheres, h.abs_max, density, cg);
-        });
-    builders.join();
+    const bool lights = n_need > 0 || have < (size_t)n_target;
+    if (!lights) need.clear();
+    CU(cudaEventRecord(s->upd_ev[0], st));
+    if ((rc = build_grids_on_device(s, cell, need, st, &inf.h2d_bytes)) != ERT_OK) return rc;
+    CU(cudaEventRecord(s->upd_ev[1], st));
+    CU(cudaEventSynchronize(s->upd_ev[1]));
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, s->upd_ev[0], s->upd_ev[1]));
+    inf.device_ms += ms;
     if (cell) {
-        h.cgrid = std::move(cg);
         h.cgrid_dropped = false;
-        if ((rc = upload_cell_grid(s)) != ERT_OK) return rc;
         inf.done |= ERT_DID_REBUILD_CELL_GRID;
     }
-    if (n_need > 0 || have < (size_t)n_target) {
-        size_t keep = 0;
-        while (keep < built.size() && built[keep]) keep++;
-        lg.resize(keep);
-        h.lgrids = std::move(lg);
+    if (lights) {
         h.lgrids_dropped = false;
-        if ((rc = upload_light_grids(s)) != ERT_OK) return rc;
         inf.done |= ERT_DID_REBUILD_LIGHT_GRIDS;
         inf.light_grids_rebuilt = n_need;
     }
@@ -1434,6 +1480,7 @@ int update_apply(ert_scene *s, UpdateTables &t, const ert_camera &camera, uint32
         double lo[3], hi[3];
         for (int a = 0; a < 3; a++) { lo[a] = dkey_value(u.lo[a]); hi[a] = dkey_value(u.hi[a]); }
         set_sort_grid(h, lo, hi);
+        for (int a = 0; a < 3; a++) { h.sph_lo[a] = lo[a]; h.sph_hi[a] = hi[a]; }
         h.derived_stale = true;
         inf.done |= ERT_DID_REFIT_SPHERES;
         if (h.sph_build_area > 0) inf.sphere_area_ratio = u.area_sph / h.sph_build_area;
@@ -1461,10 +1508,9 @@ int update_apply(ert_scene *s, UpdateTables &t, const ert_camera &camera, uint32
     bool lg_any = false;
     for (char c : lg_stale) lg_any = lg_any || c;
     if (flags & ERT_UPDATE_REBUILD_GRIDS) {
-        const bool cell = cell_stale || h.cgrid_dropped;
-        const uint64_t before = s->uploaded;
-        if ((cell || lg_any || h.lgrids_dropped) && (rc = rebuild_grids(s, cell, lg_stale, inf)) != ERT_OK) return rc;
-        inf.h2d_bytes += s->uploaded - before;
+        // a grid the spheres refused (a knot of more than kCellGridMaxCount) is tried again when they move
+        const bool cell = cell_stale || h.cgrid_dropped || (sph_geo && h.n_spheres >= kCellGridMinSpheres);
+        if ((cell || lg_any || h.lgrids_dropped) && (rc = rebuild_grids(s, cell, lg_stale, st, inf)) != ERT_OK) return rc;
     } else {
         if (cell_stale) {
             h.cgrid.enabled = false;
@@ -1604,6 +1650,16 @@ int ert_scene_clone(const ert_scene *src, int device, ert_scene **out)
     }
     try {
         rc = upload_scene(s);
+        // grids built on the source's device: the same builders on this one, from the same tables
+        HostScene &h = s->host;
+        std::vector<char> need(h.lgrids.size(), 0);
+        bool any = h.cgrid_dev;
+        for (size_t g = 0; g < need.size(); g++) any |= (need[g] = h.lgrid_dev[g] ? 1 : 0) != 0;
+        if (rc == ERT_OK && any) {
+            const size_t n_grids = h.lgrids.size();
+            rc = build_grids_on_device(s, h.cgrid_dev, need, s->slots[0].stream, nullptr);
+            if (rc == ERT_OK && h.lgrids.size() != n_grids) rc = fail(ERT_ERR_CUDA, "a direction grid of the source failed to build again");
+        }
     } catch (const std::exception &e) {
         g_err = std::string("out of host memory while uploading the scene: ") + e.what();
         rc = ERT_ERR_NOMEM;

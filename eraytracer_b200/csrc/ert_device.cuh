@@ -16,6 +16,7 @@
 #include <stdint.h>
 
 #include "bvh_build.h"
+#include "light_grid.h"
 #include "tri_walk.h"
 
 namespace ert {
@@ -84,13 +85,6 @@ struct DevScene {
     double tri_edge_max, tri_abs_max;   // the tree's constants of tri_walk.h
 };
 
-// One entry of a light's direction grid: 32 bytes, one 256-bit load.
-struct alignas(32) LightGridCand {
-    float cx, cy, cz, R;         // filter sphere
-    int sphere;                  // sphere index
-    float dmin;                  // lower bound of the distance light -> sphere
-    int pad[2];
-};
 struct LightGridDev {
     const unsigned int *cell_off;    // [6*res*res + 1]
     const LightGridCand *head;       // [6*res*res] the first (nearest) candidate of every cell, its pad[] holding

@@ -6,43 +6,13 @@
 #include <cstring>
 #include <thread>
 
+#include "grid_math.h"
 #include "host_threads.h"
 
 namespace ert {
 namespace {
 
-constexpr double kQuarterPi = 0.78539816339744830962;
-// Shadow rays find their cell in FP32 (light_grid_cell_f32: direction rounded to float, one reciprocal, two
-// products — every step within 6e-8 relative, |u| <= 1, so the cell coordinate is off by < 5e-7, and a direction
-// that close to a face edge may land on the neighbouring face).  The slack below is four times that, on the
-// half-angle and on the projected bounds, so a sphere is listed in every cell the FP32 computation can name for a
-// direction that touches it.
-constexpr double kAngleSlack = 2e-6;      // radians added to every half-angle
-constexpr double kCoordSlack = 2e-6;      // added to the projected bounds
-
 struct Rect { int32_t sphere; uint8_t face; uint16_t u0, u1, v0, v1; };
-
-// 1-D bound: directions (x, z) with z > 0 and |x/z| <= 1 that can touch the disc (cx, cz, r).
-// Returns false when none can.  lo/hi are bounds of x/z inside [-1, 1].
-bool axis_bound(double cx, double cz, double r, double &lo, double &hi)
-{
-    double rho2 = cx * cx + cz * cz;
-    if (rho2 <= r * r) { lo = -1.0; hi = 1.0; return true; }       // the origin is inside the disc
-    double rho = std::sqrt(rho2);
-    double theta = std::atan2(cx, cz);                               // from +z towards +x
-    double alpha = std::asin(std::min(1.0, r / rho)) + kAngleSlack;
-    if (std::fabs(theta) - alpha > kQuarterPi) return false;
-    double a0 = std::max(theta - alpha, -kQuarterPi), a1 = std::min(theta + alpha, kQuarterPi);
-    lo = std::max(-1.0, std::tan(a0) - kCoordSlack);
-    hi = std::min(1.0, std::tan(a1) + kCoordSlack);
-    return lo <= hi;
-}
-
-inline int cell_index(double x, int res)
-{
-    int i = (int)std::floor((x + 1.0) * 0.5 * res);
-    return std::min(std::max(i, 0), res - 1);
-}
 
 }  // namespace
 
@@ -94,26 +64,16 @@ bool build_light_grid(const double *centers, const double *radii, const float *f
         auto &rv = rects[t];
         rv.reserve((size_t)(i1 - i0) * 3 / 2);
         for (int64_t i = i0; i < i1; i++) {
-            double c[3] = {centers[3 * i] - light[0], centers[3 * i + 1] - light[1], centers[3 * i + 2] - light[2]};
-            double r = std::fabs(radii[i]);
-            r = r * (1.0 + 1e-6) + 1e-9;
-            double d2 = c[0] * c[0] + c[1] * c[1] + c[2] * c[2];
-            if (!(d2 > r * r)) { always[t].push_back((int32_t)i); continue; }   // also catches NaN
-            for (int m = 0; m < 3; m++) {
-                int a = (m + 1) % 3, b = (m + 2) % 3;
-                for (int sgn = 0; sgn < 2; sgn++) {
-                    double cz = sgn ? -c[m] : c[m];
-                    if (cz + r <= 0.0) continue;                    // entirely behind this face
-                    double ulo, uhi, vlo, vhi;
-                    if (!axis_bound(c[a], cz, r, ulo, uhi)) continue;
-                    if (!axis_bound(c[b], cz, r, vlo, vhi)) continue;
-                    Rect q;
-                    q.sphere = (int32_t)i;
-                    q.face = (uint8_t)(2 * m + sgn);
-                    q.u0 = (uint16_t)cell_index(ulo, res); q.u1 = (uint16_t)cell_index(uhi, res);
-                    q.v0 = (uint16_t)cell_index(vlo, res); q.v1 = (uint16_t)cell_index(vhi, res);
-                    rv.push_back(q);
-                }
+            LightRect lr[6];
+            const int nr = light_rects(&centers[3 * i], radii[i], light, res, lr);
+            if (nr < 0) { always[t].push_back((int32_t)i); continue; }
+            for (int j = 0; j < nr; j++) {
+                Rect q;
+                q.sphere = (int32_t)i;
+                q.face = (uint8_t)lr[j].face;
+                q.u0 = (uint16_t)lr[j].u0; q.u1 = (uint16_t)lr[j].u1;
+                q.v0 = (uint16_t)lr[j].v0; q.v1 = (uint16_t)lr[j].v1;
+                rv.push_back(q);
             }
         }
     };
@@ -144,10 +104,7 @@ bool build_light_grid(const double *centers, const double *radii, const float *f
         for (const Rect &q : rv) {
             double c[3] = {centers[3 * (size_t)q.sphere] - light[0], centers[3 * (size_t)q.sphere + 1] - light[1],
                            centers[3 * (size_t)q.sphere + 2] - light[2]};
-            double dist = std::sqrt(c[0] * c[0] + c[1] * c[1] + c[2] * c[2]) - std::fabs(radii[q.sphere]);
-            // lower bound in float, with relative slack for the caller's FP32 comparisons
-            float dmin = (float)(dist * (1.0 - 1e-5) - 1e-6);
-            if ((double)dmin > dist) dmin = std::nextafterf(dmin, -INFINITY);
+            const float dmin = light_dmin(c, radii[q.sphere]);
             for (int v = q.v0; v <= q.v1; v++)
                 for (int u = q.u0; u <= q.u1; u++) {
                     size_t cell = ((size_t)q.face * res + v) * res + u;
@@ -168,6 +125,30 @@ bool build_light_grid(const double *centers, const double *radii, const float *f
     out.fs.resize((size_t)total * 4);
     for (size_t e = 0; e < (size_t)total; e++) memcpy(&out.fs[4 * e], filter + 4 * (size_t)out.entries[e].sphere, 16);
     return true;
+}
+
+void pack_light_grid(const LightGrid &G, std::vector<LightGridCand> &cand, std::vector<LightGridCand> &head)
+{
+    cand.resize(G.entries.size());
+    for (size_t e = 0; e < cand.size(); e++) {
+        LightGridCand &c = cand[e];
+        c.cx = G.fs[4 * e]; c.cy = G.fs[4 * e + 1]; c.cz = G.fs[4 * e + 2]; c.R = G.fs[4 * e + 3];
+        c.sphere = G.entries[e].sphere; c.dmin = G.entries[e].dmin; c.pad[0] = c.pad[1] = 0;
+    }
+    // per-cell heads: the nearest candidate inline, the rest by range
+    const size_t n_cells = G.cell_off.empty() ? 0 : G.cell_off.size() - 1;
+    head.resize(n_cells);
+    for (size_t c = 0; c < n_cells; c++) {
+        const uint32_t e0 = G.cell_off[c], e1 = G.cell_off[c + 1];
+        LightGridCand &hd = head[c];
+        if (e0 < e1) {
+            hd = cand[e0];
+            hd.pad[0] = (int)(e0 + 1); hd.pad[1] = (int)e1;
+        } else {
+            hd.cx = hd.cy = hd.cz = 0.f; hd.R = -3.0e38f; hd.sphere = -1; hd.dmin = INFINITY;
+            hd.pad[0] = hd.pad[1] = 0;
+        }
+    }
 }
 
 }  // namespace ert

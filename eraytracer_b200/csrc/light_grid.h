@@ -23,6 +23,14 @@ struct LightGridEntry {          // 8 bytes next to a 16-byte filter sphere
     float dmin;                  // lower bound of the distance from the light to the sphere
 };
 
+// One entry of a light's direction grid on the device: 32 bytes, one 256-bit load.
+struct alignas(32) LightGridCand {
+    float cx, cy, cz, R;         // filter sphere
+    int sphere;                  // sphere index
+    float dmin;                  // lower bound of the distance light -> sphere
+    int pad[2];
+};
+
 struct LightGrid {
     int res = 0;                             // cells per cube-face edge
     std::vector<uint32_t> cell_off;          // [6*res*res + 1] offsets into the entry arrays
@@ -35,6 +43,11 @@ struct LightGrid {
 // Returns false (and leaves `out` empty) when the grid would need more than kLightGridMaxEntries entries.
 bool build_light_grid(const double *centers, const double *radii, const float *filter, int64_t n,
                       const double light[3], int res, LightGrid &out);
+
+// The layout the shadow kernels walk (LightGridDev in ert_device.cuh): every entry with its filter sphere (cand), and
+// per cell its nearest candidate (head) with pad[] = the range [first + 1, end) of the others in cand; an empty cell's
+// head has R = -3e38, sphere -1, dmin = +inf.
+void pack_light_grid(const LightGrid &g, std::vector<LightGridCand> &cand, std::vector<LightGridCand> &head);
 
 // Face/cell of a direction, shared by the builder's tests and (re-stated) by the device code:
 // major axis m = first axis of largest |d|, face = 2*m + (d[m] < 0), u = d[(m+1)%3]/|d[m]|,

@@ -85,7 +85,9 @@ class FlatScene:
                                  self.planes, device=device)
 
     def update(self, dev, rebuild_grids=False, rebuild=False):
-        """Puts these tables into the device scene `dev` (an upload of a scene with the same list shape)."""
+        """Puts these tables into the device scene `dev` (an upload of a scene with the same list shape).  With
+        rebuild_grids, cell and direction grids the change made stale (or an earlier update dropped) are built again
+        on the device, byte-identical to what a fresh upload of these tables builds; without, they are dropped."""
         return dev.update(self.camera, self.lights, self.spheres, self.triangles, self.planes,
                           rebuild_grids=rebuild_grids, rebuild=rebuild)
 

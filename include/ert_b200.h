@@ -205,7 +205,7 @@ ERT_API int ert_scene_clone(const ert_scene *src, int device, ert_scene **out);
 ERT_API int ert_scene_destroy(ert_scene *scene);
 
 /* ---- in-place update ------------------------------------------------------ */
-#define ERT_UPDATE_REBUILD_GRIDS 1u  /* rebuild stale cell / direction grids with the host builders */
+#define ERT_UPDATE_REBUILD_GRIDS 1u  /* rebuild stale cell / direction grids on the device */
 #define ERT_UPDATE_REBUILD       2u  /* full rebuild of every structure in place (the create path), handle kept */
 
 /* ert_update_info.changed: the tables that differ from the scene's (element for element, by `order`) */
@@ -223,8 +223,8 @@ ERT_API int ert_scene_destroy(ert_scene *scene);
 #define ERT_DID_REFIT_TRIANGLES      2u  /* triangle BVH refitted on the device */
 #define ERT_DID_DROP_CELL_GRID       4u  /* the cell grid went stale and was dropped */
 #define ERT_DID_DROP_LIGHT_GRIDS     8u  /* direction grids went stale and were dropped */
-#define ERT_DID_REBUILD_CELL_GRID   16u  /* ERT_UPDATE_REBUILD_GRIDS: the cell grid was built again on the host */
-#define ERT_DID_REBUILD_LIGHT_GRIDS 32u  /* ERT_UPDATE_REBUILD_GRIDS: direction grids were built again on the host */
+#define ERT_DID_REBUILD_CELL_GRID   16u  /* ERT_UPDATE_REBUILD_GRIDS: the cell grid was built again on the device */
+#define ERT_DID_REBUILD_LIGHT_GRIDS 32u  /* ERT_UPDATE_REBUILD_GRIDS: direction grids were built again on the device */
 #define ERT_DID_REBUILD_TRI_BVH     64u  /* a tree triangle broke the builder's admission rule: triangle BVH rebuilt on the host */
 #define ERT_DID_REBUILD            128u  /* ERT_UPDATE_REBUILD: every structure built again on the host */
 
@@ -235,9 +235,9 @@ typedef struct ert_update_info {
     int32_t light_grids;            /* lights with a direction grid after the update */
     int32_t light_grids_rebuilt;
     int32_t reserved;
-    uint64_t h2d_bytes;             /* element tables uploaded (and grids / trees rebuilt on the host) */
+    uint64_t h2d_bytes;             /* element tables uploaded (and trees rebuilt on the host, the direction grids' descriptors) */
     double host_ms;                 /* wall time of the call */
-    double device_ms;               /* CUDA events around the uploads and the update kernels */
+    double device_ms;               /* CUDA events around the uploads, the update kernels and the grid builds */
     /* per tree: total child-box surface area now over the area at its last build (1 when unchanged or absent);
      * a refitted tree degrades as this grows, ERT_UPDATE_REBUILD resets it */
     double sphere_area_ratio;
