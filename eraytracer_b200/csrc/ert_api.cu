@@ -26,6 +26,7 @@
 #include "ert_update.cuh"
 #include "grid_build.cuh"
 #include "scene_math.h"
+#include "scene_tables.h"
 
 // ERT_ACCEL_LINEAR: scenes up to this many spheres stay in the single-launch tiled kernel (one resident
 // tile, no queue traffic); larger ones run the wavefront with the brute-force scan kernels.
@@ -65,16 +66,8 @@ int cuda_fail(cudaError_t e, const char *what)
 // Host copy of the flattened scene (kept so ert_scene_clone needs no rebuild).
 struct HostScene {
     ert_camera camera;
-    std::vector<double> lights;        // [n][9]
-    std::vector<int> light_order;      // their list positions (ascending)
-    std::vector<double> planes, plane_mat;
-    std::vector<int> plane_order;
-    std::vector<double> tris, tri_mat;
-    std::vector<int> tri_order;
-    std::vector<double> sph_exact;     // [n][4]
-    std::vector<double> sph_mat;       // [n][6]
-    std::vector<double> sph_refl;      // [n]
-    std::vector<int> sph_order;
+    std::vector<double> tab[T_COUNT];  // the element tables (scene_tables.h)
+    std::vector<int> order[K_COUNT];   // the list positions of each kind's elements (lights, spheres: ascending)
     std::vector<float> sph_filter;     // [n][4]
     std::vector<float> sph_pairs;      // pair-interleaved, padded to whole scan tiles (ert_scan.cuh)
     std::vector<float> leaf_filter;    // [n][4]
@@ -142,6 +135,7 @@ struct ert_scene {
     int wf_grid_fin = 0;               // wf_finalize: a streaming pass, every resident slot filled
     HostScene host;
     DevScene dev{};
+    const double *tab_dev[T_COUNT] = {};        // host.tab on the device, where the DevScene fields point
     std::vector<void *> allocs;
     // the grids' arrays, whether uploaded from the host builders or built on the device (grid_build.cuh); each
     // direction grid owns its own, so an update rebuilds only the stale ones
@@ -163,16 +157,6 @@ struct ert_scene {
 
 namespace {
 
-bool finite3(const double *v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); }
-bool finite_mat(const ert_material &m)
-{
-    return finite3(m.colour) && std::isfinite(m.specular_power) && std::isfinite(m.shininess) &&
-           std::isfinite(m.reflectivity);
-}
-void push_mat(std::vector<double> &v, const ert_material &m)
-{
-    v.insert(v.end(), {m.colour[0], m.colour[1], m.colour[2], m.specular_power, m.shininess, m.reflectivity});
-}
 float f_up(double x) { return f_round_up(x); }
 
 // the uniform grid that orders the wavefront queues, from the bounds of every [c - |r|, c + |r|]
@@ -208,106 +192,32 @@ bool cell_grid_wanted(double &density)
 
 int flatten(const ert_scene_desc *d, HostScene &h)
 {
-    if (!d) return fail(ERT_ERR_BADARG, "scene descriptor is NULL");
-    if (d->n_lights < 0 || d->n_spheres < 0 || d->n_triangles < 0 || d->n_planes < 0)
-        return fail(ERT_ERR_BADARG, "negative element count");
-    if ((d->n_lights && !d->lights) || (d->n_spheres && !d->spheres) || (d->n_triangles && !d->triangles) ||
-        (d->n_planes && !d->planes))
-        return fail(ERT_ERR_BADARG, "element table pointer is NULL");
-    if (d->n_spheres >= (1 << 28) || d->n_planes >= (1 << 28) || d->n_triangles >= (1 << 28) ||
-        d->n_lights >= (1 << 20))
-        return fail(ERT_ERR_BADARG, "too many elements");
-    const ert_camera &c = d->camera;
-    if (!finite3(c.location) || !std::isfinite(c.fov) || !std::isfinite(c.screen_width) ||
-        !std::isfinite(c.screen_height))
-        return fail(ERT_ERR_BADARG, "camera has a non-finite field");
-    h.camera = c;
-
-    // list positions must be distinct: they decide ties (erl:319) and the light fold order (erl:211)
-    {
-        std::vector<int32_t> all;
-        all.reserve((size_t)(d->n_lights + d->n_spheres + d->n_triangles + d->n_planes));
-        for (int64_t i = 0; i < d->n_lights; i++) all.push_back(d->lights[i].order);
-        for (int64_t i = 0; i < d->n_spheres; i++) all.push_back(d->spheres[i].order);
-        for (int64_t i = 0; i < d->n_triangles; i++) all.push_back(d->triangles[i].order);
-        for (int64_t i = 0; i < d->n_planes; i++) all.push_back(d->planes[i].order);
-        std::sort(all.begin(), all.end());
-        for (size_t i = 0; i < all.size(); i++) {
-            if (all[i] < 0) return fail(ERT_ERR_BADARG, "negative list position in `order`");
-            if (i && all[i] == all[i - 1]) return fail(ERT_ERR_BADARG, "duplicate list position in `order`");
-        }
+    SourceOrder src;
+    std::string err = check_create(d, src, h.order);
+    if (!err.empty()) return fail(ERT_ERR_BADARG, err);
+    double *tab[T_COUNT];
+    for (int t = 0; t < T_COUNT; t++) {
+        h.tab[t].resize(h.order[kTables[t].kind].size() * kTables[t].per);
+        tab[t] = h.tab[t].data();
     }
-
-    // lights, in list order
-    std::vector<int64_t> lidx((size_t)d->n_lights);
-    for (int64_t i = 0; i < d->n_lights; i++) lidx[(size_t)i] = i;
-    std::sort(lidx.begin(), lidx.end(), [&](int64_t a, int64_t b) { return d->lights[a].order < d->lights[b].order; });
-    h.n_lights = (int)d->n_lights;
-    for (int64_t k : lidx) {
-        const ert_point_light &l = d->lights[k];
-        if (!finite3(l.diffuse_colour) || !finite3(l.location) || !finite3(l.specular_colour))
-            return fail(ERT_ERR_BADARG, "point_light has a non-finite field");
-        h.light_order.push_back(l.order);
-        h.lights.insert(h.lights.end(), {l.diffuse_colour[0], l.diffuse_colour[1], l.diffuse_colour[2], l.location[0],
-                                         l.location[1], l.location[2], l.specular_colour[0], l.specular_colour[1],
-                                         l.specular_colour[2]});
-    }
-    h.n_planes = (int)d->n_planes;
-    for (int64_t i = 0; i < d->n_planes; i++) {
-        const ert_plane &p = d->planes[i];
-        if (!finite3(p.normal) || !std::isfinite(p.distance) || !finite_mat(p.material))
-            return fail(ERT_ERR_BADARG, "plane has a non-finite field");
-        h.planes.insert(h.planes.end(), {p.normal[0], p.normal[1], p.normal[2], p.distance});
-        push_mat(h.plane_mat, p.material);
-        h.plane_order.push_back(p.order);
-    }
-    h.n_tris = (int)d->n_triangles;
-    for (int64_t i = 0; i < d->n_triangles; i++) {
-        const ert_triangle &t = d->triangles[i];
-        if (!finite3(t.v1) || !finite3(t.v2) || !finite3(t.v3) || !finite_mat(t.material))
-            return fail(ERT_ERR_BADARG, "triangle has a non-finite field");
-        h.tris.insert(h.tris.end(), {t.v1[0], t.v1[1], t.v1[2], t.v2[0], t.v2[1], t.v2[2], t.v3[0], t.v3[1], t.v3[2]});
-        push_mat(h.tri_mat, t.material);
-        h.tri_order.push_back(t.order);
-    }
-    // spheres, sorted by list position so sphere index order == list order
-    std::vector<int64_t> sidx((size_t)d->n_spheres);
-    for (int64_t i = 0; i < d->n_spheres; i++) sidx[(size_t)i] = i;
-    bool sorted = true;
-    for (int64_t i = 1; i < d->n_spheres; i++)
-        if (d->spheres[i].order < d->spheres[i - 1].order) { sorted = false; break; }
-    if (!sorted)
-        std::sort(sidx.begin(), sidx.end(),
-                  [&](int64_t a, int64_t b) { return d->spheres[a].order < d->spheres[b].order; });
-    h.n_spheres = (int)d->n_spheres;
-    h.sph_exact.resize((size_t)h.n_spheres * 4);
-    h.sph_mat.resize((size_t)h.n_spheres * 6);
-    h.sph_refl.resize((size_t)h.n_spheres);
-    h.sph_order.resize((size_t)h.n_spheres);
+    if (!(err = pack_tables(*d, src, tab)).empty()) return fail(ERT_ERR_BADARG, err);
+    h.camera = d->camera;
+    h.n_lights = (int)d->n_lights; h.n_planes = (int)d->n_planes;
+    h.n_tris = (int)d->n_triangles; h.n_spheres = (int)d->n_spheres;
     h.sph_filter.resize((size_t)h.n_spheres * 4);
     std::vector<double> centers((size_t)h.n_spheres * 3), radii((size_t)h.n_spheres);
-    for (int64_t k = 0; k < d->n_spheres; k++) {
-        const ert_sphere &s = d->spheres[sidx[(size_t)k]];
-        if (!finite3(s.center) || !std::isfinite(s.radius) || !finite_mat(s.material))
-            return fail(ERT_ERR_BADARG, "sphere has a non-finite field");
-        double *e = &h.sph_exact[(size_t)k * 4];
-        e[0] = s.center[0]; e[1] = s.center[1]; e[2] = s.center[2]; e[3] = s.radius;
-        double *m = &h.sph_mat[(size_t)k * 6];
-        m[0] = s.material.colour[0]; m[1] = s.material.colour[1]; m[2] = s.material.colour[2];
-        m[3] = s.material.specular_power; m[4] = s.material.shininess; m[5] = s.material.reflectivity;
-        h.sph_refl[(size_t)k] = s.material.reflectivity;
-        h.sph_order[(size_t)k] = s.order;
+    for (int64_t k = 0; k < h.n_spheres; k++) {
+        const double *c = &h.tab[T_SPH_EXACT][(size_t)k * 4], r = c[3];
         float pad_c, eta_c;
-        make_filter_sphere(s.center, s.radius, &h.sph_filter[(size_t)k * 4], pad_c, eta_c);
+        make_filter_sphere(c, r, &h.sph_filter[(size_t)k * 4], pad_c, eta_c);
         h.pad_c_max = std::max(h.pad_c_max, pad_c);
         h.eta_c_max = std::max(h.eta_c_max, eta_c);
-        float ar = f_up(std::fabs(s.radius));
-        h.r_max = std::max(h.r_max, ar);
+        h.r_max = std::max(h.r_max, f_up(std::fabs(r)));
         for (int a = 0; a < 3; a++) {
-            centers[(size_t)k * 3 + a] = s.center[a];
-            h.abs_max = std::max(h.abs_max, f_up(std::fabs(s.center[a]) + std::fabs(s.radius)));
+            centers[(size_t)k * 3 + a] = c[a];
+            h.abs_max = std::max(h.abs_max, f_up(std::fabs(c[a]) + std::fabs(r)));
         }
-        radii[(size_t)k] = s.radius;
+        radii[(size_t)k] = r;
     }
     {
         // the same filter spheres pair-interleaved for the packed brute-force scan; the padding never passes
@@ -333,7 +243,7 @@ int flatten(const ert_scene_desc *d, HostScene &h)
         });
     }
     h.has_tri_bvh = h.n_tris >= kTriBvhMin;
-    if (h.has_tri_bvh) builders.spawn([&h] { build_triangle_bvh(h.tris.data(), h.n_tris, h.tbvh); });
+    if (h.has_tri_bvh) builders.spawn([&h] { build_triangle_bvh(h.tab[T_TRIS].data(), h.n_tris, h.tbvh); });
     if (h.n_spheres > 0) {
         double lo[3] = {DBL_MAX, DBL_MAX, DBL_MAX}, hi[3] = {-DBL_MAX, -DBL_MAX, -DBL_MAX};
         for (int64_t k = 0; k < h.n_spheres; k++)
@@ -363,7 +273,7 @@ int flatten(const ert_scene_desc *d, HostScene &h)
         for (int g = 0; g < n_grids; g++)
             builders.spawn([&h, &centers, &radii, &lg_built, g, res] {
                 lg_built[(size_t)g] = build_light_grid(centers.data(), radii.data(), h.sph_filter.data(), h.n_spheres,
-                                                       &h.lights[(size_t)g * 9 + 3], res, h.lgrids[(size_t)g]) ? 1 : 0;
+                                                       &h.tab[T_LIGHTS][(size_t)g * 9 + 3], res, h.lgrids[(size_t)g]) ? 1 : 0;
             });
     }
     builders.join();
@@ -516,17 +426,15 @@ int upload_tables(ert_scene *s)
         if ((rc = upload<T>(s, vec, &p__)) != ERT_OK) return rc;                  \
         d.field = reinterpret_cast<decltype(d.field)>(p__);                       \
     } while (0)
-    UP(h.lights, lights, double);
-    UP(h.planes, planes, double);
-    UP(h.plane_mat, plane_mat, double);
-    UP(h.plane_order, plane_order, int);
-    UP(h.tris, tris, double);
-    UP(h.tri_mat, tri_mat, double);
-    UP(h.tri_order, tri_order, int);
-    UP(h.sph_exact, sph_exact, double);
-    UP(h.sph_mat, sph_mat, double);
-    UP(h.sph_refl, sph_refl, double);
-    UP(h.sph_order, sph_order, int);
+    for (int t = 0; t < T_COUNT; t++)
+        if ((rc = upload(s, h.tab[t], &s->tab_dev[t])) != ERT_OK) return rc;
+    const double *const *tp = s->tab_dev;
+    d.lights = tp[T_LIGHTS]; d.planes = tp[T_PLANES]; d.plane_mat = tp[T_PLANE_MAT]; d.tris = tp[T_TRIS];
+    d.tri_mat = tp[T_TRI_MAT]; d.sph_mat = tp[T_SPH_MAT]; d.sph_refl = tp[T_SPH_REFL];
+    d.sph_exact = reinterpret_cast<const double4 *>(tp[T_SPH_EXACT]);
+    UP(h.order[K_PLANES], plane_order, int);
+    UP(h.order[K_TRIS], tri_order, int);
+    UP(h.order[K_SPHERES], sph_order, int);
     UP(h.sph_filter, sph_filter, float);
     UP(h.sph_pairs, sph_pairs, float);
     UP(h.leaf_filter, leaf_filter, float);
@@ -1094,135 +1002,41 @@ int finish_slot(ert_scene *s, Slot &sl)
 
 // ---- in-place update (ert_scene_update) ---------------------------------------------------------------------------
 
-// Scene element i (list position want[i]) is element map[i] of the new table; an empty map is the identity (the
-// caller lists the elements as the scene does, the animation case: one linear pass).
-template <typename E>
-int map_by_order(const E *tab, int64_t n, const std::vector<int> &want, const char *kind, std::vector<int64_t> &map)
-{
-    map.clear();
-    bool same = true;
-    for (int64_t i = 0; i < n && same; i++) same = tab[i].order == want[(size_t)i];
-    if (same) return ERT_OK;
-    std::vector<std::pair<int32_t, int64_t>> got((size_t)n), had((size_t)n);
-    for (int64_t i = 0; i < n; i++) {
-        got[(size_t)i] = {tab[i].order, i};
-        had[(size_t)i] = {want[(size_t)i], i};
-    }
-    std::sort(got.begin(), got.end());
-    std::sort(had.begin(), had.end());
-    for (size_t i = 1; i < got.size(); i++)
-        if (got[i].first == got[i - 1].first)
-            return fail(ERT_ERR_BADARG, std::string("duplicate list position in `order` among the ") + kind);
-    map.assign((size_t)n, 0);
-    for (size_t i = 0; i < got.size(); i++) {
-        if (got[i].first != had[i].first)
-            return fail(ERT_ERR_BADARG, std::string("the ") + kind + " do not have the list positions of the scene's create");
-        map[(size_t)had[i].second] = got[i].second;
-    }
-    return ERT_OK;
-}
-inline int64_t src_of(const std::vector<int64_t> &map, int64_t i) { return map.empty() ? i : map[(size_t)i]; }
+// the new element tables of an update in the staging buffer, and which of them differ from the scene's
+struct UpdateTables { double *p[T_COUNT]; bool changed[T_COUNT]; };
 
-// The element tables an update may upload, in the order they sit in the staging buffer.
-enum { T_LIGHTS, T_PLANES, T_PLANE_MAT, T_TRIS, T_TRI_MAT, T_SPH_EXACT, T_SPH_MAT, T_SPH_REFL, T_COUNT };
-
-struct UpdateTables {
-    double *p[T_COUNT];
-    size_t n[T_COUNT];                 // doubles
-    bool changed[T_COUNT];
-    std::vector<double> *host[T_COUNT];
-    const void *dev[T_COUNT];
-};
-
-// Checks desc against the scene's list shape and every value, and writes the new tables into the staging buffer in
-// the scene's element order.  Nothing of the scene is written.
-int update_stage(ert_scene *s, const ert_scene_desc *d, UpdateTables &t)
+// Checks desc against the scene's list shape and every value, writes the new tables into the staging buffer in the
+// scene's element order and sets inf.changed.  Nothing of the scene is written.
+int update_stage(ert_scene *s, const ert_scene_desc *d, UpdateTables &t, ert_update_info &inf)
 {
     HostScene &h = s->host;
-    if (!d) return fail(ERT_ERR_BADARG, "scene descriptor is NULL");
-    if (d->n_lights != h.n_lights || d->n_spheres != h.n_spheres || d->n_triangles != h.n_tris ||
-        d->n_planes != h.n_planes)
-        return fail(ERT_ERR_BADARG, "element counts differ from the scene's (a new list shape needs ert_scene_create)");
-    if ((d->n_lights && !d->lights) || (d->n_spheres && !d->spheres) || (d->n_triangles && !d->triangles) ||
-        (d->n_planes && !d->planes))
-        return fail(ERT_ERR_BADARG, "element table pointer is NULL");
-    const ert_camera &c = d->camera;
-    if (!finite3(c.location) || !std::isfinite(c.fov) || !std::isfinite(c.screen_width) ||
-        !std::isfinite(c.screen_height))
-        return fail(ERT_ERR_BADARG, "camera has a non-finite field");
-    std::vector<int64_t> ml, ms, mt, mp;
-    int rc;
-    if ((rc = map_by_order(d->lights, d->n_lights, h.light_order, "lights", ml)) != ERT_OK) return rc;
-    if ((rc = map_by_order(d->spheres, d->n_spheres, h.sph_order, "spheres", ms)) != ERT_OK) return rc;
-    if ((rc = map_by_order(d->triangles, d->n_triangles, h.tri_order, "triangles", mt)) != ERT_OK) return rc;
-    if ((rc = map_by_order(d->planes, d->n_planes, h.plane_order, "planes", mp)) != ERT_OK) return rc;
-
-    const DevScene &dv = s->dev;
-    const size_t ns = (size_t)h.n_spheres, nt = (size_t)h.n_tris, np = (size_t)h.n_planes;
-    const size_t counts[T_COUNT] = {9 * (size_t)h.n_lights, 4 * np, 6 * np, 9 * nt, 6 * nt, 4 * ns, 6 * ns, ns};
-    std::vector<double> *host[T_COUNT] = {&h.lights, &h.planes, &h.plane_mat, &h.tris, &h.tri_mat,
-                                          &h.sph_exact, &h.sph_mat, &h.sph_refl};
-    const void *dev[T_COUNT] = {dv.lights, dv.planes, dv.plane_mat, dv.tris, dv.tri_mat, dv.sph_exact, dv.sph_mat,
-                                dv.sph_refl};
-    size_t total = 0;
-    for (int k = 0; k < T_COUNT; k++) total += counts[k];
-    if (s->staging_cap < total * sizeof(double)) {
+    SourceOrder src;
+    std::string err = check_update(d, h.order, src);
+    if (!err.empty()) return fail(ERT_ERR_BADARG, err);
+    size_t off[T_COUNT + 1] = {0};
+    for (int k = 0; k < T_COUNT; k++) off[k + 1] = off[k] + h.tab[k].size();
+    if (s->staging_cap < off[T_COUNT] * sizeof(double)) {
         if (s->staging) CU(cudaFreeHost(s->staging));
         s->staging = nullptr;
         s->staging_cap = 0;
-        if (cudaMallocHost(&s->staging, std::max<size_t>(total, 1) * sizeof(double)) != cudaSuccess) {
+        if (cudaMallocHost(&s->staging, std::max<size_t>(off[T_COUNT], 1) * sizeof(double)) != cudaSuccess) {
             cudaGetLastError();
             s->staging = nullptr;
             return fail(ERT_ERR_NOMEM, "out of pinned host memory for the update's staging buffer");
         }
-        s->staging_cap = total * sizeof(double);
+        s->staging_cap = off[T_COUNT] * sizeof(double);
     }
-    double *p = (double *)s->staging;
+    for (int k = 0; k < T_COUNT; k++) t.p[k] = (double *)s->staging + off[k];
+    if (!(err = pack_tables(*d, src, t.p)).empty()) return fail(ERT_ERR_BADARG, err);
     for (int k = 0; k < T_COUNT; k++) {
-        t.p[k] = p;
-        t.n[k] = counts[k];
-        t.host[k] = host[k];
-        t.dev[k] = dev[k];
-        p += counts[k];
+        const size_t n = h.tab[k].size();
+        t.changed[k] = s->broken || (n && memcmp(t.p[k], h.tab[k].data(), n * sizeof(double)) != 0);
+        if (t.changed[k] && n) inf.changed |= kTables[k].changed;
     }
-    for (int64_t i = 0; i < d->n_lights; i++) {
-        const ert_point_light &l = d->lights[src_of(ml, i)];
-        if (!finite3(l.diffuse_colour) || !finite3(l.location) || !finite3(l.specular_colour))
-            return fail(ERT_ERR_BADARG, "point_light has a non-finite field");
-        double *o = t.p[T_LIGHTS] + 9 * i;
-        for (int a = 0; a < 3; a++) { o[a] = l.diffuse_colour[a]; o[3 + a] = l.location[a]; o[6 + a] = l.specular_colour[a]; }
-    }
-    auto mat = [](double *o, const ert_material &m) {
-        o[0] = m.colour[0]; o[1] = m.colour[1]; o[2] = m.colour[2];
-        o[3] = m.specular_power; o[4] = m.shininess; o[5] = m.reflectivity;
-    };
-    for (int64_t i = 0; i < d->n_planes; i++) {
-        const ert_plane &q = d->planes[src_of(mp, i)];
-        if (!finite3(q.normal) || !std::isfinite(q.distance) || !finite_mat(q.material))
-            return fail(ERT_ERR_BADARG, "plane has a non-finite field");
-        double *o = t.p[T_PLANES] + 4 * i;
-        o[0] = q.normal[0]; o[1] = q.normal[1]; o[2] = q.normal[2]; o[3] = q.distance;
-        mat(t.p[T_PLANE_MAT] + 6 * i, q.material);
-    }
-    for (int64_t i = 0; i < d->n_triangles; i++) {
-        const ert_triangle &q = d->triangles[src_of(mt, i)];
-        if (!finite3(q.v1) || !finite3(q.v2) || !finite3(q.v3) || !finite_mat(q.material))
-            return fail(ERT_ERR_BADARG, "triangle has a non-finite field");
-        double *o = t.p[T_TRIS] + 9 * i;
-        for (int a = 0; a < 3; a++) { o[a] = q.v1[a]; o[3 + a] = q.v2[a]; o[6 + a] = q.v3[a]; }
-        mat(t.p[T_TRI_MAT] + 6 * i, q.material);
-    }
-    for (int64_t i = 0; i < d->n_spheres; i++) {
-        const ert_sphere &q = d->spheres[src_of(ms, i)];
-        if (!finite3(q.center) || !std::isfinite(q.radius) || !finite_mat(q.material))
-            return fail(ERT_ERR_BADARG, "sphere has a non-finite field");
-        double *o = t.p[T_SPH_EXACT] + 4 * i;
-        o[0] = q.center[0]; o[1] = q.center[1]; o[2] = q.center[2]; o[3] = q.radius;
-        mat(t.p[T_SPH_MAT] + 6 * i, q.material);
-        t.p[T_SPH_REFL][i] = q.material.reflectivity;
-    }
-    for (int k = 0; k < T_COUNT; k++)
-        t.changed[k] = s->broken || (t.n[k] && memcmp(t.p[k], host[k]->data(), t.n[k] * sizeof(double)) != 0);
+    for (int64_t i = 0; i < h.n_lights; i++)
+        if (memcmp(&t.p[T_LIGHTS][i * 9 + 3], &h.tab[T_LIGHTS][(size_t)i * 9 + 3], 3 * sizeof(double)) != 0)
+            inf.changed |= ERT_CHANGED_LIGHT_POS;
+    if (memcmp(&d->camera, &h.camera, sizeof d->camera) != 0) inf.changed |= ERT_CHANGED_CAMERA;
     return ERT_OK;
 }
 
@@ -1302,7 +1116,7 @@ int rebuild_tri_bvh(ert_scene *s)
     HostScene &h = s->host;
     DevScene &d = s->dev;
     TriBvh t;
-    build_triangle_bvh(h.tris.data(), h.n_tris, t);
+    build_triangle_bvh(h.tab[T_TRIS].data(), h.n_tris, t);
     if (t.bvh.depth >= kBvhStack) return fail(ERT_ERR_BADARG, "triangle BVH is deeper than the traversal stack");
     int rc;
     const void *old[4] = {d.tri_nodes, d.tri_leaf, d.tri_leaf_id, d.tri_always};
@@ -1349,7 +1163,7 @@ int build_grids_on_device(ert_scene *s, bool cell, const std::vector<char> &need
         for (; keep < need.size(); keep++) {
             if (!need[keep]) continue;
             LightGridDevOut &o = s->lg_buf[keep];
-            CU(build_light_grid_device(d.sph_exact, d.sph_filter, h.n_spheres, &h.lights[keep * 9 + 3], res,
+            CU(build_light_grid_device(d.sph_exact, d.sph_filter, h.n_spheres, &h.tab[T_LIGHTS][keep * 9 + 3], res,
                                        kLightGridMaxEntries, s->grid_tmp, o, st));
             if (!o.ok) break;
         }
@@ -1405,19 +1219,6 @@ int rebuild_grids(ert_scene *s, bool cell, const std::vector<char> &stale, cudaS
 
 // Everything after the checks: the host mirror takes the staged tables, the changed ones go to the device, the
 // kernels of ert_update.cuh recompute what create derived from them, and stale grids are dropped or rebuilt.
-void update_changes(const HostScene &h, const UpdateTables &t, const ert_camera &camera, ert_update_info &inf)
-{
-    for (int64_t i = 0; i < h.n_lights; i++)
-        if (memcmp(&t.p[T_LIGHTS][i * 9 + 3], &h.lights[(size_t)i * 9 + 3], 3 * sizeof(double)) != 0)
-            inf.changed |= ERT_CHANGED_LIGHT_POS;
-    if (memcmp(&camera, &h.camera, sizeof camera) != 0) inf.changed |= ERT_CHANGED_CAMERA;
-    const uint32_t bit[T_COUNT] = {ERT_CHANGED_LIGHTS, ERT_CHANGED_PLANES, ERT_CHANGED_PLANES, ERT_CHANGED_TRIANGLES,
-                                   ERT_CHANGED_TRIANGLE_MAT, ERT_CHANGED_SPHERES, ERT_CHANGED_SPHERE_MAT,
-                                   ERT_CHANGED_SPHERE_MAT};
-    for (int k = 0; k < T_COUNT; k++)
-        if (t.changed[k] && t.n[k]) inf.changed |= bit[k];
-}
-
 int update_apply(ert_scene *s, UpdateTables &t, const ert_camera &camera, uint32_t flags, ert_update_info &inf)
 {
     HostScene &h = s->host;
@@ -1430,7 +1231,7 @@ int update_apply(ert_scene *s, UpdateTables &t, const ert_camera &camera, uint32
     // lights whose direction grid went stale
     std::vector<char> lg_stale(h.lgrids.size(), 0);
     for (size_t g = 0; g < h.lgrids.size(); g++)
-        lg_stale[g] = sph_geo || was_broken || memcmp(&t.p[T_LIGHTS][g * 9 + 3], &h.lights[g * 9 + 3], 3 * sizeof(double)) != 0;
+        lg_stale[g] = sph_geo || was_broken || memcmp(&t.p[T_LIGHTS][g * 9 + 3], &h.tab[T_LIGHTS][g * 9 + 3], 3 * sizeof(double)) != 0;
     s->broken = true;                 // until every step below has succeeded
     h.camera = camera;
     if (!s->upd_dev) CU(cudaMalloc(&s->upd_dev, sizeof(UpdateScalars)));
@@ -1440,10 +1241,10 @@ int update_apply(ert_scene *s, UpdateTables &t, const ert_camera &camera, uint32
 
     CU(cudaEventRecord(s->upd_ev[0], st));
     for (int k = 0; k < T_COUNT; k++) {
-        if (!t.changed[k] || !t.n[k]) continue;
-        const size_t bytes = t.n[k] * sizeof(double);
-        memcpy(t.host[k]->data(), t.p[k], bytes);
-        CU(cudaMemcpyAsync(const_cast<void *>(t.dev[k]), t.p[k], bytes, cudaMemcpyHostToDevice, st));
+        if (!t.changed[k] || h.tab[k].empty()) continue;
+        const size_t bytes = h.tab[k].size() * sizeof(double);
+        memcpy(h.tab[k].data(), t.p[k], bytes);
+        CU(cudaMemcpyAsync(const_cast<double *>(s->tab_dev[k]), t.p[k], bytes, cudaMemcpyHostToDevice, st));
         inf.h2d_bytes += bytes;
     }
     UpdateScalars &u = *s->upd_host;
@@ -1693,7 +1494,7 @@ int ert_scene_update(ert_scene *scene, const ert_scene_desc *desc, uint32_t flag
     UpdateTables t{};
     int rc;
     try {
-        rc = update_stage(scene, desc, t);
+        rc = update_stage(scene, desc, t, inf);
     } catch (const std::exception &) {
         return fail(ERT_ERR_NOMEM, "out of host memory while checking the update");
     }
@@ -1701,7 +1502,6 @@ int ert_scene_update(ert_scene *scene, const ert_scene_desc *desc, uint32_t flag
     // frames already queued render the scene they were queued with
     for (Slot &sl : scene->slots)
         if ((rc = finish_slot(scene, sl)) != ERT_OK) return rc;
-    update_changes(scene->host, t, desc->camera, inf);
     if (!scene->upd_ev[0]) CU(cudaEventCreate(&scene->upd_ev[0]));
     if (!scene->upd_ev[1]) CU(cudaEventCreate(&scene->upd_ev[1]));
     try {
@@ -1733,9 +1533,7 @@ int ert_render_async(ert_scene *scene, const ert_render_params *params, int slot
 
     const ert_render_params &p = *params;
     const ert_camera &cam = p.camera ? *p.camera : scene->host.camera;
-    if (!finite3(cam.location) || !std::isfinite(cam.fov) || !std::isfinite(cam.screen_width) ||
-        !std::isfinite(cam.screen_height))
-        return fail(ERT_ERR_BADARG, "camera has a non-finite field");
+    if (const std::string err = check_camera(cam); !err.empty()) return fail(ERT_ERR_BADARG, err);
 
     FrameParams fp{};
     fp.width = p.width; fp.height = p.height; fp.depth = p.depth; fp.format = p.format;
