@@ -34,6 +34,16 @@ struct Box {
     }
 };
 
+// SAH bin of a centroid at x bins from the range's low end: trunc(x) clamped to [0, nb - 1].  Written with compares
+// before the cast, so that a centroid past the float range (an Inf, or a NaN from Inf - Inf or Inf * 0) lands in an
+// end bin instead of being cast to int, which C++ leaves undefined.
+inline int sah_bin(float x, int nb)
+{
+    if (!(x >= 0.f)) return 0;
+    if (x >= (float)(nb - 1)) return nb - 1;
+    return (int)x;
+}
+
 struct TmpNode {
     Box box;
     int32_t left = -1, right = -1;   // tmp indices; -1 => leaf
@@ -89,8 +99,7 @@ struct Builder {
                 float scale = NB / ext;
                 for (int32_t i = first; i < first + count; i++) {
                     int32_t p = idx[i];
-                    int b = (int)((cen[3 * (size_t)p + a] - clo[a]) * scale);
-                    b = std::min(std::max(b, 0), NB - 1);
+                    const int b = sah_bin((cen[3 * (size_t)p + a] - clo[a]) * scale, NB);
                     bb[b].grow(prim[p]);
                     bc[b]++;
                 }
@@ -127,9 +136,7 @@ struct Builder {
                 int a = best_axis, bbin = best_bin;
                 auto it = std::partition(idx.begin() + first, idx.begin() + first + count,
                                          [&](int32_t p) {
-                                             int b = (int)((cen[3 * (size_t)p + a] - lo) * scale);
-                                             b = std::min(std::max(b, 0), NB - 1);
-                                             return b <= bbin;
+                                             return sah_bin((cen[3 * (size_t)p + a] - lo) * scale, NB) <= bbin;
                                          });
                 mid = (int32_t)(it - idx.begin());
             }

@@ -444,7 +444,15 @@ __device__ __forceinline__ float clamp_dir(float d)
     return d;
 }
 
-__device__ __forceinline__ void make_fray(const DevScene &sc, d3 O, d3 D, FRay &f, bool want_slabs)
+// The range of the filter bounds: a ray may use the FP32 filters, slabs and cells iff |o|_inf + abs_max lies below
+// this.  Then |c - o|^2 <= 3e34 and every slab constant (|o| + m) / d with |d| >= 1e-20 stays far inside float.
+// Beyond it |c - o|^2 - R can overflow to +Inf and stage 1 would reject a sphere the ray hits (DESIGN.md "Filter
+// bounds"), so make_fray / make_sray return false: a walk decides every sphere with the literal test instead
+// (scan_spheres_instead), and the scans that have no tree to leave pass every sphere through the filter (make_fray
+// sets its constants so that both stages do; wf_scan sets its own stage-1 threshold).
+constexpr float kFilterRange = 1e17f;
+
+__device__ __forceinline__ bool make_fray(const DevScene &sc, d3 O, d3 D, FRay &f, bool want_slabs)
 {
     f.a = D.x * D.x + D.y * D.y + D.z * D.z;
     double inv = 1.0 / sqrt(f.a);
@@ -470,6 +478,10 @@ __device__ __forceinline__ void make_fray(const DevScene &sc, d3 O, d3 D, FRay &
         f.nx = -(f.ox + sx) * f.ix; f.ny = -(f.oy + sy) * f.iy; f.nz = -(f.oz + sz) * f.iz;
         f.fx = -(f.ox - sx) * f.ix; f.fy = -(f.oy - sy) * f.iy; f.fz = -(f.oz - sz) * f.iz;
     }
+    // false for NaN and Inf as well; out of range, both stages pass every sphere
+    const bool in_range = oabs + sc.abs_max < kFilterRange;
+    if (!in_range) f.theta = f.bcull = f.m4 = __int_as_float(0x7f800000);
+    return in_range;
 }
 
 // reference Distance of the incumbent -> filter-space cull distance (upper bound)
@@ -562,6 +574,28 @@ __device__ __forceinline__ bool slab_hit(const FRay &f, float lox, float hix, fl
     float tfar = fminf(fminf(t1x, t1y), fminf(t1z, cull));
     // relative slack for the roundings of the six FFMAs
     return tnear - fabsf(tnear) * ERT_REL16 <= tfar + fabsf(tfar) * ERT_REL16;
+}
+
+// A ray beyond the filter's range (make_fray / make_sray returned false) decides every sphere with the literal test,
+// as ERT_ACCEL_EXACT does: no filter, box, cell or direction cell.  `any`: a shadow query seeded with its target,
+// which may stop at the first improvement.  Inlined (as a call, its ABI made ptxas spill in the cell-grid path
+// kernels) and kept to one rolled loop, so that the kernels that never take it keep their size.
+__device__ __forceinline__ Hit scan_spheres_instead(const DevScene *scp, d3 O, d3 D, Hit best, int skip_obj, bool any,
+                                                    int seed_obj)
+{
+    const DevScene &sc = *scp;
+    const double a = D.x * D.x + D.y * D.y + D.z * D.z;
+#pragma unroll 1
+    for (int s = 0; s < sc.n_spheres; s++) {
+        const int code = obj_code(OBJ_SPHERE, s);
+        double t;
+        if (code != skip_obj && sphere_exact(O, D, a, ld_sphere(sc.sph_exact + s), t)) {
+            const int ord = sc.sph_order[s];
+            if (better(t, ord, best)) { best.t = t; best.order = ord; best.obj = code; }
+        }
+        if (any && best.obj != seed_obj) break;
+    }
+    return best;
 }
 
 // ERT_ACCEL_BVH
@@ -878,8 +912,8 @@ __device__ __forceinline__ void resolve_free(const DevScene &sc, Query &q, Tally
         scan_spheres_exact<COUNT>(sc, q.O, q.D, a, q.best, skip, q.any, q.seed_obj, tl);
     } else {
         FRay f;
-        make_fray(sc, q.O, q.D, f, true);
-        scan_spheres_bvh<COUNT>(sc, q.O, q.D, f, q.best, skip, q.any, q.seed_obj, tl);
+        if (make_fray(sc, q.O, q.D, f, true)) scan_spheres_bvh<COUNT>(sc, q.O, q.D, f, q.best, skip, q.any, q.seed_obj, tl);
+        else q.best = scan_spheres_instead(&sc, q.O, q.D, q.best, skip, q.any, q.seed_obj);
     }
 }
 
@@ -975,7 +1009,7 @@ render_tiled_kernel(const __grid_constant__ DevScene sc, const __grid_constant__
             if (q.any && q.best.obj != q.seed_obj) active = false;
         }
         if (active) {
-            make_fray(sc, q.O, q.D, f, false);
+            make_fray(sc, q.O, q.D, f, false);          // out of range: every sphere passes the filter
             cull = cull_from(f, q.best);
         }
         if (n_tiles > 0 && !resident) {
@@ -1059,7 +1093,7 @@ trace_rays_kernel(const __grid_constant__ DevScene sc, long long n_rays, const d
         // same filter as the tiled kernel, spheres read straight from global memory
         scan_others<false, TRI>(sc, q.O, q.D, q.best, -1, tl);
         FRay f;
-        make_fray(sc, q.O, q.D, f, false);
+        make_fray(sc, q.O, q.D, f, false);              // out of range: every sphere passes the filter
         float cull = cull_from(f, q.best);
         for (int s = 0; s < sc.n_spheres; s++)
             try_sphere<false>(sc, f, q.O, q.D, __ldg(sc.sph_filter + s), s, -1, q.best, cull, tl);
@@ -1107,7 +1141,7 @@ trace_rays_warp_kernel(const __grid_constant__ DevScene sc, long long n_rays, co
     best.order = __shfl_sync(0xffffffffu, best.order, 0);
     best.obj = __shfl_sync(0xffffffffu, best.obj, 0);
     FRay f;
-    make_fray(sc, O, D, f, false);
+    make_fray(sc, O, D, f, false);                      // out of range: every sphere passes the filter
     float cull = cull_from(f, best);
     for (int s = lane; s < sc.n_spheres; s += 32)
         try_sphere<false>(sc, f, O, D, __ldg(sc.sph_filter + s), s, -1, best, cull, tl);

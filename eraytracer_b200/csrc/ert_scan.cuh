@@ -279,7 +279,7 @@ wf_scan(const __grid_constant__ DevScene sc, const __grid_constant__ FrameParams
 #pragma unroll
             for (int r = 0; r < kScanRays; r++) {
                 const unsigned long long i = beta * kScanBatch + (unsigned long long)(warp * kScanRays + r) * 32 + lane;
-                bool search = false;
+                bool search = false, filtered = false;
                 SRay f;
                 f.ox = f.oy = f.oz = 0.f; f.dx = f.dy = 0.f; f.dz = 1.f; f.theta = 0.f;
                 if (i < n) {
@@ -292,14 +292,13 @@ wf_scan(const __grid_constant__ DevScene sc, const __grid_constant__ FrameParams
                     if constexpr (SHADOW) search = !wf.sp_occ[i];     // target missed, or a plane/triangle in front of it
                     if (search) {
                         double a2, inv;
-                        make_sray(sc, O, D, f, a2, inv);
+                        filtered = make_sray(sc, O, D, f, a2, inv);
                     }
                 }
                 ox[r] = f.ox; oy[r] = f.oy; oz[r] = f.oz; dx[r] = f.dx; dy[r] = f.dy; dz[r] = f.dz;
-                const float oabs = fmaxf(fmaxf(fabsf(f.ox), fabsf(f.oy)), fabsf(f.oz));
-                // fmaxf drops NaNs and the filter must pass them: a ray whose v could be Inf - Inf has every group
-                // looked at closely (coordinates beyond 1e17, never in practice)
-                nth[r] = !search ? kInf : ((oabs + sc.abs_max < 1e17f) ? -f.theta : -kInf);
+                // a ray beyond the filter's range (make_sray) has every group looked at closely and every sphere
+                // pass stage 1, whatever the NaNs and Infs its v holds (fmaxf drops NaNs)
+                nth[r] = !search ? kInf : (filtered ? -f.theta : -kInf);
             }
         }
         const unsigned int stage = q % kScanStages, use = q / kScanStages;

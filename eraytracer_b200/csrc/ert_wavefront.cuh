@@ -163,7 +163,10 @@ struct RaySlot {
 constexpr int kRaySlotDoubles = 6;
 #define ERT_KAPPA 1.00006103515625f   /* 1 + 2^-14 >= (1+2^-16)/(1-2^-16): slab slack as one factor */
 
-__device__ __forceinline__ void make_sray(const DevScene &sc, d3 O, d3 D, SRay &f, double &a_out, double &inv_out)
+// Returns false for a ray beyond the filter's range (kFilterRange, as make_fray); its constants are then left as
+// they are, and the callers do not filter with them: a walk decides every sphere with scan_spheres_instead instead,
+// and wf_scan passes every sphere through stage 1.  (Its m4 exceeds every cell grid's eps, see grid_begin.)
+__device__ __forceinline__ bool make_sray(const DevScene &sc, d3 O, d3 D, SRay &f, double &a_out, double &inv_out)
 {
     const double a = D.x * D.x + D.y * D.y + D.z * D.z;
     // 1/sqrt(a): directions are unit vectors up to rounding except after a bounce off an
@@ -189,6 +192,7 @@ __device__ __forceinline__ void make_sray(const DevScene &sc, d3 O, d3 D, SRay &
     f.ix = __frcp_rn(clamp_dir(f.dx)); f.iy = __frcp_rn(clamp_dir(f.dy)); f.iz = __frcp_rn(clamp_dir(f.dz));
     f.klx = -(f.ox + m) * f.ix; f.kly = -(f.oy + m) * f.iy; f.klz = -(f.oz + m) * f.iz;
     f.khx = -(f.ox - m) * f.ix; f.khy = -(f.oy - m) * f.iy; f.khz = -(f.oz - m) * f.iz;
+    return oabs + sc.abs_max < kFilterRange;                // false for NaN and Inf as well
 }
 
 __device__ __forceinline__ void prefetch_l1(const void *p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
@@ -642,7 +646,8 @@ __device__ __forceinline__ void grid_big_spheres(const DevScene &sc, const SRay 
 }
 
 // A ray whose margin is too large for the grid (origin far outside the scene) walks the BVH
-// instead.  Rare, so it is a call: the walk state of the BVH stays out of the callers' registers.
+// instead, and a ray beyond the filter's range tests every sphere.  Rare, so it is a call: the
+// walk state of the BVH stays out of the callers' registers.
 __device__ __forceinline__ void walk_bvh_instead(const DevScene *scp, double *slot, int skip_obj, Hit *best_io)
 {
     const DevScene &sc = *scp;
@@ -650,7 +655,10 @@ __device__ __forceinline__ void walk_bvh_instead(const DevScene *scp, double *sl
     ray.p = slot;
     SRay f;
     double a, inv;
-    make_sray(sc, ray.O(), ray.D(), f, a, inv);
+    if (!make_sray(sc, ray.O(), ray.D(), f, a, inv)) {
+        *best_io = scan_spheres_instead(scp, ray.O(), ray.D(), *best_io, skip_obj, false, -1);
+        return;
+    }
     Hit best = *best_io;
     Tally<false> tl;
     Trav<false> tr;
@@ -715,7 +723,10 @@ __device__ void trace_ray_wavefront(const DevScene &sc, d3 O, d3 D, Hit &best)
     Trav<false> tr;
     int stack[kBvhStack];
     double a, inv;
-    make_sray(sc, O, D, f, a, inv);
+    if (!make_sray(sc, O, D, f, a, inv)) {
+        best = scan_spheres_instead(&sc, O, D, best, -1, false, -1);
+        return;
+    }
     ray.put(O, D, a, inv);
     trav_start(tr, stack, f, inv, best);
     while (!trav_step<false, false>(tr, stack, sc, ray, f, best, -1, -1, tl)) { }
@@ -1098,7 +1109,7 @@ wf_trace_path(const __grid_constant__ DevScene sc, const __grid_constant__ Frame
                     rays++;
                     scan_others<COUNT, TRI>(sc, O, D, best, -1, tl);
                     double a, inv;
-                    make_sray(sc, O, D, f, a, inv);
+                    const bool filtered = make_sray(sc, O, D, f, a, inv);
                     ray.put(O, D, a, inv);
                     if (sc.n_spheres > 0) {
                         if (FIRST && hint >= 0) {                     // first reflections have too little in common (measured: 7.505 vs 7.487 ms)
@@ -1117,6 +1128,8 @@ wf_trace_path(const __grid_constant__ DevScene sc, const __grid_constant__ Frame
                         }
                         if constexpr (GRID) {
                             walking = grid_begin<COUNT>(gw, gr, sc, ray, f, inv, skip, best, tl);
+                        } else if (!filtered) {
+                            best = scan_spheres_instead(&sc, O, D, best, skip, false, -1);
                         } else {
                             Trav<false> tr;
                             int stack[kBvhStack];
@@ -1269,7 +1282,7 @@ wf_trace_path_refill(const __grid_constant__ DevScene sc, const __grid_constant_
                     scan_others<COUNT, TRI>(sc, O, D, best, -1, tl);
                     if (sc.n_spheres > 0) {
                         double a, inv;
-                        make_sray(sc, O, D, f, a, inv);
+                        const bool filtered = make_sray(sc, O, D, f, a, inv);
                         ray.put(O, D, a, inv);
                         if constexpr (GRID) {
                             if (f.m4 <= sc.cg.eps) {
@@ -1282,6 +1295,9 @@ wf_trace_path_refill(const __grid_constant__ DevScene sc, const __grid_constant_
                                 best = tmp;
                                 gw.id = -1;                  // the first step reports the ray as done
                             }
+                        } else if (!filtered) {
+                            best = scan_spheres_instead(&sc, O, D, best, -1, false, -1);
+                            tr.node = kTravDone;             // the first step reports the ray as done
                         } else {
                             trav_start(tr, stack, f, inv, best);
                         }
@@ -1485,13 +1501,16 @@ wf_trace_shadow(const __grid_constant__ DevScene sc, const __grid_constant__ Fra
                         // this light has a direction grid: a few candidates, no walk
                         SRay f;
                         double a2, inv;
-                        make_sray(sc, O, D, f, a2, inv);
-                        lit = !light_grid_occluded<COUNT>(sc, sc.lgrids[l], f, O, D, a, inv, best, target, tl);
+                        if (make_sray(sc, O, D, f, a2, inv))
+                            lit = !light_grid_occluded<COUNT>(sc, sc.lgrids[l], f, O, D, a, inv, best, target, tl);
+                        else
+                            lit = scan_spheres_instead(&sc, O, D, best, target, true, target).obj == target;
                     } else if (lit && sc.n_spheres > 0) {
                         SRay f;
                         double a2, inv;
-                        make_sray(sc, O, D, f, a2, inv);
-                        // the warp's recent occluders, FP32 filter first
+                        const bool filtered = make_sray(sc, O, D, f, a2, inv);
+                        // the warp's recent occluders, FP32 filter first (out of range it may drop one: the literal
+                        // scan below finds it)
                         const float cull0 = cullk_from(f, inv, best);
                         for (int k = 0; k < kOccCache && lit; k++) {
                             const float4 fs = occ_f[k];
@@ -1509,7 +1528,10 @@ wf_trace_shadow(const __grid_constant__ DevScene sc, const __grid_constant__ Fra
                                 }
                             }
                         }
-                        if (lit) {
+                        if (lit && !filtered) {
+                            best = scan_spheres_instead(&sc, O, D, best, target, true, target);
+                            lit = best.obj == target;
+                        } else if (lit) {
                             ray.put(O, D, a2, inv);
                             Trav<true> tr;
                             int stack[kBvhStack];
@@ -1803,8 +1825,10 @@ wf_shadow_shade(const __grid_constant__ DevScene sc, const __grid_constant__ Fra
                     if (lit && sc.n_spheres > 0) {
                         SRay f;
                         double a2, inv;
-                        make_sray(sc, O, D, f, a2, inv);
-                        lit = !light_grid_occluded<COUNT>(sc, sc.lgrids[l], f, O, D, a, inv, best, tgt, tl);
+                        if (make_sray(sc, O, D, f, a2, inv))
+                            lit = !light_grid_occluded<COUNT>(sc, sc.lgrids[l], f, O, D, a, inv, best, tgt, tl);
+                        else
+                            lit = scan_spheres_instead(&sc, O, D, best, tgt, true, tgt).obj == tgt;
                     }
                     if (lit) atomicOr(sh_lit + slot, 1u << l);
                     PROBE(2, lit ? 1u : 0u);
