@@ -298,7 +298,8 @@ static ERL_NIF_TERM nif_scene_clone(ErlNifEnv *env, int argc, const ERL_NIF_TERM
 }
 
 /* Opts: proplist of {format, rgb8|f32|f64} | {accel, auto|exact|linear|bvh|bvh_mega|grid} |
- *       {part, {BandRows, NParts, Part}} | {camera, CameraRecord} */
+ *       {part, {BandRows, NParts, Part}} | {camera, CameraRecord} |
+ *       {supersample, N}: N x N rays per pixel, box-filtered, N an integer in 1..ERT_MAX_SUPERSAMPLE (8) */
 static int decode_opts(ErlNifEnv *env, ERL_NIF_TERM opts, ert_render_params *p, ert_camera *cam)
 {
     ERL_NIF_TERM head, tail = opts;
@@ -325,6 +326,9 @@ static int decode_opts(ErlNifEnv *env, ERL_NIF_TERM opts, ert_render_params *p, 
             if (!enif_get_tuple(env, e[1], &a3, &q) || a3 != 3) return 0;
             if (!enif_get_int(env, q[0], &p->band_rows) || !enif_get_int(env, q[1], &p->n_parts) ||
                 !enif_get_int(env, q[2], &p->part))
+                return 0;
+        } else if (is_atom_named(env, e[0], "supersample")) {
+            if (!enif_get_int(env, e[1], &p->supersample) || p->supersample < 1 || p->supersample > ERT_MAX_SUPERSAMPLE)
                 return 0;
         } else if (is_atom_named(env, e[0], "camera")) {
             if (!get_camera(env, e[1], cam)) return 0;

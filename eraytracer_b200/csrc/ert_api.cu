@@ -23,6 +23,7 @@
 #include "ert_device.cuh"
 #include "ert_wavefront.cuh"
 #include "ert_scan.cuh"
+#include "ert_supersample.cuh"
 #include "ert_update.cuh"
 #include "grid_build.cuh"
 #include "scene_math.h"
@@ -111,8 +112,13 @@ struct Slot {
     unsigned int *wf_ctr = nullptr;
     int wf_ctr_depth = 0;
     unsigned int *wf_ctr_host = nullptr;           // pinned, for the early-out check of deep recursions
-    unsigned int *wf_ctr_all_host = nullptr;       // pinned, the counters of the first ERT_MAX_BOUNCE_STATS levels
+    unsigned int *wf_ctr_all_host = nullptr;       // pinned, the counters of the first ERT_MAX_BOUNCE_STATS levels,
+    int wf_ctr_all_passes = 0;                     // one set per sample pass, room for this many passes
     int wf_levels = 0;                             // levels copied there by the last wavefront frame
+    int wf_passes = 0;                             // ... in this many sample passes
+    // supersampled frames: the F64 accumulator and the buffer of the pass being folded, allocated on first use
+    double *ss_acc = nullptr, *ss_pass = nullptr;
+    size_t ss_cap = 0;                             // bytes of each
     std::vector<cudaEvent_t> ticks;                // ERT_FLAG_TIME_KERNELS: one event before/after every launch
     std::vector<int> tick_class;                   // class of the launch between ticks[i] and ticks[i+1]
     unsigned long long *counters_dev = nullptr;
@@ -559,6 +565,8 @@ void destroy(ert_scene *s)
         if (sl.wf_ctr) cudaFree(sl.wf_ctr);
         if (sl.wf_ctr_host) cudaFreeHost(sl.wf_ctr_host);
         if (sl.wf_ctr_all_host) cudaFreeHost(sl.wf_ctr_all_host);
+        if (sl.ss_acc) cudaFree(sl.ss_acc);
+        if (sl.ss_pass) cudaFree(sl.ss_pass);
         for (cudaEvent_t e : sl.ticks) cudaEventDestroy(e);
         for (cudaEvent_t e : sl.ev_path) cudaEventDestroy(e);
         for (cudaEvent_t e : sl.ev_shade) cudaEventDestroy(e);
@@ -607,6 +615,10 @@ int check_params(const ert_render_params *p)
     if (p->n_parts > 1 && p->band_rows > 0 && (p->part < 0 || p->part >= p->n_parts))
         return fail(ERT_ERR_BADARG, "part must be in [0, n_parts)");
     if (p->band_rows < 0) return fail(ERT_ERR_BADARG, "band_rows must be >= 0");
+    if (p->supersample < 0 || p->supersample > ERT_MAX_SUPERSAMPLE)
+        return fail(ERT_ERR_BADARG, "supersample must be in [0, ERT_MAX_SUPERSAMPLE]");
+    if ((int64_t)p->width * std::max(p->supersample, 1) > INT32_MAX || (int64_t)p->height * std::max(p->supersample, 1) > INT32_MAX)
+        return fail(ERT_ERR_BADARG, "supersample * width and supersample * height must fit in int32");
     return ERT_OK;
 }
 
@@ -686,7 +698,7 @@ void launch_trace_rays(int accel, unsigned blocks, cudaStream_t st, const DevSce
 // ---- wavefront frame (ERT_ACCEL_BVH) ------------------------------------------------------
 size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
-int wf_prepare(ert_scene *s, Slot &sl, const FrameParams &fp, WfBuf &wf, bool scan)
+int wf_prepare(ert_scene *s, Slot &sl, const FrameParams &fp, WfBuf &wf, bool scan, int passes)
 {
     int tiles_x = (fp.width + 7) / 8, tiles_y = (fp.local_rows + 3) / 4;
     size_t n_pad = (size_t)tiles_x * (size_t)tiles_y * 32;
@@ -718,7 +730,12 @@ int wf_prepare(ert_scene *s, Slot &sl, const FrameParams &fp, WfBuf &wf, bool sc
         sl.wf_ctr_depth = fp.depth;
     }
     if (!sl.wf_ctr_host) CU(cudaMallocHost(&sl.wf_ctr_host, kWfCtr * sizeof(unsigned int)));
-    if (!sl.wf_ctr_all_host) CU(cudaMallocHost(&sl.wf_ctr_all_host, ERT_MAX_BOUNCE_STATS * kWfCtr * sizeof(unsigned int)));
+    if (sl.wf_ctr_all_passes < passes) {
+        if (sl.wf_ctr_all_host) CU(cudaFreeHost(sl.wf_ctr_all_host));
+        sl.wf_ctr_all_host = nullptr; sl.wf_ctr_all_passes = 0;
+        CU(cudaMallocHost(&sl.wf_ctr_all_host, (size_t)passes * ERT_MAX_BOUNCE_STATS * kWfCtr * sizeof(unsigned int)));
+        sl.wf_ctr_all_passes = passes;
+    }
     unsigned char *base = (unsigned char *)sl.wf_mem;
     double *d = (double *)(base + o_dbl);
     int *i = (int *)(base + o_int);
@@ -757,17 +774,18 @@ int wf_prepare(ert_scene *s, Slot &sl, const FrameParams &fp, WfBuf &wf, bool sc
 
 template <bool COUNT, bool TRI>
 int launch_wavefront(ert_scene *s, Slot &sl, const FrameParams &fp_in, bool unsorted, bool no_grid, bool timed,
-                     bool scan, bool cells, uint64_t *launches)
+                     bool scan, bool cells, int pass, int passes, uint64_t *launches)
 {
     WfBuf wf{};
     int rc;
     const FrameParams &fp = fp_in;
-    if ((rc = wf_prepare(s, sl, fp, wf, scan)) != ERT_OK) return rc;
+    if ((rc = wf_prepare(s, sl, fp, wf, scan, passes)) != ERT_OK) return rc;
     cudaStream_t st = sl.stream;
     FrameParams fps = fp;                           // shadow kernels count into the second counter set
     fps.counters = fp.counters + CNT_N;
-    size_t n_ticks = 0;
-    sl.tick_class.clear();
+    // the sample passes of a supersampled frame append their events to those of the passes before them
+    if (pass == 0) sl.tick_class.clear();
+    size_t n_ticks = pass == 0 ? 0 : sl.tick_class.size() + 1;
     auto tick = [&](int cls) -> int {              // cls < 0: the opening event
         if (!timed) return ERT_OK;
         if (n_ticks == sl.ticks.size()) {
@@ -780,7 +798,7 @@ int launch_wavefront(ert_scene *s, Slot &sl, const FrameParams &fp_in, bool unso
         return ERT_OK;
     };
 #define TICK(cls) do { if ((rc = tick(cls)) != ERT_OK) return rc; } while (0)
-    TICK(-1);
+    TICK(pass == 0 ? -1 : 2);                      // since the previous pass: its fold into the accumulator
     const DevScene &d = s->dev;
     CU(cudaMemsetAsync(wf.ctr, 0, (size_t)fp.depth * kWfCtr * sizeof(unsigned int), st));
     // the brute-force scan starts from a cleared colour buffer; the path kernels of bounce 0 clear it themselves
@@ -934,8 +952,9 @@ int launch_wavefront(ert_scene *s, Slot &sl, const FrameParams &fp_in, bool unso
     n++;
     TICK(2);
     sl.wf_levels = std::min(fp.depth, (int)ERT_MAX_BOUNCE_STATS);
-    CU(cudaMemcpyAsync(sl.wf_ctr_all_host, wf.ctr, (size_t)sl.wf_levels * kWfCtr * sizeof(unsigned int),
-                       cudaMemcpyDeviceToHost, st));
+    sl.wf_passes = pass + 1;
+    CU(cudaMemcpyAsync(sl.wf_ctr_all_host + (size_t)pass * ERT_MAX_BOUNCE_STATS * kWfCtr, wf.ctr,
+                       (size_t)sl.wf_levels * kWfCtr * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
     CU(cudaGetLastError());
 #undef WF_CHECK
 #undef TICK
@@ -977,11 +996,16 @@ int finish_slot(ert_scene *s, Slot &sl)
 #endif
     sl.stats.bounces_recorded = sl.wf_levels;
     for (int b = 0; b < sl.wf_levels; b++) {
-        const unsigned int *c = sl.wf_ctr_all_host + (size_t)b * kWfCtr;
-        sl.stats.bounce_hits[b] = c[WF_NHITS];
-        sl.stats.bounce_path_rays[b] = b == 0 ? sl.stats.pixels : sl.wf_ctr_all_host[(size_t)(b - 1) * kWfCtr + WF_NNEXT];
+        // summed over the sample passes of a supersampled frame
+        sl.stats.bounce_path_rays[b] = b == 0 ? sl.stats.pixels * (uint64_t)sl.wf_passes : 0;
+        for (int k = 0; k < sl.wf_passes; k++) {
+            const unsigned int *c = sl.wf_ctr_all_host + (size_t)k * ERT_MAX_BOUNCE_STATS * kWfCtr;
+            sl.stats.bounce_hits[b] += c[(size_t)b * kWfCtr + WF_NHITS];
+            if (b > 0) sl.stats.bounce_path_rays[b] += c[(size_t)(b - 1) * kWfCtr + WF_NNEXT];
+        }
     }
     sl.wf_levels = 0;
+    sl.wf_passes = 0;
     sl.stats.has_cell_grid = s->host.cgrid.enabled ? 1 : 0;
     sl.stats.path_box_tests = c0[CNT_BOX]; sl.stats.path_filter_tests = c0[CNT_FILTER];
     sl.stats.shadow_box_tests = c1[CNT_BOX]; sl.stats.shadow_filter_tests = c1[CNT_FILTER];
@@ -1544,6 +1568,10 @@ int ert_render_async(ert_scene *scene, const ert_render_params *params, int slot
     // focal_length/2 (erl:483-484) with the host libm's tan, as BEAM's math:tan would
     fp.focal = cam.screen_width / (2 * tan(cam.fov * (M_PI / 180) / 2));
     fp.screen_w = cam.screen_width; fp.screen_h = cam.screen_height;
+    const int ss = std::max(p.supersample, 1);
+    const int passes = ss * ss;
+    fp.ss = ss;
+    fp.ray_w = (double)ss * p.width; fp.ray_h = (double)ss * p.height;
 
     size_t fb_bytes = (size_t)std::max(fp.local_rows, 1) * (size_t)p.width * 3 * bytes_per_channel(p.format);
     if (sl.fb_cap < fb_bytes) {
@@ -1554,6 +1582,18 @@ int ert_render_async(ert_scene *scene, const ert_render_params *params, int slot
     }
     fp.out = sl.fb;
     fp.counters = sl.counters_dev;
+    const size_t n_px = (size_t)fp.local_rows * (size_t)p.width;
+    if (ss > 1 && sl.ss_cap < n_px * 3 * sizeof(double)) {
+        if (sl.ss_acc) CU(cudaFree(sl.ss_acc));
+        if (sl.ss_pass) CU(cudaFree(sl.ss_pass));
+        sl.ss_acc = sl.ss_pass = nullptr; sl.ss_cap = 0;
+        if (cudaMalloc(&sl.ss_acc, n_px * 3 * sizeof(double)) != cudaSuccess ||
+            cudaMalloc(&sl.ss_pass, n_px * 3 * sizeof(double)) != cudaSuccess) {
+            cudaGetLastError();
+            return fail(ERT_ERR_NOMEM, "out of device memory for the supersampling accumulator");
+        }
+        sl.ss_cap = n_px * 3 * sizeof(double);
+    }
 
     sl.params = p;
     sl.params.camera = nullptr;
@@ -1569,32 +1609,48 @@ int ert_render_async(ert_scene *scene, const ert_render_params *params, int slot
     // the wavefront serves the BVH strategy and, past one resident tile of spheres, the brute-force scan
     const bool wf_scan = accel == ERT_ACCEL_LINEAR && scene->host.n_spheres > kWfScanFrom;
     const bool wf_cells = accel == ERT_ACCEL_GRID;
-    if (fp.local_rows > 0 && (accel == ERT_ACCEL_BVH || wf_cells || wf_scan) && fp.depth > 0) {
-        uint64_t n = 0;
-        const bool unsorted = (p.flags & ERT_FLAG_WF_UNSORTED) != 0;
-        const bool no_grid = (p.flags & ERT_FLAG_NO_LIGHT_GRID) != 0;
-        const bool timed = (p.flags & ERT_FLAG_TIME_KERNELS) != 0;
-        const bool count = (p.flags & ERT_FLAG_COUNT_TESTS) != 0;
-        if (scene->host.has_tri_bvh)
-            rc = count ? launch_wavefront<true, true>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, &n)
-                       : launch_wavefront<false, true>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, &n);
-        else
-            rc = count ? launch_wavefront<true, false>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, &n)
-                       : launch_wavefront<false, false>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, &n);
-        if (rc != ERT_OK) return rc;
-        sl.stats.gpu_launches = n;
-    } else if (fp.local_rows > 0) {
-        dim3 grid((unsigned)((p.width + 31) / 32), (unsigned)((fp.local_rows + 7) / 8));
-        const bool count = (p.flags & ERT_FLAG_COUNT_TESTS) != 0;
-        if (scene->host.has_tri_bvh) {
-            if (count) launch_render<true, true>(accel, grid, sl.stream, scene->dev, fp);
-            else launch_render<false, true>(accel, grid, sl.stream, scene->dev, fp);
-        } else {
-            if (count) launch_render<true, false>(accel, grid, sl.stream, scene->dev, fp);
-            else launch_render<false, false>(accel, grid, sl.stream, scene->dev, fp);
+    // A supersampled frame is ss*ss sample passes of the strategy's launches, each in F64 into the accumulator
+    // (pass 0) or the pass buffer (the others, folded into the accumulator after the pass).
+    for (int k = 0; k < passes && fp.local_rows > 0; k++) {
+        if (ss > 1) {
+            fp.ss_i = k % ss; fp.ss_j = k / ss;
+            fp.format = ERT_FMT_F64;
+            fp.out = k == 0 ? sl.ss_acc : sl.ss_pass;
         }
-        CU(cudaGetLastError());
-        sl.stats.gpu_launches = 1;
+        if ((accel == ERT_ACCEL_BVH || wf_cells || wf_scan) && fp.depth > 0) {
+            uint64_t n = 0;
+            const bool unsorted = (p.flags & ERT_FLAG_WF_UNSORTED) != 0;
+            const bool no_grid = (p.flags & ERT_FLAG_NO_LIGHT_GRID) != 0;
+            const bool timed = (p.flags & ERT_FLAG_TIME_KERNELS) != 0;
+            const bool count = (p.flags & ERT_FLAG_COUNT_TESTS) != 0;
+            if (scene->host.has_tri_bvh)
+                rc = count ? launch_wavefront<true, true>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, k, passes, &n)
+                           : launch_wavefront<false, true>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, k, passes, &n);
+            else
+                rc = count ? launch_wavefront<true, false>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, k, passes, &n)
+                           : launch_wavefront<false, false>(scene, sl, fp, unsorted, no_grid, timed, wf_scan, wf_cells, k, passes, &n);
+            if (rc != ERT_OK) return rc;
+            sl.stats.gpu_launches += n;
+        } else {
+            dim3 grid((unsigned)((p.width + 31) / 32), (unsigned)((fp.local_rows + 7) / 8));
+            const bool count = (p.flags & ERT_FLAG_COUNT_TESTS) != 0;
+            if (scene->host.has_tri_bvh) {
+                if (count) launch_render<true, true>(accel, grid, sl.stream, scene->dev, fp);
+                else launch_render<false, true>(accel, grid, sl.stream, scene->dev, fp);
+            } else {
+                if (count) launch_render<true, false>(accel, grid, sl.stream, scene->dev, fp);
+                else launch_render<false, false>(accel, grid, sl.stream, scene->dev, fp);
+            }
+            CU(cudaGetLastError());
+            sl.stats.gpu_launches += 1;
+        }
+        if (k > 0) {
+            // the fold of the last pass divides by ss*ss and writes the requested format into the framebuffer
+            if (k + 1 < passes) ss_fold<false><<<scene->wf_grid_fin, 256, 0, sl.stream>>>(sl.ss_pass, sl.ss_acc, n_px, passes, p.format, sl.fb);
+            else ss_fold<true><<<scene->wf_grid_fin, 256, 0, sl.stream>>>(sl.ss_pass, sl.ss_acc, n_px, passes, p.format, sl.fb);
+            CU(cudaGetLastError());
+            sl.stats.gpu_launches += 1;
+        }
     }
     CU(cudaEventRecord(sl.ev1, sl.stream));
     CU(cudaMemcpyAsync(sl.counters_host, sl.counters_dev, kCounterSets * CNT_N * sizeof(unsigned long long),

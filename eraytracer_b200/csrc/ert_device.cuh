@@ -104,6 +104,11 @@ struct FrameParams {
     double screen_w, screen_h;
     void *out;                   // compact framebuffer of this part: local_rows * width pixels
     unsigned long long *counters;
+    // ray space: pixel (X, Y) casts the ray of pixel (ss*X + ss_i, ss*Y + ss_j) of the (ss*width) x (ss*height)
+    // frame (one sample pass of a supersampled frame; a plain frame has ss = 1, ss_i = ss_j = 0).  Last in the
+    // struct, with ray_w = ss*width and ray_h = ss*height as exact doubles: the existing kernels keep their registers.
+    int ss, ss_i, ss_j;
+    double ray_w, ray_h;
 };
 
 #ifdef ERT_PROBE
@@ -661,11 +666,11 @@ struct Query {
     bool need;          // false: nothing to search (lane idle or target missed)
 };
 
-// erl:486-511, with X/Width and Y/Height as at erl:95-97
+// erl:486-511, with X/Width and Y/Height as at erl:95-97 in ray space (the host keeps ss*width, ss*height <= INT32_MAX)
 __device__ __forceinline__ void primary_ray(const FrameParams &fp, int X, int Y, d3 &O, d3 &D)
 {
-    double x = (double)X / (double)fp.width;
-    double y = (double)Y / (double)fp.height;
+    double x = (double)(X * fp.ss + fp.ss_i) / fp.ray_w;
+    double y = (double)(Y * fp.ss + fp.ss_j) / fp.ray_h;
     d3 loc = mk(fp.cam[0], fp.cam[1], fp.cam[2]);
     d3 acc = loc;
     acc = vadd(vscale(mk(0.0, 0.0, 1.0), fp.focal), acc);
@@ -831,13 +836,13 @@ __device__ __forceinline__ void pix_consume(Pix &p, const DevScene &sc, const Fr
     }
 }
 
-__device__ __forceinline__ void pix_store(const Pix &p, const FrameParams &fp, int X, int local_y)
+// The one quantisation rule of every output format: colour C of element triple idx of `out`.
+__device__ __forceinline__ void colour_store(void *out, int format, size_t idx, d3 C)
 {
-    size_t idx = ((size_t)local_y * fp.width + X) * 3;
-    if (fp.format == 0) {
+    if (format == 0) {
         // erl:678-680: min(trunc(C*255), 255); negative values clamp to 0 in the byte format
-        unsigned char *o = (unsigned char *)fp.out + idx;
-        double c[3] = {p.C.x, p.C.y, p.C.z};
+        unsigned char *o = (unsigned char *)out + idx;
+        double c[3] = {C.x, C.y, C.z};
 #pragma unroll
         for (int k = 0; k < 3; k++) {
             double v = trunc(c[k] * 255.0);
@@ -845,13 +850,18 @@ __device__ __forceinline__ void pix_store(const Pix &p, const FrameParams &fp, i
             v = v > 0.0 ? v : 0.0;
             o[k] = (unsigned char)(int)v;
         }
-    } else if (fp.format == 1) {
-        float *o = (float *)fp.out + idx;
-        o[0] = (float)p.C.x; o[1] = (float)p.C.y; o[2] = (float)p.C.z;
+    } else if (format == 1) {
+        float *o = (float *)out + idx;
+        o[0] = (float)C.x; o[1] = (float)C.y; o[2] = (float)C.z;
     } else {
-        double *o = (double *)fp.out + idx;
-        o[0] = p.C.x; o[1] = p.C.y; o[2] = p.C.z;
+        double *o = (double *)out + idx;
+        o[0] = C.x; o[1] = C.y; o[2] = C.z;
     }
+}
+
+__device__ __forceinline__ void pix_store(const Pix &p, const FrameParams &fp, int X, int local_y)
+{
+    colour_store(fp.out, fp.format, ((size_t)local_y * fp.width + X) * 3, p.C);
 }
 
 // pixel coordinates of this thread: 8x4 pixels per warp, 4x2 warps per 256-thread block

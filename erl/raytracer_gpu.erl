@@ -33,6 +33,10 @@ init() ->
     erlang:load_nif(filename:join(PrivDir, "raytracer_gpu"), 0).
 
 %% ---- NIF stubs (c_src/raytracer_gpu_nif.c) ---------------------------------
+%% Opts of render/5, render_into/4, render_pixel_list/5 (and so of render_binary/5): a proplist of
+%%   {format, rgb8|f32|f64}, {accel, auto|exact|linear|bvh|bvh_mega|grid}, {part, {BandRows, NParts, Part}},
+%%   {camera, #camera{}}, and {supersample, N}: N x N rays per pixel (N an integer in 1..8), each pixel the
+%%   average of the N*N pixels of the (N*Width) x (N*Height) frame that fall in it.  Anything else is badarg.
 device_count() -> erlang:nif_error(nif_not_loaded).
 scene_info(_Scene) -> erlang:nif_error(nif_not_loaded).
 scene_upload(_Scene, _Device) -> erlang:nif_error(nif_not_loaded).

@@ -148,9 +148,20 @@ typedef struct ert_render_params {
     int32_t n_parts;
     int32_t part;
     uint32_t flags;
-    int32_t reserved;
+    /* Samples per axis N (box-filtered supersampling; 0 or 1: one ray per pixel, the reference's frame).
+     * With 2 <= N <= ERT_MAX_SUPERSAMPLE, sample k = j*N + i (i, j in [0, N)) of pixel (X, Y) is the unclamped
+     * FP64 colour of pixel (N*X + i, N*Y + j) of the (N*width) x (N*height) frame of the same scene, camera,
+     * depth and accel; the pixel is acc / (double)(N*N) with acc = c_0, then acc = acc + c_k for k = 1 .. N*N-1,
+     * stored in `format` by the rules of the formats above.  Parts, depth 0 and `camera` behave as for one
+     * sample.  ert_stats: `pixels` counts output pixels; rays, the test counters, bounce_path_rays[] and
+     * bounce_hits[] sum over all samples (bounce_path_rays[0] = pixels*N*N); times, gpu_launches and the
+     * ERT_FLAG_TIME_KERNELS split span all sample passes.  N < 0, N > ERT_MAX_SUPERSAMPLE, or N*width or
+     * N*height above INT32_MAX is ERT_ERR_BADARG. */
+    int32_t supersample;
     const ert_camera *camera;   /* NULL => the camera stored with the scene */
 } ert_render_params;
+
+#define ERT_MAX_SUPERSAMPLE 8
 
 #define ERT_MAX_BOUNCE_STATS 16
 
