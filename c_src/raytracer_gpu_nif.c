@@ -299,7 +299,8 @@ static ERL_NIF_TERM nif_scene_clone(ErlNifEnv *env, int argc, const ERL_NIF_TERM
 
 /* Opts: proplist of {format, rgb8|f32|f64} | {accel, auto|exact|linear|bvh|bvh_mega|grid} |
  *       {part, {BandRows, NParts, Part}} | {camera, CameraRecord} |
- *       {supersample, N}: N x N rays per pixel, box-filtered, N an integer in 1..ERT_MAX_SUPERSAMPLE (8) */
+ *       {supersample, N}: N x N rays per pixel, box-filtered, N an integer in 1..ERT_MAX_SUPERSAMPLE (8) |
+ *       {camera_rotation, true | false}: turn the primary rays by the camera's rotation (ERT_FLAG_CAMERA_ROTATION) */
 static int decode_opts(ErlNifEnv *env, ERL_NIF_TERM opts, ert_render_params *p, ert_camera *cam)
 {
     ERL_NIF_TERM head, tail = opts;
@@ -330,6 +331,10 @@ static int decode_opts(ErlNifEnv *env, ERL_NIF_TERM opts, ert_render_params *p, 
         } else if (is_atom_named(env, e[0], "supersample")) {
             if (!enif_get_int(env, e[1], &p->supersample) || p->supersample < 1 || p->supersample > ERT_MAX_SUPERSAMPLE)
                 return 0;
+        } else if (is_atom_named(env, e[0], "camera_rotation")) {
+            if (is_atom_named(env, e[1], "true")) p->flags |= ERT_FLAG_CAMERA_ROTATION;
+            else if (is_atom_named(env, e[1], "false")) p->flags &= ~ERT_FLAG_CAMERA_ROTATION;
+            else return 0;
         } else if (is_atom_named(env, e[0], "camera")) {
             if (!get_camera(env, e[1], cam)) return 0;
             p->camera = cam;

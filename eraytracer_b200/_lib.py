@@ -19,6 +19,7 @@ FLAG_COUNT_TESTS = 1
 FLAG_WF_UNSORTED = 2
 FLAG_NO_LIGHT_GRID = 4
 FLAG_TIME_KERNELS = 8
+FLAG_CAMERA_ROTATION = 16
 MAX_SLOTS = 4
 MAX_SUPERSAMPLE = 8
 UPDATE_REBUILD_GRIDS = 1
@@ -259,23 +260,26 @@ class Scene:
         except Exception:
             pass
 
-    def _params(self, width, height, depth, fmt, accel, band_rows, n_parts, part, flags, camera, supersample=1):
+    def _params(self, width, height, depth, fmt, accel, band_rows, n_parts, part, flags, camera, supersample=1,
+                camera_rotation=False):
         p = RenderParams()
         p.width, p.height, p.depth = int(width), int(height), int(depth)
         p.format = FORMATS[fmt] if isinstance(fmt, str) else int(fmt)
         p.accel = ACCELS[accel] if isinstance(accel, str) else int(accel)
         p.band_rows, p.n_parts, p.part = int(band_rows), int(n_parts), int(part)
-        p.flags = int(flags)
+        p.flags = int(flags) | (FLAG_CAMERA_ROTATION if camera_rotation else 0)
         p.supersample = int(supersample)
         self._cam_keep = camera
         p.camera = ctypes.pointer(camera) if camera is not None else None
         return p
 
     def render(self, width, height, depth, fmt="f64", accel="auto", band_rows=0, n_parts=1,
-               part=0, flags=0, camera=None, out=None, supersample=1):
+               part=0, flags=0, camera=None, out=None, supersample=1, camera_rotation=False):
         """Synchronous render into a numpy frame (H, W, 3); returns (frame, stats dict).  supersample=N casts N x N
-        rays per pixel and box-filters them (ert_render_params.supersample)."""
-        p = self._params(width, height, depth, fmt, accel, band_rows, n_parts, part, flags, camera, supersample)
+        rays per pixel and box-filters them (ert_render_params.supersample); camera_rotation=True turns the primary
+        rays by the camera's rotation (ERT_FLAG_CAMERA_ROTATION)."""
+        p = self._params(width, height, depth, fmt, accel, band_rows, n_parts, part, flags, camera, supersample,
+                         camera_rotation)
         if p.width <= 0 or p.height <= 0:
             # let the library produce the error (mirrors the guards at raytracer.erl:89)
             check(load().ert_render(self.handle, ctypes.byref(p), None, 0))
@@ -287,8 +291,10 @@ class Scene:
         return out, self.stats(0)
 
     def render_async(self, width, height, depth, slot=0, fmt="rgb8", accel="auto", band_rows=0,
-                     n_parts=1, part=0, flags=0, camera=None, host_ptr=None, host_bytes=0, supersample=1):
-        p = self._params(width, height, depth, fmt, accel, band_rows, n_parts, part, flags, camera, supersample)
+                     n_parts=1, part=0, flags=0, camera=None, host_ptr=None, host_bytes=0, supersample=1,
+                     camera_rotation=False):
+        p = self._params(width, height, depth, fmt, accel, band_rows, n_parts, part, flags, camera, supersample,
+                         camera_rotation)
         check(load().ert_render_async(self.handle, ctypes.byref(p), int(slot), host_ptr,
                                       int(host_bytes)))
 

@@ -1558,8 +1558,13 @@ int ert_render_async(ert_scene *scene, const ert_render_params *params, int slot
     const ert_render_params &p = *params;
     const ert_camera &cam = p.camera ? *p.camera : scene->host.camera;
     if (const std::string err = check_camera(cam); !err.empty()) return fail(ERT_ERR_BADARG, err);
+    const bool rotated = (p.flags & ERT_FLAG_CAMERA_ROTATION) != 0;
+    if (rotated)
+        if (const std::string err = check_camera_rotation(cam); !err.empty()) return fail(ERT_ERR_BADARG, err);
 
     FrameParams fp{};
+    // an identity matrix keeps today's primary rays, and so the frame without the flag
+    if (rotated) fp.rotate = camera_matrix(cam.rotation, fp.rot) ? 0 : 1;
     fp.width = p.width; fp.height = p.height; fp.depth = p.depth; fp.format = p.format;
     fp.band_rows = p.band_rows; fp.n_parts = p.n_parts <= 1 ? 1 : p.n_parts; fp.part = p.part;
     if (fp.n_parts == 1 || p.band_rows <= 0) { fp.n_parts = 1; fp.part = 0; fp.band_rows = 0; }

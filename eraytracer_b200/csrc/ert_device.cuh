@@ -109,6 +109,10 @@ struct FrameParams {
     // struct, with ray_w = ss*width and ray_h = ss*height as exact doubles: the existing kernels keep their registers.
     int ss, ss_i, ss_j;
     double ray_w, ray_h;
+    // ERT_FLAG_CAMERA_ROTATION with a matrix other than the identity: primary directions are turned by the row-major
+    // rot (include/ert_b200.h).  Appended so that the fields above keep their offsets.
+    double rot[9];
+    int rotate;
 };
 
 #ifdef ERT_PROBE
@@ -677,7 +681,14 @@ __device__ __forceinline__ void primary_ray(const FrameParams &fp, int X, int Y,
     acc = vadd(mk((x - 0.5) * fp.screen_w, 0.0, 0.0), acc);
     acc = vadd(mk(0.0, (y - 0.5) * fp.screen_h, 0.0), acc);
     O = loc;
-    D = vnormalize(vsub(acc, loc));
+    d3 v = vsub(acc, loc);
+    if (fp.rotate) {
+        // d_i = (M[i][0]*v.x + M[i][1]*v.y) + M[i][2]*v.z, uncontracted (-fmad=false)
+        const double *m = fp.rot;
+        v = mk((m[0] * v.x + m[1] * v.y) + m[2] * v.z, (m[3] * v.x + m[4] * v.y) + m[5] * v.z,
+               (m[6] * v.x + m[7] * v.y) + m[8] * v.z);
+    }
+    D = vnormalize(v);
 }
 
 __device__ __forceinline__ void pix_init(Pix &p, const DevScene &sc, const FrameParams &fp, int X, int Y, bool inside)

@@ -80,6 +80,54 @@ std::string check_camera(const ert_camera &c)
     return "camera has a non-finite field";
 }
 
+std::string check_camera_rotation(const ert_camera &c)
+{
+    return finite3(c.rotation) ? std::string() : "camera rotation has a non-finite field";
+}
+
+namespace {
+
+// (sin, cos) of deg degrees: fmod is exact, quarter turns are exact, the rest the host libm's sin and cos
+void sin_cos_deg(double deg, double &s, double &c)
+{
+    const double a = std::fmod(deg, 360.0);
+    if (a == 0.0) { s = 0.0; c = 1.0; }
+    else if (a == 90.0 || a == -270.0) { s = 1.0; c = 0.0; }
+    else if (a == 180.0 || a == -180.0) { s = 0.0; c = -1.0; }
+    else if (a == 270.0 || a == -90.0) { s = -1.0; c = 0.0; }
+    else {
+        const double r = a * (M_PI / 180.0);
+        s = std::sin(r);
+        c = std::cos(r);
+    }
+}
+
+void mat_mul(const double A[9], const double B[9], double P[9])
+{
+    for (int i = 0; i < 3; i++)
+        for (int j = 0; j < 3; j++)
+            P[3 * i + j] = (A[3 * i] * B[j] + A[3 * i + 1] * B[3 + j]) + A[3 * i + 2] * B[6 + j];
+}
+
+}  // namespace
+
+bool camera_matrix(const double rotation[3], double M[9])
+{
+    double sx, cx, sy, cy, sz, cz;
+    sin_cos_deg(rotation[0], sx, cx);
+    sin_cos_deg(rotation[1], sy, cy);
+    sin_cos_deg(rotation[2], sz, cz);
+    const double Rx[9] = {1, 0, 0, 0, cx, -sx, 0, sx, cx};
+    const double Ry[9] = {cy, 0, sy, 0, 1, 0, -sy, 0, cy};
+    const double Rz[9] = {cz, -sz, 0, sz, cz, 0, 0, 0, 1};
+    double XZ[9];
+    mat_mul(Rx, Rz, XZ);
+    mat_mul(Ry, XZ, M);
+    for (int k = 0; k < 9; k++)
+        if (M[k] != (k % 4 == 0 ? 1.0 : 0.0)) return false;
+    return true;
+}
+
 std::string check_create(const ert_scene_desc *d, SourceOrder &src, std::vector<int> order[K_COUNT])
 {
     if (!d) return "scene descriptor is NULL";

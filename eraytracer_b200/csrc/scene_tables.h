@@ -29,6 +29,11 @@ using SourceOrder = std::array<std::vector<int64_t>, K_COUNT>;
 
 // The checks return the message of the first defect (an ERT_ERR_BADARG), or an empty string.
 std::string check_camera(const ert_camera &c);
+// ERT_FLAG_CAMERA_ROTATION: the rotation must be finite
+std::string check_camera_rotation(const ert_camera &c);
+// M = Ry(ry) . (Rx(rx) . Rz(rz)) of rotation = (rx, ry, rz) in degrees, row-major (include/ert_b200.h); returns
+// true when M is exactly the identity
+bool camera_matrix(const double rotation[3], double M[9]);
 // ert_scene_create: the header, then list positions >= 0 and distinct across all kinds.  src: lights and spheres in
 // list order, planes and triangles as listed; order[k]: the list positions of kind k in that order.
 std::string check_create(const ert_scene_desc *d, SourceOrder &src, std::vector<int> order[K_COUNT]);

@@ -29,19 +29,22 @@ def _function_clause(name, args):
     raise ValueError("function_clause: no clause of %s matches %r" % (name, args))
 
 
-def render_frame(width, height, scene_list, recursion_depth, fmt="f64", accel="auto", device=0, supersample=1):
+def render_frame(width, height, scene_list, recursion_depth, fmt="f64", accel="auto", device=0, supersample=1,
+                 camera_rotation=False):
     """Renders one frame on one GPU; returns (frame[H,W,3], stats).  supersample=N box-filters N x N rays per
-    pixel: the pixels of the (N*width) x (N*height) frame that fall in it."""
+    pixel: the pixels of the (N*width) x (N*height) frame that fall in it.  camera_rotation=True turns the primary
+    rays by the camera's rotation, which the reference ignores (ERT_FLAG_CAMERA_ROTATION)."""
     flat = scene_list if isinstance(scene_list, _scene.FlatScene) else _scene.flatten(scene_list)
     dev_scene = flat.upload(device)
     try:
-        return dev_scene.render(width, height, recursion_depth, fmt=fmt, accel=accel, supersample=supersample)
+        return dev_scene.render(width, height, recursion_depth, fmt=fmt, accel=accel, supersample=supersample,
+                                camera_rotation=camera_rotation)
     finally:
         dev_scene.close()
 
 
 def render_frame_multi_gpu(width, height, scene_list, recursion_depth, fmt="f64", accel="auto",
-                           devices=None, band_rows=16, supersample=1):
+                           devices=None, band_rows=16, supersample=1, camera_rotation=False):
     """One frame split into row bands dealt round-robin to the GPUs of this box
     (the row-band mapping of distribute_work/7, raytracer.erl:139-149).  Every GPU copies
     its bands straight into one pinned host frame; there is no gather step."""
@@ -63,7 +66,8 @@ def render_frame_multi_gpu(width, height, scene_list, recursion_depth, fmt="f64"
         for part, sc in enumerate(scenes):
             sc.render_async(width, height, recursion_depth, slot=0, fmt=fmt, accel=accel,
                             band_rows=band_rows, n_parts=len(scenes), part=part,
-                            host_ptr=pinned.ptr, host_bytes=nbytes, supersample=supersample)
+                            host_ptr=pinned.ptr, host_bytes=nbytes, supersample=supersample,
+                            camera_rotation=camera_rotation)
         for sc in scenes:
             sc.wait(0)
         stats = [sc.stats(0) for sc in scenes]

@@ -70,6 +70,22 @@ def camera_struct(rec):
     return cam
 
 
+def look_at(location, target):
+    """The camera rotation (rx, ry, 0.0), in degrees, whose forward axis (ERT_FLAG_CAMERA_ROTATION) points from
+    `location` to `target` (#vector{} records or 3-sequences).  ry = atan2(fx, fz), rx = atan2(-fy, sqrt(fx*fx +
+    fz*fz)) of f = target - location, each turned into degrees as a * 180.0 / pi; raytracer_gpu:look_at/2 is the
+    same function in Erlang.  Integers stay integers until atan2, as in Erlang (so -0 is 0)."""
+    def exact(x):
+        _num(x)
+        return int(x) if isinstance(x, (int, np.integer)) else float(x)
+    lx, ly, lz = (exact(v) for v in (location[1:] if len(location) == 4 else location))
+    tx, ty, tz = (exact(v) for v in (target[1:] if len(target) == 4 else target))
+    fx, fy, fz = tx - lx, ty - ly, tz - lz
+    ry = math.atan2(fx, fz)
+    rx = math.atan2(-fy, math.sqrt(fx * fx + fz * fz))
+    return (rx * 180.0 / math.pi, ry * 180.0 / math.pi, 0.0)
+
+
 class FlatScene:
     """The four element tables plus the camera, ready for ert_scene_create."""
 

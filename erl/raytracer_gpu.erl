@@ -22,7 +22,8 @@
          render_binary/5,
          write_binary_to_ppm/4,
          device_count/0, scene_info/1, scene_upload/2, scene_clone/2, render/5, render_pixel_list/5,
-         frame_alloc/3, render_into/4, frame_binary/1]).
+         frame_alloc/3, render_into/4, frame_binary/1,
+         look_at/2]).
 -on_load(init/0).
 
 init() ->
@@ -35,8 +36,11 @@ init() ->
 %% ---- NIF stubs (c_src/raytracer_gpu_nif.c) ---------------------------------
 %% Opts of render/5, render_into/4, render_pixel_list/5 (and so of render_binary/5): a proplist of
 %%   {format, rgb8|f32|f64}, {accel, auto|exact|linear|bvh|bvh_mega|grid}, {part, {BandRows, NParts, Part}},
-%%   {camera, #camera{}}, and {supersample, N}: N x N rays per pixel (N an integer in 1..8), each pixel the
-%%   average of the N*N pixels of the (N*Width) x (N*Height) frame that fall in it.  Anything else is badarg.
+%%   {camera, #camera{}}, {supersample, N}: N x N rays per pixel (N an integer in 1..8), each pixel the
+%%   average of the N*N pixels of the (N*Width) x (N*Height) frame that fall in it, and {camera_rotation, true}:
+%%   the primary rays turned by the camera's rotation {vector, Rx, Ry, Rz} in degrees, M = Ry . Rx . Rz about the
+%%   world axes (+y is down: {vector, 0, 90, 0} looks along +x, {vector, 90, 0, 0} up; see look_at/2).  The
+%%   reference ignores the rotation, and so does the default {camera_rotation, false}.  Anything else is badarg.
 device_count() -> erlang:nif_error(nif_not_loaded).
 scene_info(_Scene) -> erlang:nif_error(nif_not_loaded).
 scene_upload(_Scene, _Device) -> erlang:nif_error(nif_not_loaded).
@@ -102,6 +106,16 @@ write_binary_to_ppm(Width, Height, FrameRgb8, Filename) ->
     Body = [[integer_to_list(V), $\s] || <<V:8>> <= FrameRgb8],
     file:write_file(Filename,
                     [io_lib:format("P3~n~p ~p~n~p~n", [Width, Height, 255]), Body]).
+
+%% The camera rotation whose forward axis points from Location to Target, for {camera_rotation, true}:
+%% Ry = atan2(Fx, Fz), Rx = atan2(-Fy, sqrt(Fx*Fx + Fz*Fz)) of F = Target - Location, in degrees, no roll.
+look_at({vector, Lx, Ly, Lz}, {vector, Tx, Ty, Tz}) ->
+    Fx = Tx - Lx,
+    Fy = Ty - Ly,
+    Fz = Tz - Lz,
+    Ry = math:atan2(Fx, Fz),
+    Rx = math:atan2(-Fy, math:sqrt(Fx * Fx + Fz * Fz)),
+    {vector, Rx * 180.0 / math:pi(), Ry * 180.0 / math:pi(), 0.0}.
 
 ok_or_exit({ok, _} = Ok) -> Ok;
 ok_or_exit({error, Reason}) -> exit({raytracer_gpu, Reason}).

@@ -56,7 +56,7 @@ typedef struct ert_material {      /* -record(material, ...) erl:77 */
 
 typedef struct ert_camera {        /* -record(camera, ...) erl:76, screen erl:75 */
     double location[3];
-    double rotation[3];            /* stored, ignored exactly like erl:487 */
+    double rotation[3];            /* degrees; ignored like erl:487 unless ERT_FLAG_CAMERA_ROTATION is set */
     double fov;                    /* degrees */
     double screen_width;
     double screen_height;
@@ -135,6 +135,22 @@ typedef struct ert_scene_desc {
                                    * direction grid (A/B switch; same frame) */
 #define ERT_FLAG_WF_UNSORTED  2u  /* ERT_ACCEL_BVH: skip the binning of hits by location (A/B switch; the
                                    * frame is identical, only the schedule of the queues changes) */
+/* Turn the primary rays by the camera's `rotation` (the per-call camera, or the scene's).  Without this flag the
+ * rotation is not read and every frame is the reference's, which ignores it (erl:487).  With it:
+ *   - primary ray: v = point_on_screen - location as today (erl:486-507), O = location, D = vnormalize(d) with
+ *     d_i = (M[i][0]*v.x + M[i][1]*v.y) + M[i][2]*v.z in FP64, nothing contracted;
+ *   - M = Ry(ry) . (Rx(rx) . Rz(rz)) with (rx, ry, rz) = rotation in degrees, right-handed rotations about the
+ *     world axes: Rx = [[1,0,0],[0,c,-s],[0,s,c]], Ry = [[c,0,s],[0,1,0],[-s,0,c]], Rz = [[c,-s,0],[s,c,0],[0,0,1]],
+ *     each product entry (A[i][0]*B[0][j] + A[i][1]*B[1][j]) + A[i][2]*B[2][j], computed once per call on the host;
+ *   - angle: a = fmod(deg, 360.0) (exact); a in {0, +-90, +-180, +-270} gives the exact (s, c) in {-1, 0, 1} (s = +0
+ *     where it is 0), any other a gives s = sin(r), c = cos(r) with r = a * (M_PI / 180.0) (the host libm);
+ *   - if M is exactly the identity (e.g. (0,0,0), (360,-720,0), (180,180,180)) the frame is bit-identical to the
+ *     same call without the flag.
+ * World +y is down (floors at y = 5, lights at negative y), so (0,90,0) looks along +x, (0,180,0) along -z,
+ * (90,0,0) along -y (up), and rz rolls the picture about the view axis.  Supersampling (each sub-pixel ray is
+ * turned), parts, slots, ert_download and ert_stats behave as without the flag.  A non-finite rotation is
+ * ERT_ERR_BADARG with the flag and is accepted without it. */
+#define ERT_FLAG_CAMERA_ROTATION 16u
 
 typedef struct ert_render_params {
     int32_t width, height;      /* pixels, both > 0 (guards at erl:89) */
